@@ -2,6 +2,7 @@
 """bench.py -- EM channel-estimation trials/s on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C] [--trials-per-step B]
+                    [--dump-outputs DIR]
 
 Workload (default --config 2 = BASELINE.json configs[1], the north-star size): one NMSE-vs-T_d sweep point of
 Proposed_method_NMSEvsTd.py scaled to N=64 RIS elements, 4x4 MIMO, 16-QAM (K = 65536 joint hypotheses per data
@@ -164,6 +165,35 @@ class ClockSampler:
         return out
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+DUMP_SAMPLE_SEED = 20261
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes the per-trial outputs `arrays` (name -> array with the trial index outermost) to
+    out_dir/<name>.npy as float64; complex arrays gain a trailing (real, imag) axis.  When the files would exceed
+    `limit` bytes in all, the same fixed, seeded sample of trials is written from every array, and its trial
+    indices go to out_dir/trial_index.npy.  Returns the number of trials written."""
+    import numpy as np
+
+    conv = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a)
+        conv[name] = a.view(np.float64).reshape(a.shape + (2,)) if a.dtype.kind == "c" else a.astype(np.float64)
+    B = next(iter(conv.values())).shape[0]
+    per_trial = sum(a.nbytes for a in conv.values()) // max(1, B)
+    payload = limit - 256 * (len(conv) + 1)          # room for the .npy headers
+    keep = B if per_trial * B <= payload else max(1, payload // (per_trial + 8))
+    os.makedirs(out_dir, exist_ok=True)
+    idx = None
+    if keep < B:
+        idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(B, size=keep, replace=False))
+        np.save(os.path.join(out_dir, "trial_index.npy"), idx.astype(np.float64))
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a if idx is None else a[idx])
+    return keep
+
+
 def workload_dict(w):
     d = w.as_dict()
     d.update(partition_r=w.partition_r, quirks=w.quirks, zero_start=w.zero_start)
@@ -321,7 +351,7 @@ def run_ours(args):
         barrier()
         engine.profile_begin()
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        nfs = max(1, min(args.steps, 3))
+        nfs = args.steps
         f0.record()
         for _ in range(nfs):
             step_fs()
@@ -362,10 +392,9 @@ def run_ours(args):
             ok = hout.status == 0
             return np.array([float(hout.nmse[ok].sum()), float(ok.sum()), float((~ok).sum())])
 
-        # >= 40 synchronous calls for the headline (~2.4 s): on this pool's VM hosts single calls sporadically take
-        # 1.3-5x longer; with 40 calls one such call moves the mean by < 10 % (the median shows the steady state)
-        e2e_steps = max(args.steps, 40) if w.key == 2 else args.steps
-        # warm-up: pool allocation and >= 1.5 s of steady calls.  On this pool's VM hosts single calls sporadically
+        # --steps synchronous calls.  Single calls sporadically take 1.3-5x longer on a shared host, so with few
+        # steps one such call moves the mean noticeably; e2e.median_step_ms shows the steady state.
+        # warm-up: pool allocation and >= 1.5 s of steady calls.  On a shared host single calls sporadically
         # take 1.5-2x longer for ~0.3 s at a time (SM clock and the copy rate unchanged; the device-timed `value`
         # queues its kernels ahead and does not see it): e2e.value is the honest mean over the timed calls,
         # e2e.median_step_ms shows the steady state
@@ -393,7 +422,7 @@ def run_ours(args):
         barrier()
         step_ms, accs = [], []
         t0 = time.perf_counter()
-        for _ in range(e2e_steps):
+        for _ in range(args.steps):
             ta = time.perf_counter()
             e2e_step()          # synchronous: returns after the D2H copies completed
             accs.append(point_acc())
@@ -404,9 +433,9 @@ def run_ours(args):
         te = torch.tensor([t1 - t0], dtype=torch.float64, device=dev)
         if world > 1:
             tdist.all_reduce(te, op=tdist.ReduceOp.MAX)
-        e2e = dict(value=world * B * e2e_steps / float(te.item()), unit=UNIT,
+        e2e = dict(value=world * B * args.steps / float(te.item()), unit=UNIT,
                    h2d_bytes_per_step=int(input_bytes) * world, d2h_bytes_per_step=int(d2h_bytes) * world,
-                   bytes_are="whole job (all ranks)", steps=e2e_steps, warmup_calls=nw,
+                   bytes_are="whole job (all ranks)", steps=args.steps, warmup_calls=nw,
                    step_ms=[round(x, 2) for x in step_ms], median_step_ms=round(statistics.median(step_ms), 2),
                    h2d_gbs_measured=h2d_gbs,
                    collective="one NCCL sum of %d float64 inside the timed region" % acc_global.size if world > 1 else None,
@@ -599,6 +628,8 @@ def run_ours(args):
                 gpu_launches=int(launches), clocks=clocks, roofline=roofline, kernels=kernels, cpu_baseline=cpu,
                 full_scan=full,
                 check=dict(nmse_mean=nmse_mean, nmse_ls_start=nmse_init, flagged_trials=int((st != 0).sum())))
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, dev_out)
     print(json.dumps(line))
     if world > 1:
         tdist.barrier()
@@ -609,7 +640,8 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=6)
+    ap.add_argument("--steps", type=int, default=6,
+                    help="timed steps of every leg (device route, full scan, e2e, on-device sweep points)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=[1, 2, 3, 4, 41, 5],
@@ -620,7 +652,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-scan", action="store_true")
     ap.add_argument("--kernels-only", action="store_true", help="device-resident leg only (kernel tuning runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (theta, kstar, lse, nmse, "
+                         "iters, status of rank 0's trials) to DIR/<name>.npy as float64, at most 64 MB in all; "
+                         "inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -120,6 +120,35 @@ def test_headline_config_all_routes_bitwise_equal_and_match_oracle(S):
     assert hout.nmse[:32].mean() < 0.2 * nm0
 
 
+def test_bench_dump_outputs_shapes_and_reproducibility(S, tmp_path):
+    """`bench.py --dump-outputs` on workload 1 (on-device inputs): two runs with the same arguments write the
+    same arrays (same inputs, same results), in the shapes a caller of the device route receives."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    w = S.workloads.WORKLOADS[1]
+    B = 64
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--config", "1", "--steps", "2",
+                              "--trials-per-step", str(B), "--kernels-only", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 2
+        dumps.append({f[:-4]: np.load(d / f) for f in sorted(os.listdir(d))})
+    a, b = dumps
+    assert set(a) == {"theta", "kstar", "lse", "nmse", "iters", "status"}
+    assert a["theta"].shape == (B, w.L, w.n_rx, 2) and a["kstar"].shape == (B, w.T_d)
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert (a["status"] == 0).all() and (a["iters"] == w.itera).all()
+    for k in a:
+        assert same(a[k], b[k]), k
+
+
 @pytest.mark.parametrize("shared", ["none", "pilots", "all"])
 def test_chunked_workspace_small(S, shared):
     """B = 7 trials through a workspace of 3: per-trial, pilot-shared and fully shared phase layouts

@@ -106,6 +106,40 @@ def test_bench_work_models_match_design_section_5():
     assert f8["gram"] > 0 and f8["chol"] > 1.1e10                          # SURVEY: ~1.2e10 flops per Cholesky at L = 2056
 
 
+def test_bench_dump_outputs_format_and_size_limit(tmp_path):
+    """bench.py --dump-outputs: every array as float64 (complex ones with a trailing real/imag axis); above the
+    size limit the same seeded sample of trials from every array, with its trial indices, within the limit."""
+    import bench
+
+    rng = np.random.default_rng(0)
+    B = 50
+    arrays = dict(theta=rng.standard_normal((B, 6, 2)) + 1j * rng.standard_normal((B, 6, 2)),
+                  kstar=rng.integers(0, 16, (B, 7)).astype(np.int32), nmse=rng.random(B))
+    assert bench.dump_outputs(str(tmp_path / "all"), arrays) == B
+    assert sorted(os.listdir(tmp_path / "all")) == ["kstar.npy", "nmse.npy", "theta.npy"]
+    th, ks = np.load(tmp_path / "all" / "theta.npy"), np.load(tmp_path / "all" / "kstar.npy")
+    assert th.dtype == np.float64 and np.array_equal(th[..., 0] + 1j * th[..., 1], arrays["theta"])
+    assert ks.dtype == np.float64 and np.array_equal(ks, arrays["kstar"])
+
+    limit = 4096
+    n = bench.dump_outputs(str(tmp_path / "a"), arrays, limit=limit)
+    assert 0 < n < B and bench.dump_outputs(str(tmp_path / "b"), arrays, limit=limit) == n
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["kstar.npy", "nmse.npy", "theta.npy", "trial_index.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= limit
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f
+    idx = np.load(tmp_path / "a" / "trial_index.npy").astype(np.int64)
+    assert len(idx) == n and np.all(np.diff(idx) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "nmse.npy"), arrays["nmse"][idx])
+
+
+def test_bench_rejects_fewer_than_one_step():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (CPU oracle port) on the smallest workload: same metric / unit / config keys,
     impl = reference, a cpu_baseline describing the run, zero-copy e2e."""
