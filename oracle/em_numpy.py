@@ -249,6 +249,53 @@ def posterior_stats(Yd, PsiD, Theta, cons, n_tx, varn, hard=False, chunk=None):
     return m, R, kstar, lse
 
 
+def posterior_stats_split(Yd, PsiD, Theta, cons, n_tx, varn, hard=False):
+    """posterior_stats for trees too large for one hypothesis table (2^24 leaves: 4 streams of 64-QAM, 6 of
+    16-QAM).  The streams are split into a leading half A and a trailing half B (k = a * K_B + b); the residual
+    y - H_A x_a - H_B x_b and its squared norm are still formed directly for every (a, b), block by block, and
+    the posterior sums reduce over b (statistics of A), over a (statistics of B) and through one
+    conj(X_A)^T beta X_B product (cross terms of R)."""
+    T_d = Yd.shape[0]
+    M = len(cons)
+    nA = n_tx // 2
+    XA, XB = hypothesis_table(cons, nA), hypothesis_table(cons, n_tx - nA)
+    KA, KB = len(XA), len(XB)
+    Heff = effective_channels(PsiD, Theta, n_tx)
+    s2 = float(varn) ** 2
+    m = np.zeros((T_d, n_tx), dtype=np.complex128)
+    R = np.zeros((T_d, n_tx, n_tx), dtype=np.complex128)
+    kstar = np.zeros(T_d, dtype=np.int64)
+    lse = np.zeros(T_d)
+    rows = max(1, (1 << 21) // KB)
+    for t in range(T_d):
+        u = Yd[t][None, :] - XA @ Heff[t][:, :nA].T            # (KA, n_rx)
+        v = XB @ Heff[t][:, nA:].T                             # (KB, n_rx)
+        d2 = np.empty((KA, KB))
+        for a0 in range(0, KA, rows):
+            r = u[a0:a0 + rows, None, :] - v[None, :, :]
+            d2[a0:a0 + rows] = (r.real ** 2 + r.imag ** 2).sum(axis=2)
+        k = int(np.argmin(d2))
+        dmin = d2.flat[k]
+        e = np.exp(-(d2 - dmin) / s2)
+        se = e.sum()
+        kstar[t] = k
+        lse[t] = -dmin / s2 + np.log(se)
+        if hard:
+            x = np.concatenate([XA[k // KB], XB[k % KB]])
+            m[t] = x.conj()
+            R[t] = x.conj()[:, None] * x[None, :]
+            continue
+        beta = e / se
+        bA, bB = beta.sum(axis=1), beta.sum(axis=0)
+        m[t, :nA], m[t, nA:] = bA @ XA.conj(), bB @ XB.conj()
+        R[t, :nA, :nA] = np.einsum("a,ai,aj->ij", bA, XA.conj(), XA)
+        R[t, nA:, nA:] = np.einsum("b,bi,bj->ij", bB, XB.conj(), XB)
+        R[t, :nA, nA:] = XA.conj().T @ beta @ XB
+        R[t, nA:, :nA] = R[t, :nA, nA:].conj().T
+    assert KA * KB == M ** n_tx
+    return m, R, kstar, lse
+
+
 # --------------------------------------------------------------------------
 # M-step pieces
 # --------------------------------------------------------------------------

@@ -56,8 +56,9 @@ static int make_dims(const sbce_cfg* c, Dims* d, bool with_estep = true) {
     int sq = 0;
     if (c->M == 4) sq = 2; else if (c->M == 16) sq = 4; else if (c->M == 64) sq = 8; else return SBCE_E_UNSUPPORTED;
     if (c->n_tx > 8 || c->n_rx > 8) return SBCE_E_UNSUPPORTED;
-    // the normal-equation kernels stage chunks of the phase rows in shared memory (mstep.cu: gram_supports)
-    if (!gram_supports(c->N + 1, c->n_tx)) return SBCE_E_UNSUPPORTED;
+    // the normal-equation kernels stage chunks of the phase rows in shared memory; gram_supports() is the same
+    // size computation the Gram launchers use (mstep.cu: gram_smem)
+    if (!gram_supports(c->N + 1, c->n_tx, c->n_rx)) return SBCE_E_UNSUPPORTED;
     if (c->n_tx <= 4 && !(c->n_rx <= 4 || c->n_rx == 6 || c->n_rx == 8)) return SBCE_E_UNSUPPORTED;
     if (c->mode < SBCE_MODE_SOFT || c->mode > SBCE_MODE_MMSE) return SBCE_E_UNSUPPORTED;
     if (with_estep) {

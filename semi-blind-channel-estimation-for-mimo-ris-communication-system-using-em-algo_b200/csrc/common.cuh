@@ -113,7 +113,7 @@ cudaError_t launch_enum(const Dims& d, int nb, const double* qr, const double* v
 cudaError_t launch_normal_equations(const Dims& d, int nb, const double* Psi, int T, const double* Y,
                                     const double* sm, const double* sR, const double* Ginit, double* Gout,
                                     const int32_t* active, cudaStream_t s);
-bool gram_supports(int N1, int n_tx);   // phase rows short enough for the shared-memory staging of the Gram kernels
+bool gram_supports(int N1, int n_tx, int n_rx);   // the Gram launch of this shape fits in shared memory (mstep.cu)
 cudaError_t launch_chol_solve(const Dims& d, int nb, double* G, double* theta, const int32_t* active, int32_t* stat,
                               double* th_scratch, cudaStream_t s);
 // metrics (metrics.cu)

@@ -609,16 +609,42 @@ __global__ void __launch_bounds__(GR_THREADS, 1) k_gram_mma(Dims d, int T, int T
 // shared memory the right-hand-side CTA needs at least: one 8-symbol MMA step of psi and of the padded Zc rows
 static size_t rhs_smem_min(int N1, int ntx, int n_rx) { return sizeof(cplx) * (size_t)(8 * (N1 + ntx * n_rx + 2)); }
 
-// largest chunk length (multiple of 8, at most 32) whose two stages fit in `budget` bytes
-static int gram_chunk(int N1, int ntx, size_t budget) {
-    int tc = 32;
-    while (tc > 8 && sizeof(cplx) * (size_t)(2 * tc * (N1 + ntx * ntx)) > budget) tc >>= 1;
-    return tc;
+constexpr size_t GRAM_SMEM_CAP = 227 * 1024;   // opt-in shared memory per block on sm_100
+
+// Dynamic shared memory of the one Gram launch for a shape, and the pair CTAs' chunk length.  The pair CTAs need
+// their operand stages; the right-hand-side CTA of the same launch sizes its chunk from whatever it finds (16
+// symbols when they fit under the cap, one 8-symbol MMA step at least).  make_dims() admits a shape through
+// gram_supports(), the launchers below request exactly this: an admitted shape is a shape that launches.
+static size_t gram_smem(int N1, int ntx, int n_rx, int* tc_out) {
+    const size_t rhs1 = rhs_smem_min(N1, ntx, n_rx);
+    size_t pair, rhs_want = 2 * rhs1;
+    int tc;
+    if (ntx <= 3) {           // scalar k_gram: two cp.async stages, chunk shrunk for very long phase rows
+        tc = GR_TC;
+        while (tc > 2 && sizeof(cplx) * (size_t)(2 * tc * (N1 + ntx * ntx)) > 100 * 1024) tc >>= 1;
+        pair = sizeof(cplx) * (size_t)(2 * tc * (N1 + ntx * ntx));
+        rhs_want = rhs1;
+    } else if (ntx == 4 && sizeof(cplx) * (size_t)(GT_STAGES * GT_TC * (N1 + 16)) <= 160 * 1024) {
+        tc = GT_TC;               // k_gram_tma4: four-stage TMA ring (N <= 143)
+        pair = sizeof(cplx) * (size_t)(GT_STAGES * GT_TC * (N1 + 16));
+    } else {                      // k_gram_mma<NTX>: two stages of the largest chunk under 100 KB, 8 symbols at least
+        tc = 32;
+        while (tc > 8 && sizeof(cplx) * (size_t)(2 * tc * (N1 + ntx * ntx)) > 100 * 1024) tc >>= 1;
+        pair = sizeof(cplx) * (size_t)(2 * tc * (N1 + ntx * ntx));
+    }
+    if (tc_out) *tc_out = tc;
+    size_t smem = pair > rhs_want ? pair : rhs_want;
+    if (smem > GRAM_SMEM_CAP) smem = pair > rhs1 ? pair : rhs1;
+    return smem;
 }
 
-// Shared-memory ceiling of the Gram kernels: two stages of at least 8 symbols must fit in 227 KB.  abi.cu's
-// make_dims() rejects longer phase rows with SBCE_E_UNSUPPORTED before any launch (N + 1 + n_tx^2 <= 908).
-bool gram_supports(int N1, int n_tx) { return sizeof(cplx) * (size_t)(2 * 8 * (N1 + n_tx * n_tx)) <= 227 * 1024; }
+// Admitted phase-row lengths: N + 1 + n_tx^2 <= 908 for every n_tx (two 8-symbol stages of the generic kernel in
+// 227 KB; the documented limit, also for the scalar kernel, which would take longer rows), and the launch for
+// this shape must fit.  abi.cu's make_dims() answers SBCE_E_UNSUPPORTED otherwise, before any launch.
+bool gram_supports(int N1, int n_tx, int n_rx) {
+    return sizeof(cplx) * (size_t)(2 * 8 * (N1 + n_tx * n_tx)) <= GRAM_SMEM_CAP &&
+           gram_smem(N1, n_tx, n_rx, nullptr) <= GRAM_SMEM_CAP;
+}
 
 template <int NTX>
 static cudaError_t run_gram_wide(const Dims& d, int nb, const double* Psi, int T, const double* sR, const double* Y,
@@ -627,12 +653,9 @@ static cudaError_t run_gram_wide(const Dims& d, int nb, const double* Psi, int T
     static SmemOptIn optin;
     const int P = d.N1 * (d.N1 + 1) / 2;
     dim3 grid((P + GW_PAIRS - 1) / GW_PAIRS + 1, nb);   // + 1: the right-hand-side / padding CTA
-    int tc = gram_chunk(d.N1, NTX, 100 * 1024);
-    if (sizeof(cplx) * (size_t)(2 * tc * (d.N1 + NTX * NTX)) > 227 * 1024) return cudaErrorInvalidValue;
-    size_t smem = sizeof(cplx) * (size_t)(2 * tc * (d.N1 + NTX * NTX));
-    const size_t smem_rhs = 2 * rhs_smem_min(d.N1, NTX, d.n_rx);                    // 16-symbol chunks at least
-    if (smem_rhs > smem) smem = smem_rhs;
-    if (smem > 227 * 1024) return cudaErrorInvalidValue;
+    int tc = 0;
+    const size_t smem = gram_smem(d.N1, NTX, d.n_rx, &tc);
+    if (smem > GRAM_SMEM_CAP) return cudaErrorInvalidValue;
     cudaError_t e = opt_in_smem(optin, (const void*)k_gram_mma<NTX>, smem);
     if (e != cudaSuccess) return e;
     k_gram_mma<NTX><<<grid, GR_THREADS, smem, s>>>(d, T, tc, (const cplx*)Psi, (const cplx*)sR, (const cplx*)Y,
@@ -649,12 +672,9 @@ static cudaError_t run_gram_scalar(const Dims& d, int nb, const double* Psi, int
     static SmemOptIn optin;
     const int P = d.N1 * (d.N1 + 1) / 2;
     dim3 grid((P + GR_THREADS - 1) / GR_THREADS + 1, nb);   // + 1: the right-hand-side / padding CTA
-    int tc = GR_TC;
-    while (tc > 2 && sizeof(cplx) * (size_t)(2 * tc * (d.N1 + NTX * NTX)) > 100 * 1024) tc >>= 1;
-    size_t smem = sizeof(cplx) * (size_t)(2 * tc * (d.N1 + NTX * NTX));          // two cp.async stages (pair CTAs)
-    const size_t smem_rhs = rhs_smem_min(d.N1, NTX, d.n_rx);                      // rhs CTA: one MMA step at least
-    if (smem_rhs > smem) smem = smem_rhs;
-    if (smem > 227 * 1024) return cudaErrorInvalidValue;
+    int tc = 0;
+    const size_t smem = gram_smem(d.N1, NTX, d.n_rx, &tc);
+    if (smem > GRAM_SMEM_CAP) return cudaErrorInvalidValue;
     cudaError_t e = opt_in_smem(optin, (const void*)k_gram<NTX>, smem);
     if (e != cudaSuccess) return e;
     k_gram<NTX><<<grid, GR_THREADS, smem, s>>>(d, T, tc, (const cplx*)Psi, (const cplx*)sR, (const cplx*)Y,
@@ -669,12 +689,11 @@ static cudaError_t run_gram4(const Dims& d, int nb, const double* Psi, int T, co
                              cudaStream_t s) {
     constexpr int NTX = 4;
     static SmemOptIn optin;
-    size_t smem = sizeof(cplx) * (size_t)(GT_STAGES * GT_TC * (d.N1 + NTX * NTX));
-    if (smem > 160 * 1024) return run_gram_wide<4>(d, nb, Psi, T, sR, Y, sm, Ginit, Gout, active, s);
+    if (sizeof(cplx) * (size_t)(GT_STAGES * GT_TC * (d.N1 + NTX * NTX)) > 160 * 1024)
+        return run_gram_wide<4>(d, nb, Psi, T, sR, Y, sm, Ginit, Gout, active, s);
     const int P = d.N1 * (d.N1 + 1) / 2;
     dim3 grid((P + GR_THREADS - 1) / GR_THREADS + 1, nb);   // + 1: the right-hand-side / padding CTA
-    const size_t smem_rhs = 2 * rhs_smem_min(d.N1, NTX, d.n_rx);
-    if (smem_rhs > smem) smem = smem_rhs;
+    const size_t smem = gram_smem(d.N1, NTX, d.n_rx, nullptr);
     cudaError_t e = opt_in_smem(optin, (const void*)k_gram_tma4, smem);
     if (e != cudaSuccess) return e;
     k_gram_tma4<<<grid, GT_THREADS, smem, s>>>(d, T, (const cplx*)Psi, (const cplx*)sR, (const cplx*)Y,

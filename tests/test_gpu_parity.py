@@ -44,6 +44,11 @@ ESTEP_CASES = [
     # multiple of 8), symbol counts that are not multiples of 16 / 32 / 128
     (15, 1, 8, 4, 37, 0.3), (17, 2, 4, 16, 33, 0.4), (20, 3, 4, 4, 40, 0.3), (16, 4, 4, 4, 130, 0.2),
     (23, 4, 6, 4, 19, 0.3), (18, 3, 8, 4, 21, 0.4), (31, 4, 8, 4, 45, 0.3), (40, 2, 6, 16, 29, 0.5),
+    # 64-QAM on 3 and 4 streams (16-lane PAM groups of the narrow flush), peaked and flat posteriors (varn >= 4
+    # overflows the candidate queue); 6 streams of 16-QAM (2^24 leaves)
+    (5, 3, 4, 64, 4, 0.2), (5, 3, 4, 64, 4, 6.0), (4, 4, 4, 64, 1, 0.2), (4, 4, 4, 64, 1, 5.0), (3, 6, 6, 16, 1, 0.4),
+    # effective channel too long for shared memory and for the tensor path (BASELINE.json config 3: N = 256)
+    (256, 4, 4, 4, 6, 0.3),
 ]
 
 
@@ -67,8 +72,9 @@ def test_estep_matches_oracle(S, orc, case, hard):
     torch.cuda.synchronize()
     m, R, ks, ls = m.cpu().numpy(), R.cpu().numpy(), ks.cpu().numpy(), ls.cpu().numpy()
     cons = orc.qam_constellation(M)
+    stats = orc.posterior_stats if M ** n_tx <= 1 << 18 else orc.posterior_stats_split
     for b in range(B):
-        mo, Ro, ko, lo = orc.posterior_stats(tb.Yd[b], tb.PsiD[b], theta[b], cons, n_tx, varn, hard=hard)
+        mo, Ro, ko, lo = stats(tb.Yd[b], tb.PsiD[b], theta[b], cons, n_tx, varn, hard=hard)
         assert np.array_equal(ks[b], ko), "hard-decision indices must be bit-exact"
         assert np.abs(m[b] - mo).max() < 1e-10 * max(1.0, np.abs(mo).max())
         assert np.abs(R[b] - Ro).max() < 1e-10 * max(1.0, np.abs(Ro).max())
@@ -138,16 +144,38 @@ MSTEP_CASES = [(8, 2, 2, 4, 12, 30), (32, 2, 2, 4, 40, 50), (6, 1, 4, 16, 8, 20)
                (12, 8, 8, 16, 60, 120),
                # long channels: n_tx = 4 beyond the fixed-chunk Gram kernel (N = 256), and a solution vector
                # that no longer fits in shared memory (L = 1288, n_rx = 8 -> global scratch)
-               (256, 4, 2, 4, 600, 800), (256, 2, 2, 4, 300, 400), (160, 8, 8, 4, 800, 900)]
+               (256, 4, 2, 4, 600, 800), (256, 2, 2, 4, 300, 400), (160, 8, 8, 4, 800, 900),
+               # random Hermitian PD statistics ("pd": no enumeration).  n_tx = 1, L = N + 1 = 2..17: every
+               # residue of L mod 16 of the blocked Cholesky, incl. n_rx = 1 (three zero rows under the matrix)
+               *[(N, 1, (1, 2, 3, 4, 6, 8)[N % 6], 4, 3, 2 * N + 4, "pd") for N in range(1, 17)],
+               # block lengths 1, 15, 16, 17, 64, 65 (ragged chunk, one stage, ring wrap-around) on the scalar,
+               # TMA (n_tx = 4, N <= 143) and generic Gram
+               *[(N, n_tx, 3, 4, T_p, T_d, "pd") for N, n_tx in ((20, 2), (10, 4), (6, 6))
+                 for T_p, T_d in ((1, 65), (65, 1), (15, 64), (64, 15), (16, 17), (17, 16))],
+               # n_tx = 4 on both sides of the TMA / generic Gram switch
+               (143, 4, 2, 4, 64, 300, "pd"), (144, 4, 2, 4, 64, 300, "pd"),
+               # n_rx = 8, Lp = 48 / 56: the solution vector on both sides of the shared / global scratch switch
+               (5, 8, 8, 4, 16, 20, "pd"), (6, 8, 8, 4, 16, 20, "pd")]
+
+
+def random_pd_stats(rng, B, T, n_tx):
+    """Per-symbol statistics m (random) and R = (A + A^H)/2 + c I (exactly Hermitian, positive definite)."""
+    A = rng.standard_normal((B, T, n_tx, n_tx)) + 1j * rng.standard_normal((B, T, n_tx, n_tx))
+    R = 0.5 * (A + A.conj().transpose(0, 1, 3, 2))
+    R += (np.linalg.norm(A, ord=2, axis=(2, 3)) + 0.5)[:, :, None, None] * np.eye(n_tx)
+    m = rng.standard_normal((B, T, n_tx)) + 1j * rng.standard_normal((B, T, n_tx))
+    return m, R
 
 
 @pytest.mark.parametrize("case", MSTEP_CASES)
 def test_mstep_matches_oracle(S, orc, case):
     import torch
 
-    N, n_tx, n_rx, M, T_p, T_d = case
+    N, n_tx, n_rx, M, T_p, T_d, *kind = case
     B = 2
     tb = S.signal_model.generate_batch(N, n_tx, n_rx, M, T_p, T_d, 0.1, B, seed=5, legacy=False)
+    if kind == ["pd"]:   # random pilot phases: the pilot block observes every RIS element, even when T_d = 1
+        tb.PsiP[:] = np.exp(2j * np.pi * np.random.default_rng(N + T_p).random(tb.PsiP.shape))
     cons = orc.qam_constellation(M)
     # (the M-step does not depend on the mode; 8 streams of 16-QAM only exist in the partitioned modes)
     prob = S.Problem(N=N, n_tx=n_tx, n_rx=n_rx, M=M, T_p=T_p, T_d=T_d, itera=1,
@@ -157,7 +185,10 @@ def test_mstep_matches_oracle(S, orc, case):
     sm = np.empty((B, T_d, n_tx), np.complex128)
     sR = np.empty((B, T_d, n_tx, n_tx), np.complex128)
     for b in range(B):
-        if M ** n_tx <= 4096 or (n_tx > 4 and N < 10 and M == 4):
+        if kind == ["pd"]:
+            m_, R_ = random_pd_stats(np.random.default_rng(N * 100 + T_d + b), 1, T_d, n_tx)
+            sm[b], sR[b] = m_[0], R_[0]
+        elif M ** n_tx <= 4096 or (n_tx > 4 and N < 10 and M == 4):
             sm[b], sR[b], _, _ = orc.posterior_stats(tb.Yd[b], tb.PsiD[b], 0.7 * tb.h[b], cons, n_tx, 2.0)
         else:
             sm[b], sR[b] = orc.pilot_stats(tb.Xd[b])
@@ -400,6 +431,8 @@ BATCH_CASES = [
     (16, 4, 4, 4, 160, 72, 3, 0.3, "hard"),
     (20, 4, 4, 16, 100, 96, 2, 0.2, "soft"),
     (24, 3, 4, 4, 144, 90, 3, 0.3, "soft"),
+    (16, 1, 1, 16, 16, 60, 4, 0.1, "soft"),      # one receive antenna (three zero rows under the Cholesky factor)
+    (10, 3, 3, 64, 24, 30, 2, 0.3, "soft"),      # 3 streams of 64-QAM (K = 2^18)
 ]
 
 
