@@ -104,7 +104,8 @@ typedef struct sbce_cfg {
     int32_t batch;        /* trials B in this call                                             */
     int32_t mode;         /* SBCE_MODE_*                                                       */
     uint32_t flags;       /* SBCE_FLAG_*                                                       */
-    int32_t partition_p1; /* PM modes: p+1 = streams enumerated exhaustively (PM.py:74-75)     */
+    int32_t partition_p1; /* PM modes: p+1 = streams enumerated exhaustively (PM.py:74-75);
+                             M^(p+1) candidates per symbol, at most 2^24 (p1*log2(M) <= 24)    */
     int32_t reserved[5];
 } sbce_cfg;
 
@@ -161,7 +162,8 @@ int sbce_host_split_threshold(void);
 /* Stand-alone E-step sweep (posterior statistics at a given theta), device
  * pointers.  stat_m [B][T_d][n_tx], stat_R [B][T_d][n_tx][n_tx] complex128,
  * kstar [B][T_d] int32 (nullable), lse_sym [B][T_d] float64 (nullable).
- * Uses cfg->mode (SOFT/HARD/PM/PM_BETA) exactly as the EM loop does. */
+ * Uses cfg->mode exactly as the EM loop does; as there, kstar is -1 in the PM / PM_BETA
+ * modes and lse_sym is NaN in the PM, PM_BETA, ZF and MMSE modes. */
 int sbce_estep(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* stat_m,
                double* stat_R, int32_t* kstar, double* lse_sym, void* workspace,
                size_t workspace_bytes, void* stream);

@@ -508,6 +508,125 @@ def pm_stats(Yd, PsiD, Theta, cons, n_tx, varn, partition_r, weighted, quirks=Tr
     return m, R
 
 
+def _boundary_margin(z, sqM):
+    """Smallest distance of the real and imaginary parts of z to a decision boundary of the per-axis slicer
+    (levels at the odd integers -sqM+1..sqM-1, boundaries at the even integers between them)."""
+    bounds = np.arange(-sqM + 2, sqM - 1, 2, dtype=np.float64)
+    v = np.concatenate([np.ravel(np.real(z)), np.ravel(np.imag(z))])
+    if v.size == 0:
+        return math.inf
+    return float(np.abs(v[:, None] - bounds[None, :]).min())
+
+
+def _order_trace(channel):
+    """Stream order of `Proposed method/PM.py:65-70` and, over its rounds, the smallest relative gap between the
+    largest and second-largest diag(pinv(A^H A)) (the arg-max decision of the round)."""
+    n_tx = channel.shape[1]
+    j, j_c, arr, gap = [], list(range(n_tx)), channel, math.inf
+    for _ in range(n_tx):
+        yeta = np.diag(np.linalg.pinv(arr.conj().T @ arr))
+        k = _argmax_complex_first(yeta)
+        if len(yeta) > 1:
+            s = np.sort(yeta.real)
+            gap = min(gap, float((s[-1] - s[-2]) / abs(s[-1])))
+        j.append(j_c[k])
+        arr = np.delete(arr, k, axis=1)
+        del j_c[k]
+    return j, gap
+
+
+def _fsum_c(v):
+    return complex(math.fsum(np.real(v)), math.fsum(np.imag(v)))
+
+
+def pm_stats_trace(Yd, PsiD, Theta, cons, n_tx, varn, p1, weighted, quirks=True):
+    """pm_stats (p1 = p+1 streams enumerated) with a per-symbol trace for kernel tests.  Returns (m, R, trace);
+    trace[t] holds the stream `order`, the candidate list `cands` (as the statistics use it), the `weights`
+    (normalised for PM-beta, 1 for PM), and the margins of every discrete decision on the way:
+        order_gap  relative gap between the largest and second-largest diag(pinv(A^H A)) of each ordering round
+        slice_gap  smallest distance of a zero-forced value z of set B to a decision boundary of its axis
+    m_t and R_t are summed exactly (math.fsum) over weights normalised in long double."""
+    T_d, N1 = PsiD.shape
+    N = N1 - 1
+    n_rx = Yd.shape[1]
+    M = len(cons)
+    sqM = int(round(math.sqrt(M)))
+    Th = Theta.reshape(N1, n_tx, n_rx)
+    Heff = effective_channels(PsiD, Theta, n_tx)
+    tabA = hypothesis_table(cons, p1)
+    nB = n_tx - p1
+    m = np.zeros((T_d, n_tx), dtype=np.complex128)
+    R = np.zeros((T_d, n_tx, n_tx), dtype=np.complex128)
+    trace = []
+    for t in range(T_d):
+        chan = Th[0].T + np.einsum("n,njr->rj", PsiD[t, :N], Th[1:]) if quirks else Heff[t]
+        order, order_gap = _order_trace(chan)
+        cands = np.empty((len(tabA), n_tx), dtype=np.complex128)
+        cands[:, :p1] = tabA
+        slice_gap = math.inf
+        if nB > 0:
+            A, Bc = chan[:, order[:p1]], chan[:, order[p1:]]
+            z = (np.linalg.inv(Bc.conj().T @ Bc) @ Bc.conj().T @ (Yd[t][:, None] - A @ tabA.T)).T   # (K, nB)
+            slice_gap = _boundary_margin(z, sqM)
+            cands[:, p1:] = cons[np.argmin(np.abs(z[:, :, None] - cons[None, None, :]) ** 2, axis=2)]
+        if not quirks:
+            fixed = np.empty_like(cands)
+            fixed[:, order] = cands
+            cands = fixed
+        if weighted:
+            res = Yd[t][None, :] - cands @ Heff[t].T
+            d2 = (res.real ** 2 + res.imag ** 2).sum(axis=1)
+            e = np.exp(-(d2 - d2.min()).astype(np.longdouble) / np.longdouble(varn) ** 2)
+            w = (e / e.sum()).astype(np.float64)
+        else:
+            w = np.ones(len(cands))
+        for i in range(n_tx):
+            m[t, i] = _fsum_c(w * cands[:, i].conj())
+            for k in range(n_tx):
+                R[t, i, k] = _fsum_c(w * cands[:, i].conj() * cands[:, k])
+        trace.append(dict(order=order, cands=cands, weights=w, order_gap=order_gap, slice_gap=slice_gap))
+    return m, R, trace
+
+
+def detector_stats_trace(Yd, PsiD, Theta, cons, n_tx, varn, kind, quirks=True):
+    """detector_stats with the decisions and their margins, for kernel tests.  Returns (m, R, kstar, trace);
+    kstar[t] is the joint hypothesis index of the decision, trace[t] holds the estimate `est` (ZF: pinv(H) y in
+    float64; MMSE: inv(H^H H + varn^2 I) H^H y) and
+        slice_gap  proper slicer (quirks off): smallest distance of est to a decision boundary of its axis
+        pair_gap   as-coded slicer (quirks on): gap between the best and second-best (stream, point) distance."""
+    T_d, N1 = PsiD.shape
+    N = N1 - 1
+    n_rx = Yd.shape[1]
+    M = len(cons)
+    sqM = int(round(math.sqrt(M)))
+    Th = Theta.reshape(N1, n_tx, n_rx)
+    Heff = effective_channels(PsiD, Theta, n_tx)
+    m = np.zeros((T_d, n_tx), dtype=np.complex128)
+    R = np.zeros((T_d, n_tx, n_tx), dtype=np.complex128)
+    kstar = np.zeros(T_d, dtype=np.int64)
+    trace = []
+    for t in range(T_d):
+        chan = Th[0].T + np.einsum("n,njr->rj", PsiD[t, :N], Th[1:]) if quirks else Heff[t]
+        if kind == "zf":
+            est = np.linalg.pinv(chan) @ Yd[t]
+        else:
+            est = np.linalg.inv(chan.conj().T @ chan + (varn ** 2) * np.eye(n_tx)) @ chan.conj().T @ Yd[t]
+        tr = dict(est=est, slice_gap=math.inf, pair_gap=math.inf)
+        if quirks:
+            dig = slicer_as_coded(est, cons, n_tx)
+            dist = np.sort(np.abs(est.reshape(-1, 1) - cons.reshape(1, -1)).ravel())
+            tr["pair_gap"] = float(dist[1] - dist[0]) if dist.size > 1 else math.inf
+        else:
+            dig = np.array([int(np.argmin(np.abs(est[j] - cons) ** 2)) for j in range(n_tx)])
+            tr["slice_gap"] = _boundary_margin(est, sqM)
+        kstar[t] = int(sum(int(dig[j]) * M ** (n_tx - 1 - j) for j in range(n_tx)))
+        x = cons[dig]
+        m[t] = x.conj()
+        R[t] = x.conj()[:, None] * x[None, :]
+        trace.append(tr)
+    return m, R, kstar, trace
+
+
 def em_pm(Yd, Yp, PsiD, PsiP, Xp, M, varn, itera, theta0, h_true=None, partition_r=0,
           weighted=False, genie_stop=True, quirks=True, how=None, return_trace=False):
     """Partitioned EM: `Proposed method/PM.py:47-116` (weighted=False, lstsq) and

@@ -82,6 +82,8 @@ static int make_dims(const sbce_cfg* c, Dims* d, bool with_estep = true) {
     d->rec = qr_record_doubles(c->n_tx);
     if (c->mode == SBCE_MODE_PM || c->mode == SBCE_MODE_PM_BETA) {
         if (c->partition_p1 < 1 || c->partition_p1 > c->n_tx) return SBCE_E_SHAPE;
+        // M^p1 candidates per symbol (an int in k_pm_stats): the same 2^24 bound as the exhaustive tree
+        if (with_estep && c->partition_p1 * d->bitsM > 24) return SBCE_E_UNSUPPORTED;
     }
     if (c->mode >= SBCE_MODE_PM && c->n_rx < c->n_tx) return SBCE_E_UNSUPPORTED;
     if (c->flags & SBCE_FLAG_SUPERIMPOSED) {
@@ -240,7 +242,7 @@ const char* sbce_error_string(int code) {
         case 0: return "ok";
         case SBCE_E_NULL: return "required pointer is null";
         case SBCE_E_SHAPE: return "invalid shape parameter";
-        case SBCE_E_UNSUPPORTED: return "unsupported configuration (n_tx,n_rx<=8; n_tx<=4: n_rx in {1,2,3,4,6,8}; M in {4,16,64}; N+1+n_tx^2<=908; exhaustive modes with n_tx>4 need n_tx*log2(M)<=24)";
+        case SBCE_E_UNSUPPORTED: return "unsupported configuration (n_tx,n_rx<=8; n_tx<=4: n_rx in {1,2,3,4,6,8}; M in {4,16,64}; N+1+n_tx^2<=908; exhaustive modes with n_tx>4 need n_tx*log2(M)<=24; PM modes need partition_p1*log2(M)<=24)";
         case SBCE_E_WORKSPACE: return "workspace too small for one trial";
         case SBCE_E_NODEVICE: return "no CUDA device";
         default: return code > 0 ? cudaGetErrorString((cudaError_t)code) : "unknown error";
@@ -311,12 +313,18 @@ int sbce_estep(const sbce_cfg* cfg, const sbce_io* io, const double* theta, doub
     const int chunk = trials_fitting(d, workspace_bytes, cfg->batch);
     if (chunk < 1) return SBCE_E_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
+    // as in em_chunk: the modes that take no joint decision return kstar = -1 and the modes that never form the
+    // log-sum return lse_sym = NaN (all-ones bytes), not whatever the caller's buffers held
+    const bool tree = d.mode == SBCE_MODE_SOFT || d.mode == SBCE_MODE_HARD;
+    const bool decides = tree || d.mode == SBCE_MODE_ZF || d.mode == SBCE_MODE_MMSE;
     for (int b0 = 0; b0 < cfg->batch; b0 += chunk) {
         const int nb = (cfg->batch - b0 < chunk) ? cfg->batch - b0 : chunk;
         Workspace ws;
         carve_workspace(d, nb, workspace, &ws);
         sbce_io o = offset_io(d, *io, (size_t)b0);
         const size_t sb = (size_t)b0 * d.T_d;
+        if (kstar && !decides) CK(cudaMemsetAsync(kstar + sb, 0xFF, (size_t)nb * d.T_d * sizeof(int32_t), s));
+        if (lse_sym && !tree) CK(cudaMemsetAsync(lse_sym + sb, 0xFF, (size_t)nb * d.T_d * sizeof(double), s));
         rc = estep_dispatch(d, nb, o.Yd, o.PsiD, theta + (size_t)b0 * d.L * d.n_rx * 2, o.varn, nullptr, ws,
                             stat_m + sb * d.n_tx * 2, stat_R + sb * d.n_tx * d.n_tx * 2, kstar ? kstar + sb : nullptr,
                             lse_sym ? lse_sym + sb : nullptr, (d.flags & SBCE_FLAG_SUPERIMPOSED) ? o.Xp : nullptr, s);

@@ -84,11 +84,52 @@ __device__ int slice_qam(cplx z, int sqM, int hb) {
     return (bq << hb) | bi;
 }
 
+// x = pinv(H) y for an n_rx x n_tx channel of full column rank (n_rx >= n_tx) through a Householder QR of H:
+// R x = (Q^H y)[:n_tx].  Normal equations would square cond(H) and lose the last pivot near cond 1e8.
+// A and w are overwritten (the factors and Q^H y).
 template <int PM_MAXT>
-__global__ void __launch_bounds__(128) k_pm_stats(Dims d, const cplx* __restrict__ Yd, const cplx* __restrict__ PsiD,
-                                                  const cplx* __restrict__ theta, const double* __restrict__ varn,
-                                                  const int32_t* __restrict__ active, cplx* __restrict__ stat_m,
-                                                  cplx* __restrict__ stat_R, int32_t* __restrict__ kstar) {
+__device__ void zf_solve_qr(cplx (*A)[PM_MAXT], cplx* w, int n_rx, int n_tx, cplx* est) {
+    for (int c = 0; c < n_tx; ++c) {
+        // reflector v = x - alpha e_0 with alpha = -e^{i arg x_0} ||x||, x = A[c:, c]; P = I - v v^H / (v^H x)
+        double nx = 0.0;
+        for (int r = c; r < n_rx; ++r) nx += cnorm2(A[r][c]);
+        nx = sqrt(nx);
+        const double a0 = sqrt(cnorm2(A[c][c]));
+        const cplx ph = a0 > 0.0 ? cscale(A[c][c], 1.0 / a0) : mk(1.0, 0.0);
+        const cplx alpha = cscale(ph, -nx);
+        const double vx = nx * (nx + a0);     // v^H x, real and >= 0
+        if (vx > 0.0) {
+            A[c][c] = csub(A[c][c], alpha);   // column c now holds v
+            for (int j = c + 1; j < n_tx; ++j) {
+                cplx s = mk(0, 0);
+                for (int r = c; r < n_rx; ++r) cfmac(s, A[r][j], A[r][c]);  // v^H A[c:, j]
+                s = cscale(s, 1.0 / vx);
+                for (int r = c; r < n_rx; ++r) { const cplx u = cmul(A[r][c], s); A[r][j] = csub(A[r][j], u); }
+            }
+            cplx s = mk(0, 0);
+            for (int r = c; r < n_rx; ++r) cfmac(s, w[r], A[r][c]);          // v^H w[c:]
+            s = cscale(s, 1.0 / vx);
+            for (int r = c; r < n_rx; ++r) { const cplx u = cmul(A[r][c], s); w[r] = csub(w[r], u); }
+        }
+        A[c][c] = alpha;
+    }
+    for (int a = n_tx - 1; a >= 0; --a) {
+        cplx v = w[a];
+        for (int q = a + 1; q < n_tx; ++q) { cplx nv = cmul(A[a][q], est[q]); v = csub(v, nv); }
+        // a zero column (theta = 0 gives H = 0) contributes 0, as pinv(0) = 0 does
+        const double dn = cnorm2(A[a][a]);
+        est[a] = dn > 0.0 ? cscale(cmulc(v, A[a][a]), 1.0 / dn) : mk(0, 0);
+    }
+}
+
+// Body of k_pm_stats (DET = false: PM, PM-beta) and k_det_stats (DET = true: ZF, MMSE).  Two kernels, so that the
+// detector solve does not change the register allocation of the candidate loop.  Both are bounded to 7 CTAs of 128
+// threads per SM (at most 72 registers): left to itself ptxas settles on 64 registers and spills.
+template <int PM_MAXT, bool DET>
+__device__ __forceinline__ void pm_stats_body(const Dims& d, const cplx* __restrict__ Yd, const cplx* __restrict__ PsiD,
+                                              const cplx* __restrict__ theta, const double* __restrict__ varn,
+                                              const int32_t* __restrict__ active, cplx* __restrict__ stat_m,
+                                              cplx* __restrict__ stat_R, int32_t* __restrict__ kstar) {
     const int b = blockIdx.y;
     if (active != nullptr && active[b] == 0) return;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -125,33 +166,39 @@ __global__ void __launch_bounds__(128) k_pm_stats(Dims d, const cplx* __restrict
     cplx y[PM_MAXR];
     for (int r = 0; r < n_rx; ++r) y[r] = Yd[((size_t)b * d.T_d + t) * n_rx + r];
 
-    if (d.mode == SBCE_MODE_ZF || d.mode == SBCE_MODE_MMSE) {
-        // ---- detector-driven EM (em_zf / em_mmse, PMvsMLvsZFvsMMSE.py:54-133): x = (H^H H [+ varn^2 I])^-1 H^H y,
-        // sliced to one hypothesis, rank-one statistics.  Every lane computes the same tiny solve.
-        cplx Gm[PM_MAXT][PM_MAXT], est[PM_MAXT];
-        const double reg = (d.mode == SBCE_MODE_MMSE) ? varn[b] * varn[b] : 0.0;
-        for (int a = 0; a < n_tx; ++a)
-            for (int c = 0; c <= a; ++c) {
+    if constexpr (DET) {
+        // ---- detector-driven EM (em_zf / em_mmse, PMvsMLvsZFvsMMSE.py:54-133): x = pinv(H) y (ZF) or
+        // (H^H H + varn^2 I)^-1 H^H y (MMSE), sliced to one hypothesis, rank-one statistics.  Every lane computes
+        // the same tiny solve.
+        cplx est[PM_MAXT];
+        if (d.mode == SBCE_MODE_ZF) {
+            zf_solve_qr(Hc, y, n_rx, n_tx, est);   // last use of Hc and y: factored in place
+        } else {
+            cplx Gm[PM_MAXT][PM_MAXT];
+            const double reg = varn[b] * varn[b];
+            for (int a = 0; a < n_tx; ++a)
+                for (int c = 0; c <= a; ++c) {
+                    cplx sacc = mk(0, 0);
+                    for (int r = 0; r < n_rx; ++r) cfmac(sacc, Hc[r][c], Hc[r][a]);
+                    if (a == c) sacc.x += reg;
+                    Gm[a][c] = sacc;
+                }
+            small_chol(Gm, n_tx);
+            for (int a = 0; a < n_tx; ++a) {
                 cplx sacc = mk(0, 0);
-                for (int r = 0; r < n_rx; ++r) cfmac(sacc, Hc[r][c], Hc[r][a]);
-                if (a == c) sacc.x += reg;
-                Gm[a][c] = sacc;
+                for (int r = 0; r < n_rx; ++r) cfmac(sacc, y[r], Hc[r][a]);
+                est[a] = sacc;
             }
-        small_chol(Gm, n_tx);
-        for (int a = 0; a < n_tx; ++a) {
-            cplx sacc = mk(0, 0);
-            for (int r = 0; r < n_rx; ++r) cfmac(sacc, y[r], Hc[r][a]);
-            est[a] = sacc;
-        }
-        for (int a = 0; a < n_tx; ++a) {
-            cplx v = est[a];
-            for (int q = 0; q < a; ++q) { cplx nv = cmul(Gm[a][q], est[q]); v = csub(v, nv); }
-            est[a] = cscale(v, 1.0 / Gm[a][a].x);
-        }
-        for (int a = n_tx - 1; a >= 0; --a) {
-            cplx v = est[a];
-            for (int q = a + 1; q < n_tx; ++q) cfmsc(v, est[q], Gm[q][a]);
-            est[a] = cscale(v, 1.0 / Gm[a][a].x);
+            for (int a = 0; a < n_tx; ++a) {
+                cplx v = est[a];
+                for (int q = 0; q < a; ++q) { cplx nv = cmul(Gm[a][q], est[q]); v = csub(v, nv); }
+                est[a] = cscale(v, 1.0 / Gm[a][a].x);
+            }
+            for (int a = n_tx - 1; a >= 0; --a) {
+                cplx v = est[a];
+                for (int q = a + 1; q < n_tx; ++q) cfmsc(v, est[q], Gm[q][a]);
+                est[a] = cscale(v, 1.0 / Gm[a][a].x);
+            }
         }
         int k = 0;
         if (quirks) {
@@ -327,17 +374,36 @@ __global__ void __launch_bounds__(128) k_pm_stats(Dims d, const cplx* __restrict
     }
 }
 
+template <int PM_MAXT>
+__global__ void __launch_bounds__(128, 7) k_pm_stats(Dims d, const cplx* __restrict__ Yd, const cplx* __restrict__ PsiD,
+                                                  const cplx* __restrict__ theta, const double* __restrict__ varn,
+                                                  const int32_t* __restrict__ active, cplx* __restrict__ stat_m,
+                                                  cplx* __restrict__ stat_R) {
+    pm_stats_body<PM_MAXT, false>(d, Yd, PsiD, theta, varn, active, stat_m, stat_R, nullptr);
+}
+
+template <int PM_MAXT>
+__global__ void __launch_bounds__(128, 7) k_det_stats(Dims d, const cplx* __restrict__ Yd, const cplx* __restrict__ PsiD,
+                                                   const cplx* __restrict__ theta, const double* __restrict__ varn,
+                                                   const int32_t* __restrict__ active, cplx* __restrict__ stat_m,
+                                                   cplx* __restrict__ stat_R, int32_t* __restrict__ kstar) {
+    pm_stats_body<PM_MAXT, true>(d, Yd, PsiD, theta, varn, active, stat_m, stat_R, kstar);
+}
+
 cudaError_t launch_pm_stats(const Dims& d, int nb, const double* Yd, const double* PsiD, const double* theta,
                             const double* varn, const int32_t* active, double* stat_m, double* stat_R,
                             int32_t* kstar, cudaStream_t s) {
     if (d.n_tx > 8 || d.n_rx > PM_MAXR) return cudaErrorInvalidValue;
     dim3 grid((d.T_d + 3) / 4, nb);
-    if (d.n_tx <= 4)
-        k_pm_stats<4><<<grid, 128, 0, s>>>(d, (const cplx*)Yd, (const cplx*)PsiD, (const cplx*)theta, varn, active,
-                                           (cplx*)stat_m, (cplx*)stat_R, kstar);
-    else
-        k_pm_stats<8><<<grid, 128, 0, s>>>(d, (const cplx*)Yd, (const cplx*)PsiD, (const cplx*)theta, varn, active,
-                                           (cplx*)stat_m, (cplx*)stat_R, kstar);
+    const cplx *y = (const cplx*)Yd, *psi = (const cplx*)PsiD, *th = (const cplx*)theta;
+    cplx *m = (cplx*)stat_m, *R = (cplx*)stat_R;
+    if (d.mode == SBCE_MODE_ZF || d.mode == SBCE_MODE_MMSE) {
+        if (d.n_tx <= 4) k_det_stats<4><<<grid, 128, 0, s>>>(d, y, psi, th, varn, active, m, R, kstar);
+        else k_det_stats<8><<<grid, 128, 0, s>>>(d, y, psi, th, varn, active, m, R, kstar);
+    } else {
+        if (d.n_tx <= 4) k_pm_stats<4><<<grid, 128, 0, s>>>(d, y, psi, th, varn, active, m, R);
+        else k_pm_stats<8><<<grid, 128, 0, s>>>(d, y, psi, th, varn, active, m, R);
+    }
     count_launch();
     return cudaGetLastError();
 }

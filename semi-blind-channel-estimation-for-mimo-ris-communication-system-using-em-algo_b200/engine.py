@@ -291,8 +291,10 @@ class DeviceSession:
             _lib.check(self.lib.sbce_em_batch(C.byref(cfg), C.byref(io), self.ws.data_ptr(), self.ws_bytes, stream))
         return out
 
-    def estep(self, Yd, PsiD, theta, varn, Xp=None):
-        """Stand-alone E-step sweep at `theta` -> (m, R, kstar, lse_sym) device tensors.
+    def estep(self, Yd, PsiD, theta, varn, Xp=None, out=None):
+        """Stand-alone E-step sweep at `theta` -> (m, R, kstar, lse_sym) device tensors, written into
+        `out` = (m, R, kstar, lse_sym) when given.  kstar is -1 in the PM modes and lse_sym NaN in the PM, ZF
+        and MMSE modes, whatever the buffers held.
         With Problem.superimposed the per-symbol pilot offsets Xp [B][T_d][n_tx] are required."""
         torch, p = self.torch, self.prob
         B = int(Yd.shape[0])
@@ -300,10 +302,12 @@ class DeviceSession:
             raise ValueError("superimposed pilots: estep() needs the offsets Xp [B][T_d][n_tx]")
         io = self._io(B, Yd, None, PsiD, None, Xp if p.superimposed else None, varn, None, None, None)
         dev = self.device
-        m = torch.empty((B, p.T_d, p.n_tx), dtype=torch.complex128, device=dev)
-        R = torch.empty((B, p.T_d, p.n_tx, p.n_tx), dtype=torch.complex128, device=dev)
-        ks = torch.empty((B, p.T_d), dtype=torch.int32, device=dev)
-        ls = torch.empty((B, p.T_d), dtype=torch.float64, device=dev)
+        shapes = ((B, p.T_d, p.n_tx), (B, p.T_d, p.n_tx, p.n_tx), (B, p.T_d), (B, p.T_d))
+        dtypes = (torch.complex128, torch.complex128, torch.int32, torch.float64)
+        if out is None:
+            out = [torch.empty(sh, dtype=dt, device=dev) for sh, dt in zip(shapes, dtypes)]
+        m, R, ks, ls = (self._check(o, sh, name, dt)
+                        for o, sh, name, dt in zip(out, shapes, ("m", "R", "kstar", "lse_sym"), dtypes))
         self._check(theta, (B, p.L, p.n_rx), "theta", torch.complex128)
         cfg = p.cfg(B)
         with self._on_device():

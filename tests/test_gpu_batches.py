@@ -17,7 +17,7 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
-from test_gpu_parity import BATCH_CASES, ESTEP_CASES, MSTEP_CASES, relerr  # noqa: E402
+from test_gpu_parity import BATCH_CASES, DETECTOR_CASES, ESTEP_CASES, MSTEP_CASES, PM_CASES, relerr  # noqa: E402
 
 import sbce  # noqa: E402
 
@@ -94,6 +94,12 @@ def admitted(N, n_tx, n_rx):
     return CPLX * 16 * (N + 1 + n_tx * n_tx) <= SMEM_CAP and gram_variant(N, n_tx, n_rx)[1] <= SMEM_CAP
 
 
+def pm_variant(n_tx, mode):
+    """pm.cu launch_pm_stats: k_pm_stats (PM, PM-beta) or k_det_stats (ZF, MMSE), <4> for n_tx <= 4 and <8> for the
+    wide arrays."""
+    return "%s<%d>" % ("k_det_stats" if mode in ("zf", "mmse") else "k_pm_stats", 4 if n_tx <= 4 else 8)
+
+
 def covered_items():
     """item -> list of parity-table rows that reach it."""
     items = {}
@@ -116,6 +122,10 @@ def covered_items():
         add(("enum", enum_variant(n_tx, M, mode == "hard")), ("batch", c))
         add(("gram", gram_variant(N, n_tx, n_rx)[0]), ("batch", c))
         add(("chol", chol_variant(N, n_tx, n_rx)[1]), ("batch", c))
+    for c in PM_CASES:
+        add(("pm", pm_variant(c[1], c[8])), ("pm", c))
+    for c in DETECTOR_CASES:
+        add(("pm", pm_variant(c[1], c[8])), ("detector", c))
     return items
 
 
@@ -126,6 +136,7 @@ def required_items():
     req |= {("gram", "k_gram<%d>" % n) for n in (1, 2, 3)} | {("gram", "k_gram_tma4")}
     req |= {("gram", "k_gram_mma<%d>" % n) for n in range(4, 9)}
     req |= {("chol", "smem"), ("chol", "global")}
+    req |= {("pm", pm_variant(n, mode)) for n in (4, 8) for mode in ("pm", "zf")}
     return req
 
 
@@ -225,6 +236,23 @@ def test_mstep_launches_the_mirrored_kernels(S, orc, case):
     gram = [n for n in names if "k_gram" in n]
     assert gram and all(_pattern(gram_variant(N, n_tx, n_rx)[0]).search(n) for n in gram), names
     assert any("k_chol_solve" in n for n in names), names
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n_tx,mode", [(3, "pm_beta"), (6, "pm"), (2, "zf"), (6, "mmse")])
+def test_pm_estep_launches_the_mirrored_kernel(S, n_tx, mode):
+    import torch
+
+    N, n_rx, M, T_d = 6, n_tx, 4, 9
+    tb = S.signal_model.generate_batch(N, n_tx, n_rx, M, 4, T_d, 0.3, 1, seed=3, legacy=False)
+    ses = S.DeviceSession(S.Problem(N=N, n_tx=n_tx, n_rx=n_rx, M=M, T_p=4, T_d=T_d, itera=1, mode=mode,
+                                    partition_r=2), 1)
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(ses.device)
+    args = [t(a) for a in (tb.Yd, tb.PsiD, tb.h, tb.varn)]
+    ses.estep(*args)
+    names = _kernel_names(lambda: ses.estep(*args))
+    pm = [n for n in names if "k_pm_stats" in n or "k_det_stats" in n]
+    assert pm and all(_pattern(pm_variant(n_tx, mode)).search(n) for n in pm), names
 
 
 # ---------------------------------------------------------------------------
@@ -440,7 +468,7 @@ def test_results_do_not_depend_on_workspace_or_output_contents(S, orc, case):
         out = {}
         out["run"] = _run_device(ses, inp)
         m, R, ks, ls = ses.estep(t(inp["Yd"]), t(inp["PsiD"]), t(inp["theta0"]), t(inp["varn"]))
-        out["estep"] = [x.cpu().numpy() for x in ((m, R, ks) if prob.mode == "pm_beta" else (m, R, ks, ls))]
+        out["estep"] = [x.cpu().numpy() for x in (m, R, ks, ls)]
         out["mstep"] = [x.cpu().numpy() for x in ses.mstep(t(inp["Yd"]), t(inp["Yp"]), t(inp["PsiD"]),
                                                             t(inp["PsiP"]), t(inp["Xp"]), t(sm), t(sR))]
         out["ls"] = [x.cpu().numpy() for x in ses.ls_start(t(inp["Yp"]), t(inp["PsiP"]), t(inp["Xp"]))]
@@ -470,6 +498,16 @@ def test_results_do_not_depend_on_workspace_or_output_contents(S, orc, case):
         assert np.isnan(dirty["llf"][b, it[b]:]).all() and np.isnan(dirty["lse"][b, it[b]:]).all(), b
     if prob.mode == "pm_beta":
         assert (dirty["kstar"] == -1).all() and np.isnan(dirty["lse"]).all()
+    # the same for the stand-alone E-step: kstar = -1 and lse = NaN where the mode produces neither
+    eout = [torch.empty_like(torch.from_numpy(a)).to(dev) for a in ref["estep"]]
+    for o in eout:
+        _fill(o, "random", seed=8)
+    got = [x.cpu().numpy() for x in ses.estep(t(inp["Yd"]), t(inp["PsiD"]), t(inp["theta0"]), t(inp["varn"]),
+                                              out=eout)]
+    for i, (a, b) in enumerate(zip(ref["estep"], got)):
+        assert _same_bits(a, b), ("dirty estep outputs", i)
+    if prob.mode == "pm_beta":
+        assert (got[2] == -1).all() and np.isnan(got[3]).all()
 
 
 @pytest.mark.gpu

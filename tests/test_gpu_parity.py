@@ -562,11 +562,17 @@ def test_em_zf_mmse_golden(S, orc, name):
     assert relerr(th.reshape(g["h"].shape), g["theta_mmse_ref"]) < RTOL
 
 
-@pytest.mark.parametrize("case", [(8, 2, 2, 4, 8, 30, 3, 0.3, "zf", True), (8, 2, 2, 4, 8, 30, 3, 0.3, "mmse", True),
-                                  (8, 3, 3, 4, 8, 30, 3, 0.5, "zf", False), (6, 4, 4, 16, 6, 40, 2, 0.5, "mmse", False),
-                                  (6, 2, 4, 16, 6, 30, 3, 1.0, "zf", True), (6, 3, 4, 4, 6, 30, 3, 2.0, "mmse", True),
-                                  (6, 8, 8, 4, 16, 70, 2, 0.5, "zf", False), (6, 6, 8, 16, 6, 60, 2, 0.5, "mmse", False),
-                                  (6, 5, 6, 4, 6, 50, 2, 0.5, "mmse", True)])
+DETECTOR_CASES = [
+    # N, n_tx, n_rx, M, T_p, T_d, itera, varn, mode, quirks
+    (8, 2, 2, 4, 8, 30, 3, 0.3, "zf", True), (8, 2, 2, 4, 8, 30, 3, 0.3, "mmse", True),
+    (8, 3, 3, 4, 8, 30, 3, 0.5, "zf", False), (6, 4, 4, 16, 6, 40, 2, 0.5, "mmse", False),
+    (6, 2, 4, 16, 6, 30, 3, 1.0, "zf", True), (6, 3, 4, 4, 6, 30, 3, 2.0, "mmse", True),
+    (6, 8, 8, 4, 16, 70, 2, 0.5, "zf", False), (6, 6, 8, 16, 6, 60, 2, 0.5, "mmse", False),
+    (6, 5, 6, 4, 6, 50, 2, 0.5, "mmse", True),
+]
+
+
+@pytest.mark.parametrize("case", DETECTOR_CASES)
 def test_em_detector_batch_matches_oracle(S, orc, case):
     N, n_tx, n_rx, M, T_p, T_d, itera, varn, mode, quirks = case
     B = 4
