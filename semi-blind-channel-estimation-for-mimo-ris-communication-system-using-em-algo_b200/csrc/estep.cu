@@ -17,17 +17,19 @@
 //     reduces [Heff_t | y_t] to upper-triangular form with Householder
 //     reflections in registers (real non-negative diagonal).  Then
 //     d2(x) = c0 + sum_i | ytilde_i - sum_{j>=i} R_ij x_j |^2  exactly.
-//  2. k_enum: one WARP per data symbol walks the hypothesis tree stream
-//     n_tx-1 -> 1 with partial residuals in registers; the top levels are split
-//     across lanes, the inner levels are warp-uniform loops fed by shared-memory
-//     tables R_ij*c_m.  Because R_00 is real, the last stream separates into its
+//  2. k_enum: one HALF-WARP (16 lanes) per data symbol up to 4 streams, two
+//     symbols per warp (a whole warp per symbol for 5..8 streams), walks the
+//     hypothesis tree stream n_tx-1 -> 1 with partial residuals in registers; the
+//     top levels are split across the group's lanes, the inner levels are
+//     group-uniform loops fed by shared-memory tables R_ij*c_m.  Every collective
+//     is a group collective, so the two symbols of a warp may take different paths.  Because R_00 is real, the last stream separates into its
 //     in-phase and quadrature PAM components, so the sum over the M leaves of a
 //     node is a product of two sqrt(M)-term sums: every hypothesis is accounted
 //     for exactly, at O(1) work per node when the node's best leaf is more than
 //     64 varn^2 above the running minimum (its whole weight is < 2e-28 of the
 //     normaliser and rounds away in FP64, exactly as in the reference where
 //     float(beta) underflows).  Online max-subtracted accumulation per lane,
-//     warp-shuffle log-sum-exp merge at the end; the incomplete-data
+//     group-shuffle log-sum-exp merge at the end; the incomplete-data
 //     log-likelihood sum_k exp(-d2/varn^2) falls out of the same reduction.
 #include <math.h>
 
@@ -402,10 +404,10 @@ __global__ void __launch_bounds__(128) k_heff_qr_rows(Dims d, const cplx* __rest
 }
 
 // ---------------------------------------------------------------------------
-// 2. hypothesis-tree enumeration, one warp per symbol
+// 2. hypothesis-tree enumeration, one half-warp (n_tx <= 4) or warp per symbol
 // ---------------------------------------------------------------------------
 constexpr double SBCE_THR = 64.0;  // nodes whose best leaf is > THR*varn^2 above the incumbent weigh < e^-64
-constexpr int ENUM_QCAP = 1024;    // per-warp candidate queue (node codes)
+__device__ __forceinline__ double shfl_xor_h(unsigned hm, double v, int o) { return __shfl_xor_sync(hm, v, o); }
 
 template <int NTX, int SQM>
 struct EnumT {
@@ -413,13 +415,26 @@ struct EnumT {
     static constexpr int BITS = (SQM == 2 ? 2 : (SQM == 4 ? 4 : 6));
     static constexpr int HB = BITS / 2;
     static constexpr int NODE_STREAMS = NTX - 1;
-    static constexpr int PLWANT = (5 + BITS - 1) / BITS;  // prefix streams so that M^PL >= 32
+    static constexpr int PLWANT = (5 + BITS - 1) / BITS;  // prefix streams so that M^PL >= 32 (two rounds of 16)
     static constexpr int PL = NODE_STREAMS < PLWANT ? NODE_STREAMS : PLWANT;
     static constexpr int NPREF = 1 << (BITS * PL);
     static constexpr int NPAIR = NTX * (NTX - 1) / 2;
     static constexpr int NPAIR1 = NPAIR > 0 ? NPAIR : 1;
     static constexpr int NACC = 1 + 3 * NTX + 2 * NPAIR;  // S, m (re,im), R diag, R upper (re,im)
-    // per-warp shared block (doubles): tables, PAM levels, ytilde, c0, accumulators, aref, then ints
+    static constexpr int REC = NTX * (NTX + 1) + 2 * NTX + 2;   // qr_record_doubles(NTX)
+    // Lanes per symbol: a half-warp (two symbols per warp) up to 4 streams.  The deep trees of 5..8 streams keep
+    // a whole warp: their halves diverge at every level, one after the other (8x8 QPSK hard: 1.04 ms per launch
+    // on half-warps against 0.88 ms on warps).
+    static constexpr int G = NTX > 4 ? 32 : 16;
+    // Candidate queue (node codes) per symbol: 480 entries let eight 4x4 16-QAM blocks (7.1 KB each) share a
+    // quarter of the SM's 228 KB (4 CTAs per SM); the warp-per-symbol kernels keep 1024.
+    static constexpr int QCAP = G == 32 ? 1024 : 480;
+    // the calling lane's group (its symbol's lanes) as a member mask, and the lane's index in it
+    __device__ __forceinline__ static unsigned gmask() { return G == 32 ? 0xffffffffu : 0xFFFFu << (threadIdx.x & 16); }
+    __device__ __forceinline__ static int glane() { return threadIdx.x & (G - 1); }
+    // shift that brings the group's bits of a ballot down to bit 0
+    __device__ __forceinline__ static int gshift() { return threadIdx.x & (32 - G); }
+    // per-symbol shared block (doubles): tables, PAM levels, ytilde, c0, accumulators, aref, then ints
     static constexpr int O_TAB = 0;
     static constexpr int O_G = O_TAB + 2 * NPAIR1 * M;
     static constexpr int O_YT = O_G + NTX * SQM;
@@ -428,9 +443,17 @@ struct EnumT {
     static constexpr int O_AREF = O_ACC + NACC;
     static constexpr int O_S2 = O_AREF + 1;     // inv_s2
     static constexpr int O_CNT = O_S2 + 1;      // int counter lives in this double slot
-    static constexpr int O_Q = O_CNT + 1;       // ENUM_QCAP ints = ENUM_QCAP/2 doubles
-    static constexpr int O_SCR = O_Q + ENUM_QCAP / 2;   // [NACC][32] reduction scratch of the flush
-    static constexpr int WS_DOUBLES = ((O_SCR + NACC * 32) + 1) & ~1;
+    static constexpr int O_Q = O_CNT + 1;       // QCAP ints = QCAP/2 doubles
+    static constexpr int O_SCR = O_Q + QCAP / 2;   // [NACC][16] reduction scratch of the flush (QR record at start-up)
+    static constexpr int WS_DOUBLES = ((O_SCR + NACC * G) + 1) & ~1;
+    static_assert(NACC * G >= REC, "the QR record is staged in the flush scratch");
+    // The queue never drops a node (a dropped node is lost silently).  In the stream-1 level a group enqueues at
+    // most G*M nodes (G*SQM per row) between two maybe_flush() calls, whose threshold leaves room for them.  When every node
+    // stream is a prefix stream there is no such call, and at most one node per prefix is queued.
+    static_assert(PL < NODE_STREAMS || NPREF <= QCAP, "prefix-only trees must fit the queue without a flush");
+    static_assert(G * SQM < QCAP, "maybe_flush threshold");
+    // the top-level pre-pass votes with one lane per top symbol
+    static_assert(PL < 2 || M <= G, "pre-pass: one lane per top symbol");
 
     __device__ __forceinline__ static double pam(int a) { return (double)(2 * a - SQM + 1); }
     __device__ __forceinline__ static cplx cval(int m) { return mk(pam(m & (SQM - 1)), pam(m >> HB)); }
@@ -460,18 +483,20 @@ struct EnumT {
     }
 };
 
-// Cooperative, out-of-line processing of the queued candidate nodes of one symbol: every lane takes
-// queue entries round-robin, rebuilds the node's residuals from its code, sums its M leaves in closed
-// form (separable in-phase / quadrature PAM sums) and the warp adds the result to the shared
-// accumulators, kept relative to the reference distance `aref` (rescaled when the incumbent improves).
+// Cooperative, out-of-line processing of the queued candidate nodes of one symbol: every lane of the
+// symbol's group takes queue entries round-robin, rebuilds the node's residuals from its code, sums its
+// M leaves in closed form (separable in-phase / quadrature PAM sums) and the group adds the result to the
+// shared accumulators, kept relative to the reference distance `aref` (rescaled when the incumbent improves).
+// Only the calling group takes part: the other symbol of a warp may be anywhere else.
 template <int NTX, int SQM>
 __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
     typedef EnumT<NTX, SQM> E;
     constexpr int M = E::M;
-    const int lane = threadIdx.x & 31;
-    __syncwarp();
+    const int lane = E::glane();
+    const unsigned hm = E::gmask();
+    __syncwarp(hm);
     int* cntp = (int*)(ws + E::O_CNT);
-    const int n = min(*cntp, ENUM_QCAP);
+    const int n = min(*cntp, E::QCAP);
     const int* q = (const int*)(ws + E::O_Q);
     const cplx* tab = (const cplx*)(ws + E::O_TAB);
     const double* g = ws + E::O_G;
@@ -479,16 +504,16 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
     double aref = ws[E::O_AREF];
     if (warp_best < aref) {
         const double f = exp((warp_best - aref) * inv_s2);  // aref = +inf initially -> f = 0
-        for (int i = lane; i < E::NACC; i += 32) ws[E::O_ACC + i] *= f;
+        for (int i = lane; i < E::NACC; i += E::G) ws[E::O_ACC + i] *= f;
         aref = warp_best;
     }
     double* A = ws + E::O_ACC;
     // Narrow path.  At operating SNRs the queue almost always holds ONE node (the arg-min node, whose M leaves
-    // carry the whole posterior) or two; the general path below would run all 32 lanes through ~700
-    // instructions (9 exponentials in sequence per lane) for it.  Here the warp shares one entry: the lanes of
-    // a 2*SQM group take one PAM level of the in-phase or of the quadrature component each (one exponential
+    // carry the whole posterior) or two; the general path below would run all 16 lanes through ~700
+    // instructions (9 exponentials in sequence per lane) for it.  Here the group shares one entry: the lanes of
+    // a 2*SQM subgroup take one PAM level of the in-phase or of the quadrature component each (one exponential
     // per lane, min / sums by xor shuffles), every lane then holds the node's closed-form leaf sums and lane i
-    // adds statistic i.
+    // adds statistic i (mod 16).
     if (n <= 2) {
         constexpr int LG = (SQM == 2 ? 1 : (SQM == 4 ? 2 : 3));
         const int a = lane & (SQM - 1);
@@ -518,32 +543,32 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
             const double dd = ev * ev;
             double mn = dd;
 #pragma unroll
-            for (int o = SQM / 2; o > 0; o >>= 1) mn = fmin(mn, shfl_xor_d(mn, o));
+            for (int o = SQM / 2; o > 0; o >>= 1) mn = fmin(mn, shfl_xor_h(hm, mn, o));
             const double w = exp((mn - dd) * inv_s2);
             double s0 = w, s1 = pq * w, s2 = pq * pq * w;
 #pragma unroll
             for (int o = SQM / 2; o > 0; o >>= 1) {
-                s0 += shfl_xor_d(s0, o);
-                s1 += shfl_xor_d(s1, o);
-                s2 += shfl_xor_d(s2, o);
+                s0 += shfl_xor_h(hm, s0, o);
+                s1 += shfl_xor_h(hm, s1, o);
+                s2 += shfl_xor_h(hm, s2, o);
             }
-            const double o0 = shfl_xor_d(s0, SQM), o1 = shfl_xor_d(s1, SQM), o2 = shfl_xor_d(s2, SQM);
-            const double om = shfl_xor_d(mn, SQM);
+            const double o0 = shfl_xor_h(hm, s0, SQM), o1 = shfl_xor_h(hm, s1, SQM), o2 = shfl_xor_h(hm, s2, SQM);
+            const double om = shfl_xor_h(hm, mn, SQM);
             const double EI = isQ ? o0 : s0, A1 = isQ ? o1 : s1, A2 = isQ ? o2 : s2, minI = isQ ? om : mn;
             const double EQ = isQ ? s0 : o0, B1 = isQ ? s1 : o1, B2 = isQ ? s2 : o2, minQ = isQ ? mn : om;
             const double W = exp((aref - (base + minI + minQ)) * inv_s2);
             const double E0 = W * EI * EQ;
             const cplx F0 = mk(W * A1 * EQ, -W * EI * B1);  // sum over leaves of e * conj(x_0)
             const double Q0 = W * (A2 * EQ + EI * B2);      // sum over leaves of e * |x_0|^2
-            // statistic idx belongs to lane idx & 31: every lane picks its values out of the (warp-uniform) results
-            // with predicated register moves and then makes ONE shared-memory update per 32 statistics (as ~25
+            // statistic idx belongs to lane idx & 15: every lane picks its values out of the (group-uniform) results
+            // with predicated register moves and then makes ONE shared-memory update per 16 statistics (as ~25
             // single-lane read-modify-writes behind divergent branches this was 14 % of the kernel's stall
             // samples, profiles/r02m); per entry, so the order of the additions is unchanged
-            constexpr int NR = (E::NACC + 31) / 32;
+            constexpr int NR = (E::NACC + E::G - 1) / E::G;
             double mine[NR];
 #pragma unroll
             for (int r = 0; r < NR; ++r) mine[r] = 0.0;
-            auto add = [&](int idx, double v) { if ((idx & 31) == lane) mine[idx >> 5] = v; };
+            auto add = [&](int idx, double v) { if ((idx & (E::G - 1)) == lane) mine[idx / E::G] = v; };
             add(0, E0);
             add(1, F0.x);
             add(1 + NTX, F0.y);
@@ -568,28 +593,28 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
             }
 #pragma unroll
             for (int r = 0; r < NR; ++r)
-                if (32 * r + lane < E::NACC) A[32 * r + lane] += mine[r];
-            __syncwarp();
+                if (E::G * r + lane < E::NACC) A[E::G * r + lane] += mine[r];
+            __syncwarp(hm);
         }
         if (lane == 0) {
             ws[E::O_AREF] = aref;
             *cntp = 0;
         }
-        __syncwarp();
+        __syncwarp(hm);
         return;
     }
-    // General path: one queue entry per lane per round; the warp reduces every statistic right away (rare
+    // General path: one queue entry per lane per round; the group reduces every statistic right away (rare
     // path: keep the register footprint small so that it does not limit the occupancy of the scan loop)
     // per round every lane drops the NACC contributions of its queue entry into a shared scratch
-    // [NACC][32]; afterwards lane i sums statistic i over the lanes that held an entry (a transpose
+    // [NACC][16]; afterwards lane i sums statistic i over the lanes that held an entry (a transpose
     // instead of NACC butterfly reductions: ~25 stores + nround loads per lane, no shuffles)
     double* scr = ws + E::O_SCR;
     int nround = 0;
-    auto radd = [&](int idx, double v) { scr[idx * 32 + lane] = v; };
-    for (int e0 = 0; e0 < n; e0 += 32) {
+    auto radd = [&](int idx, double v) { scr[idx * E::G + lane] = v; };
+    for (int e0 = 0; e0 < n; e0 += E::G) {
         const int e = e0 + lane;
         const bool have = e < n;
-        nround = min(32, n - e0);
+        nround = min(E::G, n - e0);
         const int code = have ? q[e] : 0;
         cplx t0;
         double base = ws[E::O_C0];
@@ -651,20 +676,20 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
                     radd(1 + 3 * NTX + 2 * E::pair(i, s) + 1, E0 * cx.y);
                 }
         }
-        __syncwarp();
-        for (int i = lane; i < E::NACC; i += 32) {
+        __syncwarp(hm);
+        for (int i = lane; i < E::NACC; i += E::G) {
             double acc = 0.0;
-            for (int e2 = 0; e2 < nround; ++e2) acc += scr[i * 32 + e2];
+            for (int e2 = 0; e2 < nround; ++e2) acc += scr[i * E::G + e2];
             A[i] += acc;
         }
-        __syncwarp();
+        __syncwarp(hm);
     }
-    __syncwarp();
+    __syncwarp(hm);
     if (lane == 0) {
         ws[E::O_AREF] = aref;
         *cntp = 0;
     }
-    __syncwarp();
+    __syncwarp(hm);
 }
 
 template <int NTX, int SQM, bool HARD>
@@ -699,19 +724,22 @@ struct Scan {
             if (!HARD) {
                 int* cntp = (int*)(ws + E::O_CNT);
                 const int slot = atomicAdd(cntp, 1);
-                if (slot < ENUM_QCAP) ((int*)(ws + E::O_Q))[slot] = code;
+                if (slot < E::QCAP) ((int*)(ws + E::O_Q))[slot] = code;
             }
         }
     }
 
+    // PER_LANE: nodes a lane may enqueue before the next call
+    template <int PER_LANE>
     __device__ __forceinline__ void maybe_flush() {
         if (!HARD) {
-            __syncwarp();
+            const unsigned hm = E::gmask();
+            __syncwarp(hm);
             const int c = *(volatile int*)(ws + E::O_CNT);
-            if (c > ENUM_QCAP - 32 * SQM) {
+            if (c > E::QCAP - E::G * PER_LANE) {
                 double wb = best;
 #pragma unroll
-                for (int o = 16; o > 0; o >>= 1) wb = fmin(wb, shfl_xor_d(wb, o));
+                for (int o = E::G / 2; o > 0; o >>= 1) wb = fmin(wb, shfl_xor_h(hm, wb, o));
                 enum_flush<NTX, SQM>(ws, wb);
             }
         }
@@ -720,18 +748,20 @@ struct Scan {
     // Branch and bound.  Every leaf below a node has d2 >= the node's partial distance `base`; once
     // base > lim (incumbent + 64 varn^2) none of them can improve the arg-min or pass the enqueue test,
     // so the subtree is "dead": visiting it would change nothing.  Lanes carry a dead flag instead of
-    // returning (the loops contain warp collectives and must stay convergent); a row or subtree is
-    // skipped only when a warp vote says it is dead for all 32 lanes.
+    // returning (the loops contain group collectives and must stay convergent within the group); a row
+    // or subtree is skipped only when a vote of the group says it is dead for all its lanes.
 
-    // streams S_ ... 1 enumerated with warp-uniform loops
+    // streams S_ ... 1 enumerated with group-uniform loops
     template <int S_>
     __device__ __forceinline__ void inner(const cplx (&acc)[NTX], double base, int code, cplx r01, bool dead) {
         dead = dead || (prune && base > lim);
         if constexpr (S_ == 0) {
             if (!dead) leaf(acc[0], base, code);
         } else if constexpr (S_ == 1) {
-            if (__all_sync(0xffffffffu, dead)) return;
-            // innermost node level: |u_1|^2 and R_01 x_1 are separable in the in-phase / quadrature indices
+            if (__all_sync(E::gmask(), dead)) return;
+            // innermost node level: |u_1|^2 and R_01 x_1 are separable in the in-phase / quadrature indices.
+            // The queue is checked once per node (its M leaves per lane) when that fits, else once per row of SQM.
+            constexpr bool NODE_FLUSH = E::G * M < E::QCAP;
             const double* g1 = g + SQM;
             double dI1[SQM];
 #pragma unroll
@@ -746,7 +776,7 @@ struct Scan {
                 const double eQ = acc[1].y - g1[iQ];
                 const double bq = base + __dmul_rn(eQ, eQ);
                 const bool deadq = dead || (prune && bq > lim);
-                if (__all_sync(0xffffffffu, deadq)) continue;
+                if (__all_sync(E::gmask(), deadq)) continue;
                 const double pQ = E::pam(iQ);
                 // t = acc0 - pQ * (i r01) = acc0 - pQ*(-r01.y + i r01.x)
                 const cplx tq = mk(fma(pQ, r01.y, acc[0].x), fma(-pQ, r01.x, acc[0].y));
@@ -759,10 +789,11 @@ struct Scan {
                         leaf(t0, bq + dI1[iI], cq + (iI << (E::BITS * (NTX - 2))));
                     }
                 }
-                maybe_flush();
+                if (!NODE_FLUSH) maybe_flush<SQM>();
             }
+            if (NODE_FLUSH) maybe_flush<M>();
         } else {
-            if (__all_sync(0xffffffffu, dead)) return;
+            if (__all_sync(E::gmask(), dead)) return;
 #pragma unroll 1
             for (int m = 0; m < M; ++m) {
                 const double* gs = g + S_ * SQM;
@@ -796,6 +827,12 @@ struct Scan {
     }
 };
 
+// Up to 4 streams, two symbols per warp, one per half-warp (E::G = 16): symbol t = 2 (global warp index) + sub,
+// `gl` = lane within the group.  Every phase of a symbol (start-up, prefix rounds, both flush paths, incumbent
+// merge, outputs) fits in 16 lanes, so a warp keeps twice the symbols in flight with the same registers per
+// thread (4x4 16-QAM: 0.949 -> 0.809 ms per launch).  The halves run independently: they may have different
+// live rounds, take different flush paths or collapse; a half without a symbol (odd T_d) leaves at once.
+// 5..8 streams: one symbol per warp (E::G = 32), same code.
 // (4 CTAs per SM at 128 registers with a few spilled words beat 3 CTAs at 140 registers without: 1.16 vs 1.22 ms)
 template <int NTX, int SQM, bool HARD, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, const double* __restrict__ qr,
@@ -805,30 +842,31 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
                                                      double* __restrict__ lse_sym) {
     typedef EnumT<NTX, SQM> E;
     constexpr int M = E::M;
-    extern __shared__ __align__(16) double enum_smem[];   // [WARPS][E::WS_DOUBLES]
+    extern __shared__ __align__(16) double enum_smem[];   // [SPW WARPS][E::WS_DOUBLES]
     const int b = blockIdx.y;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int t = blockIdx.x * WARPS + warp;
+    constexpr int SPW = 32 / E::G;   // symbols per warp
+    const int warp = threadIdx.x >> 5, sub = (threadIdx.x & 31) / E::G, gl = E::glane();
+    const int t = (blockIdx.x * WARPS + warp) * SPW + sub;
     if (t >= d.T_d) return;
-    // the three global reads a warp starts with -- trial flag, noise variance, first 32 doubles of the QR record --
-    // are issued together (one after the other they were three DRAM round trips before the first useful
-    // instruction, 10 % of the kernel's stall samples in profiles/r02m)
+    // the global reads a group starts with -- trial flag, noise variance, the QR record -- are issued together
+    // (one after the other they were three DRAM round trips before the first useful instruction, 10 % of the
+    // kernel's stall samples in profiles/r02m)
     const double* grec = qr + ((size_t)b * d.T_d + t) * d.rec;
     const int32_t act = (active != nullptr) ? active[b] : 1;
     const double vn = varn[b];
-    const double rec0 = (lane < d.rec) ? grec[lane] : 0.0;
+    const double rec0 = (gl < E::REC) ? grec[gl] : 0.0;
     if (act == 0) return;
 
-    double* ws = enum_smem + (size_t)warp * E::WS_DOUBLES;
+    double* ws = enum_smem + (size_t)(SPW * warp + sub) * E::WS_DOUBLES;
     cplx* tab = (cplx*)(ws + E::O_TAB);
     double* g = ws + E::O_G;
-    // the QR record of the symbol: one coalesced load by the warp into the (still idle) flush scratch, then
+    // the QR record of the symbol: coalesced loads by the group into the (still idle) flush scratch, then
     // broadcast reads from shared memory (every lane needs all of it; 30+ uniform global loads per lane before)
     const double* rec = ws + E::O_SCR;
     {
-        if (lane < d.rec) ws[E::O_SCR + lane] = rec0;
-        for (int i = lane + 32; i < d.rec; i += 32) ws[E::O_SCR + i] = grec[i];
-        __syncwarp();
+        if (gl < E::REC) ws[E::O_SCR + gl] = rec0;
+        for (int i = gl + E::G; i < E::REC; i += E::G) ws[E::O_SCR + i] = grec[i];
+        __syncwarp(E::gmask());
     }
     cplx yt[NTX];
     cplx r01 = mk(0.0, 0.0);
@@ -855,19 +893,15 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         for (int s = 1; s < NTX; ++s)
 #pragma unroll
             for (int i = 0; i < s; ++i)
-                for (int m = lane; m < M; m += 32) tab[E::pair(i, s) * M + m] = cmul(Rm[i][s], E::cval(m));
-        if (lane < NTX * SQM) {
-            const int s = lane / SQM, a = lane % SQM;
-            double dd = 0.0;
+                for (int m = gl; m < M; m += E::G) tab[E::pair(i, s) * M + m] = cmul(Rm[i][s], E::cval(m));
+        if (gl < SQM) {
 #pragma unroll
-            for (int q = 0; q < NTX; ++q)
-                if (q == s) dd = Rm[q][q].x;
-            g[lane] = dd * E::pam(a);
+            for (int s = 0; s < NTX; ++s) g[s * SQM + gl] = Rm[s][s].x * E::pam(gl);
         }
     }
     const double c0 = rec[NTX * (NTX + 1) + 2 * NTX];
     const double s2 = vn * vn, inv_s2 = 1.0 / s2;
-    if (lane == 0) {
+    if (gl == 0) {
 #pragma unroll
         for (int i = 0; i < NTX; ++i) {
             ws[E::O_YT + 2 * i] = yt[i].x;
@@ -878,8 +912,8 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         ws[E::O_S2] = inv_s2;
         *(int*)(ws + E::O_CNT) = 0;
     }
-    for (int i = lane; i < E::NACC; i += 32) ws[E::O_ACC + i] = 0.0;
-    __syncwarp();
+    for (int i = gl; i < E::NACC; i += E::G) ws[E::O_ACC + i] = 0.0;
+    __syncwarp(E::gmask());
 
     Scan<NTX, SQM, HARD> sc;
     sc.ws = ws;
@@ -912,45 +946,56 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
     }
 
     // Top-level pre-pass (prefixes of two or more streams): lane m tests the FIRST prefix stream's symbol m against
-    // the Babai bound once.  A round of 32 prefixes whose top symbols are all dead would only compute its prefix
-    // levels to find every lane dead; it is skipped outright.  Dead under the initial bound implies dead under any
-    // later (tighter) one, and a dead round contributes nothing in either mode, so the sequence of visited live
-    // nodes -- hence the queue order and every output bit -- is unchanged.
-    unsigned top_alive = 0xffffffffu;
-    constexpr int TOP_SHIFT = E::BITS * (E::PL - 1);
+    // the Babai bound once.  A round of 16 prefixes whose top symbols are all dead would only compute its prefix
+    // levels to find every lane dead; it is dropped from the group's list of live rounds (16-QAM on 3+ streams and
+    // QPSK on 4+: one top symbol per round).  Dead under the initial bound implies dead under any later (tighter)
+    // one, and a dead round contributes nothing in either mode, so the sequence of visited live nodes -- hence
+    // the queue order and every output bit -- is unchanged.
+    constexpr int NROUND = (E::NPREF + E::G - 1) / E::G;
+    static_assert(NROUND <= 32, "one bit per round");
+    unsigned live = NROUND == 32 ? 0xffffffffu : (1u << NROUND) - 1u;
     if (E::PL >= 2 && sc.prune) {
+        constexpr int TOP_SHIFT = E::BITS * (E::PL - 1);
         bool a = false;
-        if (lane < M) {
+        if (gl < M) {
             const double* gs = g + (NTX - 1) * SQM;
-            const double eI = yt[NTX - 1].x - gs[lane & (SQM - 1)];
-            const double eQ = yt[NTX - 1].y - gs[lane >> E::HB];
+            const double eI = yt[NTX - 1].x - gs[gl & (SQM - 1)];
+            const double eQ = yt[NTX - 1].y - gs[gl >> E::HB];
             a = !(c0 + fma(eI, eI, eQ * eQ) > sc.lim);
         }
-        top_alive = __ballot_sync(0xffffffffu, a);
-    }
-    // all lanes iterate the same number of prefixes (invalid ones carry an infinite partial distance)
-    for (int pb = 0; pb < E::NPREF; pb += 32) {
-        if (E::PL >= 2) {
-            const int lo = pb >> TOP_SHIFT, hi = min(pb + 31, E::NPREF - 1) >> TOP_SHIFT;
-            const unsigned bits = (hi >= 31 ? 0xffffffffu : ((2u << hi) - 1u)) & ~((1u << lo) - 1u);
-            if ((top_alive & bits) == 0u) continue;
+        const unsigned top_alive = __ballot_sync(E::gmask(), a) >> E::gshift();   // this group's bits
+        live = 0u;
+#pragma unroll
+        for (int r = 0; r < NROUND; ++r) {
+            const int lo = (E::G * r) >> TOP_SHIFT, hi = min(E::G * r + E::G - 1, E::NPREF - 1) >> TOP_SHIFT;
+            const unsigned bits = ((2u << hi) - 1u) & ~((1u << lo) - 1u);   // hi < M <= 16
+            if (top_alive & bits) live |= 1u << r;
         }
-        const int p = pb + lane;
+    }
+    // The group walks its live rounds in increasing order.  Iteration j of both halves of a warp is their j-th
+    // live round, so two symbols with as many live rounds (at operating SNRs: one each) walk their prefixes in
+    // step; skipping dead rounds in place would leave the halves in different iterations, one after the other.
+    // All lanes of the group iterate the same prefixes (invalid ones carry an infinite partial distance).
+    while (live != 0u) {
+        const int pb = E::G * (__ffs(live) - 1);
+        live &= live - 1u;
+        const int p = pb + gl;
         const bool valid = p < E::NPREF;
         sc.template prefix<NTX - 1, E::PL>(yt, c0, 0, valid ? p : 0, r01, !valid);
     }
 
-    // ---- warp merge of the incumbent -------------------------------------------
+    // ---- group merge of the incumbent ------------------------------------------
     double best = sc.best;
     int bestk = sc.bestk;
+    const unsigned hm = E::gmask();   // (recomputed here rather than held in a register across the scan)
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ob = shfl_xor_d(best, o);
-        const int ok = __shfl_xor_sync(0xffffffffu, bestk, o);
+    for (int o = E::G / 2; o > 0; o >>= 1) {
+        const double ob = shfl_xor_h(hm, best, o);
+        const int ok = __shfl_xor_sync(hm, bestk, o);
         if (ob < best || (ob == best && ok < bestk)) { best = ob; bestk = ok; }
     }
     const size_t sidx = (size_t)b * d.T_d + t;
-    if (kstar != nullptr && lane == 0) kstar[sidx] = bestk;
+    if (kstar != nullptr && gl == 0) kstar[sidx] = bestk;
 
     bool collapsed = HARD;
     double S = 0.0;
@@ -963,7 +1008,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         if (!(S > 0.0) || !isfinite(S)) collapsed = true;
     }
     if (collapsed) {
-        if (lane == 0) {
+        if (gl == 0) {
             cplx xs[NTX];
 #pragma unroll
             for (int s = 0; s < NTX; ++s) xs[s] = E::cval((bestk >> (E::BITS * (NTX - 1 - s))) & (M - 1));
@@ -977,12 +1022,12 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         }
         return;
     }
-    // outputs: lane l < n_tx^2 writes R[i][j] with (i, j) = (l / n_tx, l % n_tx), lane j < n_tx writes m[j] -- two
-    // coalesced stores (lane 0 alone issued all n_tx + n_tx^2 of them one after the other before)
+    // outputs: lane l < n_tx^2 writes R[i][j] with (i, j) = (l / n_tx, l % n_tx) (l += 16), lane j < n_tx writes
+    // m[j] -- coalesced stores (lane 0 alone issued all n_tx + n_tx^2 of them one after the other before)
     {
         const double invS = 1.0 / S;
         const double* A = ws + E::O_ACC;
-        for (int l = lane; l < NTX * NTX; l += 32) {
+        for (int l = gl; l < NTX * NTX; l += E::G) {
             const int i = l / NTX, j = l % NTX;
             cplx v;
             if (i == j) {
@@ -995,8 +1040,8 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
             }
             stat_R[sidx * NTX * NTX + l] = v;
         }
-        if (lane < NTX) stat_m[sidx * NTX + lane] = mk(A[1 + lane] * invS, A[1 + NTX + lane] * invS);
-        if (lse_sym != nullptr && lane == 0) lse_sym[sidx] = -ws[E::O_AREF] * inv_s2 + log(S);
+        if (gl < NTX) stat_m[sidx * NTX + gl] = mk(A[1 + gl] * invS, A[1 + NTX + gl] * invS);
+        if (lse_sym != nullptr && gl == 0) lse_sym[sidx] = -ws[E::O_AREF] * inv_s2 + log(S);
     }
 }
 
@@ -1080,9 +1125,10 @@ static cudaError_t run_heff_ntx(const Dims& d, int nb, const double* Yd, const d
 template <int NTX, int SQM>
 static cudaError_t run_enum(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
                             double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
-    constexpr int WARPS = 4;
-    dim3 grid((d.T_d + WARPS - 1) / WARPS, nb);
-    constexpr size_t smem = sizeof(double) * WARPS * EnumT<NTX, SQM>::WS_DOUBLES;
+    typedef EnumT<NTX, SQM> E;
+    constexpr int WARPS = 4, SYMS = WARPS * 32 / E::G;   // symbols per CTA
+    dim3 grid((d.T_d + SYMS - 1) / SYMS, nb);
+    constexpr size_t smem = sizeof(double) * SYMS * E::WS_DOUBLES;
     static SmemOptIn optin_hard, optin_soft;
     cudaError_t e;
     if (d.mode == SBCE_MODE_HARD) {
