@@ -64,9 +64,9 @@ static int make_dims(const sbce_cfg* c, Dims* d, bool with_estep = true) {
     if (with_estep) {
         // joint hypothesis indices are int32 (kstar); the exhaustive tree is instantiated up to 2^24 leaves
         // for the wide arrays (8 streams of QPSK, 6 of 16-QAM) -- beyond that use the partitioned modes
-        const int bits = c->n_tx * (sq == 2 ? 2 : (sq == 4 ? 4 : 6));
+        const int log2M = sq == 2 ? 2 : (sq == 4 ? 4 : 6), bits = c->n_tx * log2M;
         const bool tree = c->mode == SBCE_MODE_SOFT || c->mode == SBCE_MODE_HARD;
-        if (tree && c->n_tx > 4 && bits > 24) return SBCE_E_UNSUPPORTED;
+        if (tree && !enum_instantiated(c->n_tx, log2M)) return SBCE_E_UNSUPPORTED;
         if ((c->mode == SBCE_MODE_ZF || c->mode == SBCE_MODE_MMSE) && bits > 30) return SBCE_E_UNSUPPORTED;
     }
     d->N = c->N; d->N1 = c->N + 1; d->n_tx = c->n_tx; d->n_rx = c->n_rx; d->M = c->M; d->sqM = sq;

@@ -75,8 +75,20 @@ struct Dims {
 
 // Per-symbol QR record written by the effective-channel kernel and consumed by
 // the enumeration kernel (doubles): R upper triangle row-major, real diagonal
-// stored as (d,0); then ytilde[n_tx]; then c0.
-__host__ __device__ __forceinline__ int qr_record_doubles(int n_tx) { return n_tx * (n_tx + 1) + 2 * n_tx + 2; }
+// stored as (d,0); then ytilde[n_tx]; then c0 stored as (c0,0).  Offsets of the
+// (re, im) pair of R_ij (i <= j), of ytilde_i and of c0:
+__host__ __device__ __forceinline__ constexpr int qr_rec_R(int n_tx, int i, int j) {
+    return 2 * (i * n_tx - i * (i - 1) / 2 + j - i);
+}
+__host__ __device__ __forceinline__ constexpr int qr_rec_yt(int n_tx, int i) { return n_tx * (n_tx + 1) + 2 * i; }
+__host__ __device__ __forceinline__ constexpr int qr_rec_c0(int n_tx) { return qr_rec_yt(n_tx, n_tx); }
+__host__ __device__ __forceinline__ constexpr int qr_record_doubles(int n_tx) { return n_tx * (n_tx + 1) + 2 * n_tx + 2; }
+static_assert(qr_rec_yt(8, 0) == qr_rec_R(8, 7, 7) + 2 && qr_rec_c0(8) + 2 == qr_record_doubles(8),
+              "QR record: R, ytilde and c0 are packed back to back");
+
+// The exhaustive tree (k_enum) is instantiated for every constellation up to 4 streams, and beyond that while
+// the joint hypothesis index has at most 24 bits (8 streams of QPSK, 6 of 16-QAM).
+constexpr bool enum_instantiated(int n_tx, int log2M) { return n_tx <= 4 || n_tx * log2M <= 24; }
 
 // workspace carve-up for `nb` trials in flight
 struct Workspace {

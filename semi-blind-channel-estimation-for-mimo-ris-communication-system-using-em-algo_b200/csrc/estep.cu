@@ -135,24 +135,23 @@ __device__ __forceinline__ void heff_qr_finish(const Dims& d, int b, int t, cplx
     }
 
     double* rec = qr + ((size_t)b * d.T_d + t) * d.rec;
-    int o = 0;
 #pragma unroll
     for (int i = 0; i < NTX; ++i)
 #pragma unroll
         for (int j = i; j < NTX; ++j) {
-            rec[o++] = A[i][j].x;
-            rec[o++] = (j == i) ? 0.0 : A[i][j].y;
+            rec[qr_rec_R(NTX, i, j)] = A[i][j].x;
+            rec[qr_rec_R(NTX, i, j) + 1] = (j == i) ? 0.0 : A[i][j].y;
         }
 #pragma unroll
     for (int i = 0; i < NTX; ++i) {
-        rec[o++] = y[i].x;
-        rec[o++] = y[i].y;
+        rec[qr_rec_yt(NTX, i)] = y[i].x;
+        rec[qr_rec_yt(NTX, i) + 1] = y[i].y;
     }
     double c0 = 0.0;
 #pragma unroll
     for (int i = NTX; i < NR; ++i) c0 += cnorm2(y[i]);
-    rec[o++] = c0;
-    rec[o++] = 0.0;
+    rec[qr_rec_c0(NTX)] = c0;
+    rec[qr_rec_c0(NTX) + 1] = 0.0;
 }
 
 template <int NTX, int NRX>
@@ -387,19 +386,18 @@ __global__ void __launch_bounds__(128) k_heff_qr_rows(Dims d, const cplx* __rest
     if (!tv) return;
     double* rec = qr + ((size_t)b * d.T_d + t) * d.rec;
     if (r < NTX) {
-        double* o = rec + 2 * (r * NTX - (r * (r - 1)) / 2);
 #pragma unroll
         for (int j = 0; j < NTX; ++j)
             if (j >= r) {
-                o[2 * (j - r)] = A[j].x;
-                o[2 * (j - r) + 1] = (j == r) ? 0.0 : A[j].y;
+                rec[qr_rec_R(NTX, r, j)] = A[j].x;
+                rec[qr_rec_R(NTX, r, j) + 1] = (j == r) ? 0.0 : A[j].y;
             }
-        rec[NTX * (NTX + 1) + 2 * r] = A[NTX].x;
-        rec[NTX * (NTX + 1) + 2 * r + 1] = A[NTX].y;
+        rec[qr_rec_yt(NTX, r)] = A[NTX].x;
+        rec[qr_rec_yt(NTX, r) + 1] = A[NTX].y;
     }
     if (r == 0) {
-        rec[NTX * (NTX + 1) + 2 * NTX] = c0;
-        rec[NTX * (NTX + 1) + 2 * NTX + 1] = 0.0;
+        rec[qr_rec_c0(NTX)] = c0;
+        rec[qr_rec_c0(NTX) + 1] = 0.0;
     }
 }
 
@@ -420,8 +418,10 @@ struct EnumT {
     static constexpr int NPREF = 1 << (BITS * PL);
     static constexpr int NPAIR = NTX * (NTX - 1) / 2;
     static constexpr int NPAIR1 = NPAIR > 0 ? NPAIR : 1;
-    static constexpr int NACC = 1 + 3 * NTX + 2 * NPAIR;  // S, m (re,im), R diag, R upper (re,im)
-    static constexpr int REC = NTX * (NTX + 1) + 2 * NTX + 2;   // qr_record_doubles(NTX)
+    // accumulator block (doubles): S = sum of the weights, Re m_s, Im m_s, R_ss, then (Re, Im) of R_is for i < s
+    static constexpr int A_MRE = 1, A_MIM = A_MRE + NTX, A_RD = A_MIM + NTX, A_RU = A_RD + NTX;
+    static constexpr int NACC = A_RU + 2 * NPAIR;
+    static constexpr int REC = qr_record_doubles(NTX);
     // Lanes per symbol: a half-warp (two symbols per warp) up to 4 streams.  The deep trees of 5..8 streams keep
     // a whole warp: their halves diverge at every level, one after the other (8x8 QPSK hard: 1.04 ms per launch
     // on half-warps against 0.88 ms on warps).
@@ -458,6 +458,70 @@ struct EnumT {
     __device__ __forceinline__ static double pam(int a) { return (double)(2 * a - SQM + 1); }
     __device__ __forceinline__ static cplx cval(int m) { return mk(pam(m & (SQM - 1)), pam(m >> HB)); }
     __device__ __forceinline__ static int pair(int i, int s) { return s * (s - 1) / 2 + i; }
+    __device__ __forceinline__ static int acc_R(int i, int s) { return A_RU + 2 * pair(i, s); }   // Re R_is; Im at +1
+    // symbol index of stream s in a node or hypothesis code
+    __device__ __forceinline__ static int digit(int code, int s) { return (code >> (BITS * (NTX - 1 - s))) & (M - 1); }
+
+    // One tree level, stream s taking symbol m: dist = its term of the partial distance; descend = the residuals
+    // of the streams below lose R_is c_m (out may be acc); step = both, returning base + dist.
+    __device__ __forceinline__ static double dist(const cplx (&acc)[NTX], int s, int m, const double* g) {
+        const double* gs = g + s * SQM;
+        const double eI = acc[s].x - gs[m & (SQM - 1)];
+        const double eQ = acc[s].y - gs[m >> HB];
+        return fma(eI, eI, eQ * eQ);
+    }
+    __device__ __forceinline__ static void descend(const cplx (&acc)[NTX], cplx (&out)[NTX], int s, int m,
+                                                   const cplx* tab) {
+#pragma unroll
+        for (int i = 0; i < NTX; ++i) out[i] = (i < s) ? csub(acc[i], tab[pair(i, s) * M + m]) : acc[i];
+    }
+    __device__ __forceinline__ static double step(const cplx (&acc)[NTX], cplx (&out)[NTX], int s, int m, double base,
+                                                  const double* g, const cplx* tab) {
+        const double nb = base + dist(acc, s, m, g);
+        descend(acc, out, s, m, tab);
+        return nb;
+    }
+
+    // A queued node rebuilt from its code and the symbol's shared block: returns its partial distance (streams
+    // NTX-1 .. 1), t0 = its residual on row 0.
+    __device__ __forceinline__ static double rebuild(const double* ws, int code, cplx& t0) {
+        cplx acc[NTX];
+#pragma unroll
+        for (int i = 0; i < NTX; ++i) acc[i] = mk(ws[O_YT + 2 * i], ws[O_YT + 2 * i + 1]);
+        double base = ws[O_C0];
+#pragma unroll
+        for (int s = NTX - 1; s >= 1; --s)
+            base = step(acc, acc, s, digit(code, s), base, ws + O_G, (const cplx*)(ws + O_TAB));
+        t0 = acc[0];
+        return base;
+    }
+
+    // Every statistic of one node, in accumulator order, as sink(index, value).  E0, F0, Q0: the sums over the
+    // node's M leaves of the weight, of weight * conj(x_0) and of weight * |x_0|^2; x_1.. are the node's digits.
+    template <class Sink>
+    __device__ __forceinline__ static void node_stats(int code, double E0, cplx F0, double Q0, Sink&& sink) {
+        sink(0, E0);
+        sink(A_MRE, F0.x);
+        sink(A_MIM, F0.y);
+        sink(A_RD, Q0);
+#pragma unroll
+        for (int s = 1; s < NTX; ++s) {
+            const cplx xs = cval(digit(code, s));
+            sink(A_MRE + s, E0 * xs.x);
+            sink(A_MIM + s, -E0 * xs.y);
+            sink(A_RD + s, E0 * cnorm2(xs));
+            const cplx v = cmul(F0, xs);  // conj(x_0) x_s summed over the leaves
+            sink(acc_R(0, s), v.x);
+            sink(acc_R(0, s) + 1, v.y);
+#pragma unroll
+            for (int i = 1; i < NTX; ++i)
+                if (i < s) {
+                    const cplx cx = cmulc(xs, cval(digit(code, i)));  // conj(x_i) x_s
+                    sink(acc_R(i, s), E0 * cx.x);
+                    sink(acc_R(i, s) + 1, E0 * cx.y);
+                }
+        }
+    }
 
     // nearest PAM level to v among gs[0..SQM) (increasing), first index on ties; dist = squared distance
     __device__ __forceinline__ static int slice(double v, const double* gs, double& dist) {
@@ -491,14 +555,12 @@ struct EnumT {
 template <int NTX, int SQM>
 __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
     typedef EnumT<NTX, SQM> E;
-    constexpr int M = E::M;
     const int lane = E::glane();
     const unsigned hm = E::gmask();
     __syncwarp(hm);
     int* cntp = (int*)(ws + E::O_CNT);
     const int n = min(*cntp, E::QCAP);
     const int* q = (const int*)(ws + E::O_Q);
-    const cplx* tab = (const cplx*)(ws + E::O_TAB);
     const double* g = ws + E::O_G;
     const double inv_s2 = ws[E::O_S2];
     double aref = ws[E::O_AREF];
@@ -521,24 +583,8 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
         const double pq = E::pam(a);
         for (int e = 0; e < n; ++e) {
             const int code = q[e];
-            double base = ws[E::O_C0];
             cplx t0;
-            {
-                cplx acc[NTX];
-#pragma unroll
-                for (int i = 0; i < NTX; ++i) acc[i] = mk(ws[E::O_YT + 2 * i], ws[E::O_YT + 2 * i + 1]);
-#pragma unroll
-                for (int s = NTX - 1; s >= 1; --s) {
-                    const int m = (code >> (E::BITS * (NTX - 1 - s))) & (M - 1);
-                    const double eI = acc[s].x - g[s * SQM + (m & (SQM - 1))];
-                    const double eQ = acc[s].y - g[s * SQM + (m >> E::HB)];
-                    base += fma(eI, eI, eQ * eQ);
-#pragma unroll
-                    for (int i = 0; i < NTX; ++i)
-                        if (i < s) acc[i] = csub(acc[i], tab[E::pair(i, s) * M + m]);
-                }
-                t0 = acc[0];
-            }
+            const double base = E::rebuild(ws, code, t0);
             const double ev = (isQ ? t0.y : t0.x) - g[a];
             const double dd = ev * ev;
             double mn = dd;
@@ -568,29 +614,9 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
             double mine[NR];
 #pragma unroll
             for (int r = 0; r < NR; ++r) mine[r] = 0.0;
-            auto add = [&](int idx, double v) { if ((idx & (E::G - 1)) == lane) mine[idx / E::G] = v; };
-            add(0, E0);
-            add(1, F0.x);
-            add(1 + NTX, F0.y);
-            add(1 + 2 * NTX, Q0);
-#pragma unroll
-            for (int s = 1; s < NTX; ++s) {
-                const cplx xs = E::cval((code >> (E::BITS * (NTX - 1 - s))) & (M - 1));
-                add(1 + s, E0 * xs.x);
-                add(1 + NTX + s, -E0 * xs.y);
-                add(1 + 2 * NTX + s, E0 * cnorm2(xs));
-                const cplx v = cmul(F0, xs);  // conj(x_0) x_s summed over the leaves
-                add(1 + 3 * NTX + 2 * E::pair(0, s), v.x);
-                add(1 + 3 * NTX + 2 * E::pair(0, s) + 1, v.y);
-#pragma unroll
-                for (int i = 1; i < NTX; ++i)
-                    if (i < s) {
-                        const cplx xi = E::cval((code >> (E::BITS * (NTX - 1 - i))) & (M - 1));
-                        const cplx cx = cmulc(xs, xi);  // conj(x_i) x_s
-                        add(1 + 3 * NTX + 2 * E::pair(i, s), E0 * cx.x);
-                        add(1 + 3 * NTX + 2 * E::pair(i, s) + 1, E0 * cx.y);
-                    }
-            }
+            E::node_stats(code, E0, F0, Q0, [&](int idx, double v) {
+                if ((idx & (E::G - 1)) == lane) mine[idx / E::G] = v;
+            });
 #pragma unroll
             for (int r = 0; r < NR; ++r)
                 if (E::G * r + lane < E::NACC) A[E::G * r + lane] += mine[r];
@@ -610,30 +636,13 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
     // instead of NACC butterfly reductions: ~25 stores + nround loads per lane, no shuffles)
     double* scr = ws + E::O_SCR;
     int nround = 0;
-    auto radd = [&](int idx, double v) { scr[idx * E::G + lane] = v; };
     for (int e0 = 0; e0 < n; e0 += E::G) {
         const int e = e0 + lane;
         const bool have = e < n;
         nround = min(E::G, n - e0);
         const int code = have ? q[e] : 0;
         cplx t0;
-        double base = ws[E::O_C0];
-        {
-            cplx acc[NTX];
-#pragma unroll
-            for (int i = 0; i < NTX; ++i) acc[i] = mk(ws[E::O_YT + 2 * i], ws[E::O_YT + 2 * i + 1]);
-#pragma unroll
-            for (int s = NTX - 1; s >= 1; --s) {
-                const int m = (code >> (E::BITS * (NTX - 1 - s))) & (M - 1);
-                const double eI = acc[s].x - g[s * SQM + (m & (SQM - 1))];
-                const double eQ = acc[s].y - g[s * SQM + (m >> E::HB)];
-                base += fma(eI, eI, eQ * eQ);
-#pragma unroll
-                for (int i = 0; i < NTX; ++i)
-                    if (i < s) acc[i] = csub(acc[i], tab[E::pair(i, s) * M + m]);
-            }
-            t0 = acc[0];
-        }
+        const double base = E::rebuild(ws, code, t0);
         double minI = 1e300, minQ = 1e300;
 #pragma unroll
         for (int a = 0; a < SQM; ++a) {
@@ -654,28 +663,7 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
         const double E0 = W * EI * EQ;
         const cplx F0 = mk(W * A1 * EQ, -W * EI * B1);  // sum over leaves of e * conj(x_0)
         const double Q0 = W * (A2 * EQ + EI * B2);      // sum over leaves of e * |x_0|^2
-        radd(0, E0);
-        radd(1, F0.x);
-        radd(1 + NTX, F0.y);
-        radd(1 + 2 * NTX, Q0);
-#pragma unroll
-        for (int s = 1; s < NTX; ++s) {
-            const cplx xs = E::cval((code >> (E::BITS * (NTX - 1 - s))) & (M - 1));
-            radd(1 + s, E0 * xs.x);
-            radd(1 + NTX + s, -E0 * xs.y);
-            radd(1 + 2 * NTX + s, E0 * cnorm2(xs));
-            const cplx v = cmul(F0, xs);  // conj(x_0) x_s summed over the leaves
-            radd(1 + 3 * NTX + 2 * E::pair(0, s), v.x);
-            radd(1 + 3 * NTX + 2 * E::pair(0, s) + 1, v.y);
-#pragma unroll
-            for (int i = 1; i < NTX; ++i)
-                if (i < s) {
-                    const cplx xi = E::cval((code >> (E::BITS * (NTX - 1 - i))) & (M - 1));
-                    const cplx cx = cmulc(xs, xi);  // conj(x_i) x_s
-                    radd(1 + 3 * NTX + 2 * E::pair(i, s), E0 * cx.x);
-                    radd(1 + 3 * NTX + 2 * E::pair(i, s) + 1, E0 * cx.y);
-                }
-        }
+        E::node_stats(code, E0, F0, Q0, [&](int idx, double v) { scr[idx * E::G + lane] = v; });
         __syncwarp(hm);
         for (int i = lane; i < E::NACC; i += E::G) {
             double acc = 0.0;
@@ -796,13 +784,8 @@ struct Scan {
             if (__all_sync(E::gmask(), dead)) return;
 #pragma unroll 1
             for (int m = 0; m < M; ++m) {
-                const double* gs = g + S_ * SQM;
-                const double eI = acc[S_].x - gs[m & (SQM - 1)];
-                const double eQ = acc[S_].y - gs[m >> E::HB];
-                const double nb = base + fma(eI, eI, eQ * eQ);
                 cplx nacc[NTX];
-#pragma unroll
-                for (int i = 0; i < NTX; ++i) nacc[i] = (i < S_) ? csub(acc[i], tab[E::pair(i, S_) * M + m]) : acc[i];
+                const double nb = E::step(acc, nacc, S_, m, base, g, tab);
                 inner<S_ - 1>(nacc, nb, code + (m << (E::BITS * (NTX - 1 - S_))), r01, dead);
             }
         }
@@ -815,13 +798,8 @@ struct Scan {
             inner<S_>(acc, base, code, r01, dead);
         } else {
             const int m = (p >> (E::BITS * (LEFT - 1))) & (M - 1);
-            const double* gs = g + S_ * SQM;
-            const double eI = acc[S_].x - gs[m & (SQM - 1)];
-            const double eQ = acc[S_].y - gs[m >> E::HB];
-            const double nb = base + fma(eI, eI, eQ * eQ);
             cplx nacc[NTX];
-#pragma unroll
-            for (int i = 0; i < NTX; ++i) nacc[i] = (i < S_) ? csub(acc[i], tab[E::pair(i, S_) * M + m]) : acc[i];
+            const double nb = E::step(acc, nacc, S_, m, base, g, tab);
             prefix<S_ - 1, LEFT - 1>(nacc, nb, code + (m << (E::BITS * (NTX - 1 - S_))), p, r01, dead);
         }
     }
@@ -873,19 +851,12 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
     double r00;
     {
         cplx Rm[NTX][NTX];
-        int o = 0;
 #pragma unroll
         for (int i = 0; i < NTX; ++i)
 #pragma unroll
-            for (int j = i; j < NTX; ++j) {
-                Rm[i][j] = mk(rec[o], rec[o + 1]);
-                o += 2;
-            }
+            for (int j = i; j < NTX; ++j) Rm[i][j] = mk(rec[qr_rec_R(NTX, i, j)], rec[qr_rec_R(NTX, i, j) + 1]);
 #pragma unroll
-        for (int i = 0; i < NTX; ++i) {
-            yt[i] = mk(rec[o], rec[o + 1]);
-            o += 2;
-        }
+        for (int i = 0; i < NTX; ++i) yt[i] = mk(rec[qr_rec_yt(NTX, i)], rec[qr_rec_yt(NTX, i) + 1]);
         r00 = Rm[0][0].x;
         if (NTX > 1) r01 = Rm[0][NTX > 1 ? 1 : 0];
         // tables: R_is * c_m for i<s, and the real PAM levels R_ss * pam_a
@@ -899,7 +870,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
             for (int s = 0; s < NTX; ++s) g[s * SQM + gl] = Rm[s][s].x * E::pam(gl);
         }
     }
-    const double c0 = rec[NTX * (NTX + 1) + 2 * NTX];
+    const double c0 = rec[qr_rec_c0(NTX)];
     const double s2 = vn * vn, inv_s2 = 1.0 / s2;
     if (gl == 0) {
 #pragma unroll
@@ -936,9 +907,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
             const int m = iQ * SQM + iI;
             base += dI + dQ;
             k += m << (E::BITS * (NTX - 1 - s));
-#pragma unroll
-            for (int i = 0; i < NTX; ++i)
-                if (i < s) acc[i] = csub(acc[i], tab[E::pair(i, s) * M + m]);
+            E::descend(acc, acc, s, m, tab);
         }
         sc.best = base;
         sc.bestk = k;
@@ -956,13 +925,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
     unsigned live = NROUND == 32 ? 0xffffffffu : (1u << NROUND) - 1u;
     if (E::PL >= 2 && sc.prune) {
         constexpr int TOP_SHIFT = E::BITS * (E::PL - 1);
-        bool a = false;
-        if (gl < M) {
-            const double* gs = g + (NTX - 1) * SQM;
-            const double eI = yt[NTX - 1].x - gs[gl & (SQM - 1)];
-            const double eQ = yt[NTX - 1].y - gs[gl >> E::HB];
-            a = !(c0 + fma(eI, eI, eQ * eQ) > sc.lim);
-        }
+        const bool a = gl < M && !(c0 + E::dist(yt, NTX - 1, gl, g) > sc.lim);
         const unsigned top_alive = __ballot_sync(E::gmask(), a) >> E::gshift();   // this group's bits
         live = 0u;
 #pragma unroll
@@ -1011,7 +974,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         if (gl == 0) {
             cplx xs[NTX];
 #pragma unroll
-            for (int s = 0; s < NTX; ++s) xs[s] = E::cval((bestk >> (E::BITS * (NTX - 1 - s))) & (M - 1));
+            for (int s = 0; s < NTX; ++s) xs[s] = E::cval(E::digit(bestk, s));
 #pragma unroll
             for (int i = 0; i < NTX; ++i) {
                 stat_m[sidx * NTX + i] = cconj(xs[i]);
@@ -1031,16 +994,15 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
             const int i = l / NTX, j = l % NTX;
             cplx v;
             if (i == j) {
-                v = mk(A[1 + 2 * NTX + j] * invS, 0.0);
+                v = mk(A[E::A_RD + j] * invS, 0.0);
             } else {
-                const int lo = min(i, j), hi = max(i, j);
-                const int pr = 1 + 3 * NTX + 2 * E::pair(lo, hi);
+                const int pr = E::acc_R(min(i, j), max(i, j));
                 const double a = A[pr] * invS, c = A[pr + 1] * invS;
                 v = mk(a, i < j ? c : -c);
             }
             stat_R[sidx * NTX * NTX + l] = v;
         }
-        if (gl < NTX) stat_m[sidx * NTX + gl] = mk(A[1 + gl] * invS, A[1 + NTX + gl] * invS);
+        if (gl < NTX) stat_m[sidx * NTX + gl] = mk(A[E::A_MRE + gl] * invS, A[E::A_MIM + gl] * invS);
         if (lse_sym != nullptr && gl == 0) lse_sym[sidx] = -ws[E::O_AREF] * inv_s2 + log(S);
     }
 }
@@ -1123,27 +1085,40 @@ static cudaError_t run_heff_ntx(const Dims& d, int nb, const double* Yd, const d
 }
 
 template <int NTX, int SQM>
-static cudaError_t run_enum(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
-                            double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
+static cudaError_t run_enum_sqm(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
+                                double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
     typedef EnumT<NTX, SQM> E;
     constexpr int WARPS = 4, SYMS = WARPS * 32 / E::G;   // symbols per CTA
     dim3 grid((d.T_d + SYMS - 1) / SYMS, nb);
     constexpr size_t smem = sizeof(double) * SYMS * E::WS_DOUBLES;
-    static SmemOptIn optin_hard, optin_soft;
-    cudaError_t e;
-    if (d.mode == SBCE_MODE_HARD) {
-        e = opt_in_smem(optin_hard, (const void*)k_enum<NTX, SQM, true, WARPS>, smem);
-        if (e != cudaSuccess) return e;
-        k_enum<NTX, SQM, true, WARPS><<<grid, WARPS * 32, smem, s>>>(d, qr, varn, active, (cplx*)stat_m,
-                                                                      (cplx*)stat_R, kstar, lse_sym);
-    } else {
-        e = opt_in_smem(optin_soft, (const void*)k_enum<NTX, SQM, false, WARPS>, smem);
-        if (e != cudaSuccess) return e;
-        k_enum<NTX, SQM, false, WARPS><<<grid, WARPS * 32, smem, s>>>(d, qr, varn, active, (cplx*)stat_m,
-                                                                       (cplx*)stat_R, kstar, lse_sym);
-    }
+    static SmemOptIn optin[2];   // one per kernel: [hard]
+    const bool hard = d.mode == SBCE_MODE_HARD;
+    const auto kernel = hard ? k_enum<NTX, SQM, true, WARPS> : k_enum<NTX, SQM, false, WARPS>;
+    cudaError_t e = opt_in_smem(optin[hard], (const void*)kernel, smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<grid, WARPS * 32, smem, s>>>(d, qr, varn, active, (cplx*)stat_m, (cplx*)stat_R, kstar, lse_sym);
     count_launch();
     return cudaGetLastError();
+}
+
+template <int NTX>
+static cudaError_t run_enum(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
+                            double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
+    switch (d.sqM) {   // enum_instantiated takes log2 M
+        case 2:
+            if constexpr (enum_instantiated(NTX, 2))
+                return run_enum_sqm<NTX, 2>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+            break;
+        case 4:
+            if constexpr (enum_instantiated(NTX, 4))
+                return run_enum_sqm<NTX, 4>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+            break;
+        case 8:
+            if constexpr (enum_instantiated(NTX, 6))
+                return run_enum_sqm<NTX, 8>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+            break;
+    }
+    return cudaErrorInvalidValue;
 }
 
 template <int NTX>
@@ -1154,29 +1129,6 @@ static cudaError_t run_heff_rows(const Dims& d, int nb, const double* Yd, const 
                                              (const cplx*)Xoff, qr);
     count_launch();
     return cudaGetLastError();
-}
-
-// wide trees: only constellations whose joint hypothesis index fits comfortably in 32 bits are instantiated
-// (n_tx log2 M <= 24); abi.cu::make_dims rejects the rest before any launch
-template <int NTX>
-static cudaError_t run_enum_wide(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
-                                 double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
-    if (d.sqM == 2) return run_enum<NTX, 2>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-    if constexpr (NTX <= 6) {
-        if (d.sqM == 4) return run_enum<NTX, 4>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <int NTX>
-static cudaError_t run_enum_ntx(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
-                                double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
-    switch (d.sqM) {
-        case 2: return run_enum<NTX, 2>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 4: return run_enum<NTX, 4>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 8: return run_enum<NTX, 8>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        default: return cudaErrorInvalidValue;
-    }
 }
 
 cudaError_t launch_heff_qr(const Dims& d, int nb, const double* Yd, const double* PsiD, const double* theta,
@@ -1197,14 +1149,14 @@ cudaError_t launch_heff_qr(const Dims& d, int nb, const double* Yd, const double
 cudaError_t launch_enum(const Dims& d, int nb, const double* qr, const double* varn, const int32_t* active,
                         double* stat_m, double* stat_R, int32_t* kstar, double* lse_sym, cudaStream_t s) {
     switch (d.n_tx) {
-        case 1: return run_enum_ntx<1>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 2: return run_enum_ntx<2>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 3: return run_enum_ntx<3>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 4: return run_enum_ntx<4>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 5: return run_enum_wide<5>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 6: return run_enum_wide<6>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 7: return run_enum_wide<7>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
-        case 8: return run_enum_wide<8>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 1: return run_enum<1>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 2: return run_enum<2>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 3: return run_enum<3>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 4: return run_enum<4>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 5: return run_enum<5>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 6: return run_enum<6>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 7: return run_enum<7>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
+        case 8: return run_enum<8>(d, nb, qr, varn, active, stat_m, stat_R, kstar, lse_sym, s);
         default: return cudaErrorInvalidValue;
     }
 }
