@@ -21,7 +21,8 @@
 //     symbols per warp (a whole warp per symbol for 5..8 streams), walks the
 //     hypothesis tree stream n_tx-1 -> 1 with partial residuals in registers; the
 //     top levels are split across the group's lanes, the inner levels are
-//     group-uniform loops fed by shared-memory tables R_ij*c_m.  Every collective
+//     group-uniform loops fed by shared-memory tables R_ij*c_m (on half-warps the
+//     stream-1 level is packed: the lanes split the children of one live node).  Every collective
 //     is a group collective, so the two symbols of a warp may take different paths.  Because R_00 is real, the last stream separates into its
 //     in-phase and quadrature PAM components, so the sum over the M leaves of a
 //     node is a product of two sqrt(M)-term sums: every hypothesis is accounted
@@ -442,14 +443,14 @@ struct EnumT {
     static constexpr int O_ACC = O_C0 + 1;
     static constexpr int O_AREF = O_ACC + NACC;
     static constexpr int O_S2 = O_AREF + 1;     // inv_s2
-    static constexpr int O_CNT = O_S2 + 1;      // int counter lives in this double slot
-    static constexpr int O_Q = O_CNT + 1;       // QCAP ints = QCAP/2 doubles
+    static constexpr int O_Q = O_S2 + 1;        // QCAP ints = QCAP/2 doubles (the count is a group-uniform register)
     static constexpr int O_SCR = O_Q + QCAP / 2;   // [NACC][16] reduction scratch of the flush (QR record at start-up)
     static constexpr int WS_DOUBLES = ((O_SCR + NACC * G) + 1) & ~1;
     static_assert(NACC * G >= REC, "the QR record is staged in the flush scratch");
-    // The queue never drops a node (a dropped node is lost silently).  In the stream-1 level a group enqueues at
-    // most G*M nodes (G*SQM per row) between two maybe_flush() calls, whose threshold leaves room for them.  When every node
-    // stream is a prefix stream there is no such call, and at most one node per prefix is queued.
+    // The queue never drops a node (a dropped node is lost silently).  Between two maybe_flush() calls a group
+    // enqueues at most G nodes in a packed step (one per lane), and G*M (G*SQM per row) in a stream-1 level walked by
+    // every lane for its own node; the threshold leaves room for them.  When every node stream is a prefix stream
+    // there is no such call, and at most one node per prefix is queued.
     static_assert(PL < NODE_STREAMS || NPREF <= QCAP, "prefix-only trees must fit the queue without a flush");
     static_assert(G * SQM < QCAP, "maybe_flush threshold");
     // the top-level pre-pass votes with one lane per top symbol
@@ -551,15 +552,15 @@ struct EnumT {
 // symbol's group takes queue entries round-robin, rebuilds the node's residuals from its code, sums its
 // M leaves in closed form (separable in-phase / quadrature PAM sums) and the group adds the result to the
 // shared accumulators, kept relative to the reference distance `aref` (rescaled when the incumbent improves).
+// `count` entries are queued; the caller empties the queue afterwards.
 // Only the calling group takes part: the other symbol of a warp may be anywhere else.
 template <int NTX, int SQM>
-__device__ __noinline__ void enum_flush(double* ws, double warp_best) {
+__device__ __noinline__ void enum_flush(double* ws, double warp_best, int count) {
     typedef EnumT<NTX, SQM> E;
     const int lane = E::glane();
     const unsigned hm = E::gmask();
     __syncwarp(hm);
-    int* cntp = (int*)(ws + E::O_CNT);
-    const int n = min(*cntp, E::QCAP);
+    const int n = min(count, E::QCAP);
     const int* q = (const int*)(ws + E::O_Q);
     const double* g = ws + E::O_G;
     const double inv_s2 = ws[E::O_S2];
@@ -622,10 +623,7 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
                 if (E::G * r + lane < E::NACC) A[E::G * r + lane] += mine[r];
             __syncwarp(hm);
         }
-        if (lane == 0) {
-            ws[E::O_AREF] = aref;
-            *cntp = 0;
-        }
+        if (lane == 0) ws[E::O_AREF] = aref;
         __syncwarp(hm);
         return;
     }
@@ -673,10 +671,7 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best) {
         __syncwarp(hm);
     }
     __syncwarp(hm);
-    if (lane == 0) {
-        ws[E::O_AREF] = aref;
-        *cntp = 0;
-    }
+    if (lane == 0) ws[E::O_AREF] = aref;
     __syncwarp(hm);
 }
 
@@ -691,45 +686,61 @@ struct Scan {
     double thr;       // 64 varn^2
     double best, lim; // incumbent distance and enqueue limit best + thr
     int bestk;
+    int cnt;          // queued nodes (group-uniform)
     bool prune;       // skip subtrees whose partial distance already exceeds lim (bit-identical results)
 
-    // the M leaves below a node: t0 = residual on row 0, nb = partial distance of the node, code = node digits
-    __device__ __forceinline__ void leaf(cplx t0, double nb, int code) {
+    // the M leaves below a node: t0 = residual on row 0, nb = partial distance of the node, code = node digits.
+    // Every lane of the group calls it (`live`: the lane holds a node), so that queue slots are handed out in lane
+    // order by a ballot: the queue order follows from which lane holds which node, not from the atomics' timing.
+    __device__ __forceinline__ void leaf(cplx t0, double nb, int code, bool live) {
         const double fI = E::fold(t0.x, r0), fQ = E::fold(t0.y, r0);
         const double nodemin = fma(fI, fI, fma(fQ, fQ, nb));
-        if (nodemin <= lim) {  // rare at operating SNRs
-            if (nodemin <= best) {
-                double dI, dQ;
-                const int iI = E::slice(t0.x, g, dI), iQ = E::slice(t0.y, g, dQ);
-                const double val = nb + dI + dQ;
-                const int k = code + ((iQ * SQM + iI) << (E::BITS * (NTX - 1)));
-                if (val < best || (val == best && k < bestk)) {
-                    best = val;
-                    bestk = k;
-                    lim = HARD ? val : val + thr;
-                }
-            }
-            if (!HARD) {
-                int* cntp = (int*)(ws + E::O_CNT);
-                const int slot = atomicAdd(cntp, 1);
-                if (slot < E::QCAP) ((int*)(ws + E::O_Q))[slot] = code;
+        const bool hit = live && nodemin <= lim;   // rare at operating SNRs
+        if (hit && nodemin <= best) {
+            double dI, dQ;
+            const int iI = E::slice(t0.x, g, dI), iQ = E::slice(t0.y, g, dQ);
+            const double val = nb + dI + dQ;
+            const int k = code + ((iQ * SQM + iI) << (E::BITS * (NTX - 1)));
+            if (val < best || (val == best && k < bestk)) {
+                best = val;
+                bestk = k;
+                lim = HARD ? val : val + thr;
             }
         }
+        if (!HARD) {
+            const unsigned q = __ballot_sync(E::gmask(), hit) >> E::gshift();
+            if (q != 0u) {
+                if (hit) {
+                    const int slot = cnt + __popc(q & ((1u << E::glane()) - 1u));
+                    if (slot < E::QCAP) ((int*)(ws + E::O_Q))[slot] = code;
+                }
+                cnt += __popc(q);
+            }
+        }
+    }
+
+    // group arg-min of (best, bestk), first index on ties; every lane ends with it and the matching limit
+    __device__ __forceinline__ void merge_best() {
+        const unsigned hm = E::gmask();
+#pragma unroll
+        for (int o = E::G / 2; o > 0; o >>= 1) {
+            const double ob = shfl_xor_h(hm, best, o);
+            const int ok = __shfl_xor_sync(hm, bestk, o);
+            if (ob < best || (ob == best && ok < bestk)) { best = ob; bestk = ok; }
+        }
+        lim = HARD ? best : best + thr;
     }
 
     // PER_LANE: nodes a lane may enqueue before the next call
     template <int PER_LANE>
     __device__ __forceinline__ void maybe_flush() {
-        if (!HARD) {
+        if (!HARD && cnt > E::QCAP - E::G * PER_LANE) {
             const unsigned hm = E::gmask();
-            __syncwarp(hm);
-            const int c = *(volatile int*)(ws + E::O_CNT);
-            if (c > E::QCAP - E::G * PER_LANE) {
-                double wb = best;
+            double wb = best;
 #pragma unroll
-                for (int o = E::G / 2; o > 0; o >>= 1) wb = fmin(wb, shfl_xor_h(hm, wb, o));
-                enum_flush<NTX, SQM>(ws, wb);
-            }
+            for (int o = E::G / 2; o > 0; o >>= 1) wb = fmin(wb, shfl_xor_h(hm, wb, o));
+            enum_flush<NTX, SQM>(ws, wb, cnt);
+            cnt = 0;
         }
     }
 
@@ -744,10 +755,42 @@ struct Scan {
     __device__ __forceinline__ void inner(const cplx (&acc)[NTX], double base, int code, cplx r01, bool dead) {
         dead = dead || (prune && base > lim);
         if constexpr (S_ == 0) {
-            if (!dead) leaf(acc[0], base, code);
+            leaf(acc[0], base, code, !dead);
+        } else if constexpr (S_ == 1 && M % E::G == 0) {
+            // Innermost node level, packed (half-warp groups: M is 16 or 64).  The group takes its live nodes one
+            // after the other, in lane order, and its G lanes split the M stream-1 symbols below each one, G per
+            // step, a leaf node per lane.  At operating SNRs one or two of 16 lanes are live here, and each costs
+            // one step instead of the whole group walking M nodes in lock-step for it.
+            // After every step the group merges its incumbent.  So the incumbent, the enqueue limit, the queued
+            // nodes, their order (lane order within a step) and the flush points change only in steps that hold a
+            // live node, and a step is the same slice of one node's children at the same lanes whether dead nodes
+            // are skipped or not: the pruned walk and the full scan run the same live steps in the same order.
+            const unsigned hm = E::gmask();
+            unsigned todo = __ballot_sync(hm, !dead) >> E::gshift();
+            while (todo != 0u) {
+                const int src = __ffs(todo) - 1;
+                todo &= todo - 1u;
+                cplx pacc[NTX];   // the node's residuals; rows above 1 are not read
+#pragma unroll
+                for (int i = 0; i < NTX; ++i)
+                    pacc[i] = i <= 1 ? mk(__shfl_sync(hm, acc[i].x, src, E::G), __shfl_sync(hm, acc[i].y, src, E::G))
+                                     : acc[i];
+                const double pbase = __shfl_sync(hm, base, src, E::G);
+                const int pcode = __shfl_sync(hm, code, src, E::G);
+#pragma unroll 1
+                for (int m = E::glane(); m < M; m += E::G) {
+                    cplx nacc[NTX];
+                    const double nb = E::step(pacc, nacc, 1, m, pbase, g, tab);
+                    const double b0 = best;
+                    inner<0>(nacc, nb, pcode + (m << (E::BITS * (NTX - 2))), r01, false);
+                    if (__any_sync(hm, best != b0)) merge_best();
+                    maybe_flush<1>();
+                }
+            }
         } else if constexpr (S_ == 1) {
             if (__all_sync(E::gmask(), dead)) return;
-            // innermost node level: |u_1|^2 and R_01 x_1 are separable in the in-phase / quadrature indices.
+            // innermost node level, every lane its own node (warp groups: M < G).  |u_1|^2 and R_01 x_1 are
+            // separable in the in-phase / quadrature indices.
             // The queue is checked once per node (its M leaves per lane) when that fits, else once per row of SQM.
             constexpr bool NODE_FLUSH = E::G * M < E::QCAP;
             const double* g1 = g + SQM;
@@ -769,13 +812,11 @@ struct Scan {
                 // t = acc0 - pQ * (i r01) = acc0 - pQ*(-r01.y + i r01.x)
                 const cplx tq = mk(fma(pQ, r01.y, acc[0].x), fma(-pQ, r01.x, acc[0].y));
                 const int cq = code + ((iQ * SQM) << (E::BITS * (NTX - 2)));
-                if (!deadq) {
 #pragma unroll
-                    for (int iI = 0; iI < SQM; ++iI) {
-                        const double pI = E::pam(iI);
-                        const cplx t0 = mk(fma(-pI, r01.x, tq.x), fma(-pI, r01.y, tq.y));
-                        leaf(t0, bq + dI1[iI], cq + (iI << (E::BITS * (NTX - 2))));
-                    }
+                for (int iI = 0; iI < SQM; ++iI) {
+                    const double pI = E::pam(iI);
+                    const cplx t0 = mk(fma(-pI, r01.x, tq.x), fma(-pI, r01.y, tq.y));
+                    leaf(t0, bq + dI1[iI], cq + (iI << (E::BITS * (NTX - 2))), !deadq);
                 }
                 if (!NODE_FLUSH) maybe_flush<SQM>();
             }
@@ -881,7 +922,6 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         ws[E::O_C0] = c0;
         ws[E::O_AREF] = 1e300;
         ws[E::O_S2] = inv_s2;
-        *(int*)(ws + E::O_CNT) = 0;
     }
     for (int i = gl; i < E::NACC; i += E::G) ws[E::O_ACC + i] = 0.0;
     __syncwarp(E::gmask());
@@ -892,6 +932,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
     sc.g = g;
     sc.r0 = r00;
     sc.thr = SBCE_THR * s2;
+    sc.cnt = 0;
     sc.prune = (d.flags & SBCE_FLAG_FULL_SCAN) == 0;
     // Babai point (successive slicing): a tight upper bound on min d2 -> incumbent
     {
@@ -919,7 +960,7 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
     // levels to find every lane dead; it is dropped from the group's list of live rounds (16-QAM on 3+ streams and
     // QPSK on 4+: one top symbol per round).  Dead under the initial bound implies dead under any later (tighter)
     // one, and a dead round contributes nothing in either mode, so the sequence of visited live nodes -- hence
-    // the queue order and every output bit -- is unchanged.
+    // the queue order and every output bit -- is unchanged (Scan::packed for the levels below the prefixes).
     constexpr int NROUND = (E::NPREF + E::G - 1) / E::G;
     static_assert(NROUND <= 32, "one bit per round");
     unsigned live = NROUND == 32 ? 0xffffffffu : (1u << NROUND) - 1u;
@@ -944,26 +985,23 @@ __global__ void __launch_bounds__(WARPS * 32, (NTX > 4 ? 2 : 4)) k_enum(Dims d, 
         live &= live - 1u;
         const int p = pb + gl;
         const bool valid = p < E::NPREF;
-        sc.template prefix<NTX - 1, E::PL>(yt, c0, 0, valid ? p : 0, r01, !valid);
+        // ytilde and c0 come from the shared block: held in registers across the walk, they spilled
+        cplx acc[NTX];
+#pragma unroll
+        for (int i = 0; i < NTX; ++i) acc[i] = mk(ws[E::O_YT + 2 * i], ws[E::O_YT + 2 * i + 1]);
+        sc.template prefix<NTX - 1, E::PL>(acc, ws[E::O_C0], 0, valid ? p : 0, r01, !valid);
     }
 
-    // ---- group merge of the incumbent ------------------------------------------
-    double best = sc.best;
-    int bestk = sc.bestk;
-    const unsigned hm = E::gmask();   // (recomputed here rather than held in a register across the scan)
-#pragma unroll
-    for (int o = E::G / 2; o > 0; o >>= 1) {
-        const double ob = shfl_xor_h(hm, best, o);
-        const int ok = __shfl_xor_sync(hm, bestk, o);
-        if (ob < best || (ob == best && ok < bestk)) { best = ob; bestk = ok; }
-    }
+    sc.merge_best();
+    const double best = sc.best;
+    const int bestk = sc.bestk;
     const size_t sidx = (size_t)b * d.T_d + t;
     if (kstar != nullptr && gl == 0) kstar[sidx] = bestk;
 
     bool collapsed = HARD;
     double S = 0.0;
     if (!HARD) {
-        enum_flush<NTX, SQM>(ws, best);
+        enum_flush<NTX, SQM>(ws, best, sc.cnt);
         S = ws[E::O_ACC];
         // Nothing within 64 varn^2 of the incumbent was queued: only happens when |d2| is so large that
         // its rounding error exceeds the window (e.g. a garbage start vector of norm 1e13); every weight
