@@ -222,6 +222,44 @@ int sbce_ls_start(const sbce_cfg* cfg, const sbce_io* io, double* theta0, int32_
 int sbce_accumulate_ser(const sbce_cfg* cfg, const int32_t* kstar, const double* Xd_true, int32_t batch, double* acc,
                         void* stream);
 
+/* ---- bit level: exact Gray-labelled bit LLRs at a channel estimate, and bit-error counts ----------------
+ * Labelling.  Constellation index m = iQ*sqrt(M) + iI; with q = log2 sqrt(M) and gray(a) = a ^ (a >> 1), the
+ * log2 M bits of m are gray(iI) MSB first, then gray(iQ) MSB first (QPSK: [iI, iQ], bit 0 <-> level -1).
+ * Adjacent PAM levels differ in one bit on each axis.  The reference's vendored QAM.py carries a labelling
+ * of its own that no script uses, so no reference output pins this one.
+ *
+ * LLR.  llr[b][t][j][i] = ln sum_{k: bit i of stream j = 0} exp(-d2_k/varn^2)
+ *                       - ln sum_{k: bit i of stream j = 1} exp(-d2_k/varn^2),
+ * float64, [B][T_d][n_tx][log2 M]; positive means 0 is more likely, hard bit = (llr < 0).  The prior is
+ * uniform and the exponent is the E-step's own d2/varn^2 (quirk Q1), so these are the LLRs of the posterior
+ * the EM iterates on; a caller who wants the exponent d2/varn passes sqrt(varn).
+ *
+ * Window and clamp.  The walk skips subtrees whose partial distance exceeds min_k d2_k + 96 varn^2, and the
+ * result is clamped to [-SBCE_LLR_CLAMP, SBCE_LLR_CLAMP].  Weights are measured relative to the best
+ * hypothesis (weight 1).  With K <= 2^24 hypotheses the skipped part of either sum is at most K e^-96; the
+ * larger side holds at least half the total, so at least 1/2, and whenever the true |llr| < 32 the smaller
+ * side holds at least e^-32 / 2.  The relative error of either sum, hence the absolute error of the LLR, is
+ * below 2 * 2^24 * e^-64 < 1e-20 -- the same e^-64 margin the E-step's window gives its sums.  Whenever the
+ * true |llr| >= 32 the result is exactly +-32.  SBCE_FLAG_FULL_SCAN disables the window.
+ *
+ * Every LLR of a symbol whose QR record (effective channel and observation) is not finite is NaN, not a
+ * clamp; no other symbol or trial changes. */
+#define SBCE_LLR_CLAMP 32
+
+/* Bit LLRs of every data symbol at `theta` (device pointers): reads io->Yd, PsiD, varn, and io->Xp (the
+ * offsets) with SBCE_FLAG_SUPERIMPOSED, whose LLRs are those of the data bits.  Honours SBCE_FLAG_PSI_SHARED
+ * and SBCE_FLAG_FULL_SCAN.  cfg->mode must be SBCE_MODE_SOFT or SBCE_MODE_HARD (both give the same LLRs);
+ * the shapes are those of the exhaustive tree (1-4 streams of 4/16/64-QAM, 5-8 of QPSK, 5-6 of 16-QAM: at
+ * most 24 LLRs per symbol).  llr [B][T_d][n_tx][log2 M] float64.  Workspace as the E-step's. */
+int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* llr, void* workspace,
+                 size_t workspace_bytes, void* stream);
+
+/* Bit-error accumulation for the BER curves: acc[0] += bit errors between the labels of the kstar digits
+ * and of Xd_true, acc[1] += bits compared.  Same arguments and limits as sbce_accumulate_ser; acc is 2
+ * float64 on the device. */
+int sbce_accumulate_ber(const sbce_cfg* cfg, const int32_t* kstar, const double* Xd_true, int32_t batch, double* acc,
+                        void* stream);
+
 /* Measured FP64 FMA throughput of the current device (TFLOP/s, 2 flops per
  * FMA), used as the roofline denominator for the FP64-bound kernels. */
 int sbce_measure_fp64_peak(double* tflops, double* seconds);

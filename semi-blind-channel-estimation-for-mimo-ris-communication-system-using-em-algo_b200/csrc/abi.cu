@@ -421,6 +421,45 @@ int sbce_accumulate_ser(const sbce_cfg* cfg, const int32_t* kstar, const double*
     return 0;
 }
 
+int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* llr, void* workspace,
+                 size_t workspace_bytes, void* stream) {
+    if (!cfg) return SBCE_E_NULL;
+    // the LLRs are sums over the exhaustive tree: the partitioned and detector modes have none
+    if (cfg->mode != SBCE_MODE_SOFT && cfg->mode != SBCE_MODE_HARD) return SBCE_E_UNSUPPORTED;
+    Dims d;
+    int rc = make_dims(cfg, &d);
+    if (rc) return rc;
+    if (!io || !io->Yd || !io->PsiD || !io->varn || !theta || !llr || !workspace) return SBCE_E_NULL;
+    const bool sup = (d.flags & SBCE_FLAG_SUPERIMPOSED) != 0;
+    if (sup && !io->Xp) return SBCE_E_NULL;
+    if (cfg->batch == 0) return 0;
+    const int chunk = trials_fitting(d, workspace_bytes, cfg->batch);
+    if (chunk < 1) return SBCE_E_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    for (int b0 = 0; b0 < cfg->batch; b0 += chunk) {
+        const int nb = (cfg->batch - b0 < chunk) ? cfg->batch - b0 : chunk;
+        Workspace ws;
+        carve_workspace(d, nb, workspace, &ws);
+        sbce_io o = offset_io(d, *io, (size_t)b0);
+        // the record holds y - Heff o_t with superimposed pilots: the LLRs are those of the data bits
+        CK(launch_heff_qr(d, nb, o.Yd, o.PsiD, theta + (size_t)b0 * d.L * d.n_rx * 2, nullptr, sup ? o.Xp : nullptr,
+                          ws.qr, s));
+        CK(launch_bit_llr(d, nb, ws.qr, o.varn, llr + (size_t)b0 * d.T_d * d.n_tx * d.bitsM, s));
+    }
+    return 0;
+}
+
+int sbce_accumulate_ber(const sbce_cfg* cfg, const int32_t* kstar, const double* Xd_true, int32_t batch, double* acc,
+                        void* stream) {
+    Dims d;
+    int rc = make_dims(cfg, &d, false);
+    if (rc) return rc;
+    if (!kstar || !Xd_true || !acc) return SBCE_E_NULL;
+    if (d.n_tx * d.bitsM > 30) return SBCE_E_UNSUPPORTED;
+    CK(launch_accumulate_ber(d, batch, kstar, Xd_true, acc, (cudaStream_t)stream));
+    return 0;
+}
+
 int sbce_measure_fp64_peak(double* tflops, double* seconds) {
     CK(run_fp64_peak(tflops, seconds));
     return 0;

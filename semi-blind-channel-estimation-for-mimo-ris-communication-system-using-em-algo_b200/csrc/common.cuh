@@ -147,6 +147,10 @@ cudaError_t launch_ls_start(const Dims& d, int nb, const sbce_io& io, double* th
                             cudaStream_t s);
 cudaError_t launch_accumulate_ser(const Dims& d, int nb, const int32_t* kstar, const double* Xd, double* acc,
                                   cudaStream_t s);
+cudaError_t launch_accumulate_ber(const Dims& d, int nb, const int32_t* kstar, const double* Xd, double* acc,
+                                  cudaStream_t s);
+// bit LLRs (llr.cu): qr as written by launch_heff_qr, llr [nb][T_d][n_tx][log2 M]
+cudaError_t launch_bit_llr(const Dims& d, int nb, const double* qr, const double* varn, double* llr, cudaStream_t s);
 
 void count_launch(int n = 1);
 

@@ -344,6 +344,43 @@ __global__ void k_accumulate_ser(Dims d, int nb, const int32_t* __restrict__ kst
 }
 
 // ---------------------------------------------------------------------------
+// bit-error accumulation on the device (BER curves): Gray labels of include/sbce.h, per stream gray(iI) then
+// gray(iQ).  acc[0] += bit errors, acc[1] += bits compared.  Counts are integers, so the atomics' order does
+// not matter.
+// ---------------------------------------------------------------------------
+__global__ void k_accumulate_ber(Dims d, int nb, const int32_t* __restrict__ kstar, const cplx* __restrict__ Xd,
+                                 double* __restrict__ acc) {
+    const int b = blockIdx.x;
+    if (b >= nb) return;
+    const int hb = d.bitsM / 2, top = d.sqM - 1;
+    auto gray = [](int a) { return a ^ (a >> 1); };
+    // PAM index of a level 2a - sqrt(M) + 1 (the true symbols are exact constellation points)
+    auto level = [&](double v) { return min(max((int)lround(0.5 * (v + top)), 0), top); };
+    double err = 0.0;
+    for (int t = threadIdx.x; t < d.T_d; t += blockDim.x) {
+        const int k = kstar[(size_t)b * d.T_d + t];
+        const cplx* x = Xd + ((size_t)b * d.T_d + t) * d.n_tx;
+        for (int j = 0; j < d.n_tx; ++j) {
+            const int m = (k >> (d.bitsM * (d.n_tx - 1 - j))) & (d.M - 1);
+            const int lab = (gray(m >> hb) << hb) | gray(m & top);   // label as an integer, Q bits low
+            const int tru = (gray(level(x[j].y)) << hb) | gray(level(x[j].x));
+            err += (double)__popc(lab ^ tru);
+        }
+    }
+    err = warp_sum(err);
+    __shared__ double se[32];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (lane == 0) se[warp] = err;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double e2 = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) e2 += se[w];
+        atomicAdd(&acc[0], e2);
+        atomicAdd(&acc[1], (double)d.T_d * d.n_tx * d.bitsM);
+    }
+}
+
+// ---------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------
 static GenKey make_key(const sbce_gen* g) {
@@ -447,6 +484,14 @@ cudaError_t launch_accumulate_ser(const Dims& d, int nb, const int32_t* kstar, c
                                   cudaStream_t s) {
     if (nb == 0) return cudaSuccess;
     k_accumulate_ser<<<nb, 128, 0, s>>>(d, nb, kstar, (const cplx*)Xd, acc);
+    count_launch();
+    return cudaGetLastError();
+}
+
+cudaError_t launch_accumulate_ber(const Dims& d, int nb, const int32_t* kstar, const double* Xd, double* acc,
+                                  cudaStream_t s) {
+    if (nb == 0) return cudaSuccess;
+    k_accumulate_ber<<<nb, 128, 0, s>>>(d, nb, kstar, (const cplx*)Xd, acc);
     count_launch();
     return cudaGetLastError();
 }

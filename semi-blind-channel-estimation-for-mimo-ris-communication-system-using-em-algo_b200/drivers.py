@@ -20,7 +20,7 @@ from typing import Callable, List, Sequence
 import numpy as np
 
 from . import dist, engine, signal_model
-from .qam import symbols_of
+from .qam import bit_labels, bits_of, symbols_of
 
 
 @dataclass
@@ -58,10 +58,12 @@ class PointResult:
     sym_total: float = 0.0
     ser_coded_sum: float = 0.0    # sum over trials of the as-coded SER (log_max_SER.py:162)
     n_trials: float = 0.0
+    bit_err: float = 0.0          # bit errors between the Gray labels (qam.bit_labels) of decisions and data
+    bit_total: float = 0.0
 
     def vec(self):
         return np.array([self.nmse_sum, self.n_valid, self.n_flagged, self.sym_err, self.sym_total,
-                         self.ser_coded_sum, self.n_trials], dtype=np.float64)
+                         self.ser_coded_sum, self.n_trials, self.bit_err, self.bit_total], dtype=np.float64)
 
 
 SER_MODES = ("soft", "hard", "zf", "mmse")
@@ -82,7 +84,7 @@ def _ser_as_coded_batch(Xd, Xest):
 
 def run_point_device(cfg: SweepConfig, point_index: int, device=0, per_trial=None) -> PointResult:
     """run_point with everything on the GPU: Philox generation straight into the SoA layout, LS start,
-    EM, NMSE / SER accumulation; one 6-double read-back per sweep point.  Trial b of the point is the
+    EM, NMSE / SER / BER accumulation; one 8-double read-back per sweep point.  Trial b of the point is the
     same whatever the batch size or the number of ranks (counter-based generator)."""
     import torch
 
@@ -107,6 +109,7 @@ def run_point_device(cfg: SweepConfig, point_index: int, device=0, per_trial=Non
         ses = engine.DeviceSession(prob, inflight, device=dev)
         acc_n = torch.zeros(3, dtype=torch.float64, device=dev)
         acc_s = torch.zeros(3, dtype=torch.float64, device=dev)
+        acc_b = torch.zeros(2, dtype=torch.float64, device=dev)
         for b0 in range(lo, hi, cfg.max_batch):
             nb = min(cfg.max_batch, hi - b0)
             tb = ses.generate(nb, cfg.varn, seed=cfg.seed * 1000003 + point_index, trial0=b0, pilot_design=pilot,
@@ -116,13 +119,15 @@ def run_point_device(cfg: SweepConfig, point_index: int, device=0, per_trial=Non
                           h_true=tb["h"])
             if st0 is not None:
                 res.status.bitwise_or_(st0)   # a rank-deficient pilot block flags the trial
-            ses.accumulate(res, tb["Xd"], acc_n, acc_s if cfg.mode in SER_MODES else None)
+            decides = cfg.mode in SER_MODES
+            ses.accumulate(res, tb["Xd"], acc_n, acc_s if decides else None, acc_b if decides else None)
             if per_trial is not None:
                 per_trial[b0:b0 + nb] = res.nmse.cpu().numpy()
             acc.n_trials += nb
-        a, c = acc_n.cpu().numpy(), acc_s.cpu().numpy()
+        a, c, e = acc_n.cpu().numpy(), acc_s.cpu().numpy(), acc_b.cpu().numpy()
     acc.nmse_sum, acc.n_valid, acc.n_flagged = float(a[0]), float(a[1]), float(a[2])
     acc.sym_err, acc.sym_total, acc.ser_coded_sum = float(c[0]), float(c[1]), float(c[2])
+    acc.bit_err, acc.bit_total = float(e[0]), float(e[1])
     return acc
 
 
@@ -159,12 +164,15 @@ def run_point(cfg: SweepConfig, point_index: int, runner: Callable = None, devic
             acc.sym_err += float(np.count_nonzero(tb.Xd - xest))
             acc.sym_total += float(tb.Xd.size)
             acc.ser_coded_sum += float(_ser_as_coded_batch(tb.Xd, xest).sum())
+            bits_est = bits_of(np.asarray(res.kstar), cfg.M, cfg.n_tx)
+            acc.bit_err += float(np.count_nonzero(bits_est != bit_labels(cfg.M)[tb.idx_d]))
+            acc.bit_total += float(bits_est.size)
     return acc
 
 
 def _finish(xs, accs: List[PointResult], per_trial=None, device=None):
     """Cross-rank sum of the per-point accumulators (the one collective of a sweep, SNR/all_Detectors.py:389-395
-    averages over trials) and the averaged curves.  Points without symbol decisions report ser = NaN."""
+    averages over trials) and the averaged curves.  Points without symbol decisions report ser = ber = NaN."""
     mat = np.stack([a.vec() for a in accs])
     mat = dist.allreduce_sum(mat, device=device)
     with np.errstate(invalid="ignore", divide="ignore"):
@@ -174,7 +182,8 @@ def _finish(xs, accs: List[PointResult], per_trial=None, device=None):
                    n_valid=mat[:, 1], n_flagged=mat[:, 2],
                    ser=np.where(has_ser, mat[:, 3] / np.maximum(mat[:, 4], 1.0), np.nan),
                    ser_as_coded=np.where(has_ser, mat[:, 5] / np.maximum(mat[:, 6], 1.0), np.nan),
-                   n_trials=mat[:, 6])
+                   n_trials=mat[:, 6],
+                   ber=np.where(mat[:, 8] > 0, mat[:, 7] / np.maximum(mat[:, 8], 1.0), np.nan))
     if per_trial is not None:
         out["per_trial"] = per_trial
     return out
@@ -224,5 +233,6 @@ def detectors_vs_snr(cfg: SweepConfig, snr_db: Sequence[float], modes=("pm_beta"
 
 def ser_vs_snr(cfg: SweepConfig, snr_db: Sequence[float], runner=None, device=0):
     """Hard-decision EM symbol error rate vs SNR (log_max_SER.py:147-167): returns both the
-    as-coded figure (with the reference's broadcast) and the true per-stream SER."""
+    as-coded figure (with the reference's broadcast) and the true per-stream SER, and the bit error rate
+    of the same decisions under the Gray labels of qam.bit_labels (`ber`)."""
     return nmse_vs_snr(replace(cfg, mode="hard"), snr_db, runner, device)

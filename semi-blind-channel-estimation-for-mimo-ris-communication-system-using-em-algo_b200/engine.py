@@ -316,6 +316,32 @@ class DeviceSession:
                                            ks.data_ptr(), ls.data_ptr(), self.ws.data_ptr(), self.ws_bytes, stream))
         return m, R, ks, ls
 
+    def bit_llr(self, Yd, PsiD, theta, varn, Xp=None, out=None):
+        """Exact Gray-labelled bit LLRs of every data symbol at `theta` -> (B, T_d, n_tx, log2 M) float64 device
+        tensor (written into `out` when given): ln P(bit = 0) - ln P(bit = 1) under the E-step's posterior
+        (exponent d2/varn^2, uniform prior), clamped to [-32, 32]; NaN for a symbol whose inputs are not finite.
+        Conventions: include/sbce.h (sbce_bit_llr), labels: qam.bit_labels.  Soft and hard modes only (both
+        give the same LLRs).  With Problem.superimposed the offsets Xp [B][T_d][n_tx] are required."""
+        torch, p = self.torch, self.prob
+        if p.mode not in ("soft", "hard"):
+            raise ValueError("bit LLRs are defined for the soft and hard modes, not %r" % (p.mode,))
+        B = int(Yd.shape[0])
+        if p.superimposed and Xp is None:
+            raise ValueError("superimposed pilots: bit_llr() needs the offsets Xp [B][T_d][n_tx]")
+        io = self._io(B, Yd, None, PsiD, None, Xp if p.superimposed else None, varn, None, None, None)
+        dev = self.device
+        shape = (B, p.T_d, p.n_tx, int(math.log2(p.M)))
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float64, device=dev)
+        self._check(out, shape, "out", torch.float64)
+        self._check(theta, (B, p.L, p.n_rx), "theta", torch.complex128)
+        cfg = p.cfg(B)
+        with self._on_device():
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(self.lib.sbce_bit_llr(C.byref(cfg), C.byref(io), theta.data_ptr(), out.data_ptr(),
+                                             self.ws.data_ptr(), self.ws_bytes, stream))
+        return out
+
     def mstep(self, Yd, Yp, PsiD, PsiP, Xp, stat_m, stat_R):
         """Stand-alone M-step from given data statistics -> (theta, status)."""
         torch, p = self.torch, self.prob
@@ -383,16 +409,18 @@ class DeviceSession:
                                               self.ws.data_ptr(), self.ws_bytes, stream))
         return theta0, status
 
-    def accumulate(self, res: "Result", Xd, acc_nmse, acc_ser=None):
+    def accumulate(self, res: "Result", Xd, acc_nmse, acc_ser=None, acc_ber=None):
         """Adds this batch to the per-point device accumulators: acc_nmse (3 float64: sum NMSE over valid
-        trials, valid count, flagged count), acc_ser (3 float64: symbol errors, symbols, sum of as-coded SER)."""
+        trials, valid count, flagged count), acc_ser (3 float64: symbol errors, symbols, sum of as-coded SER),
+        acc_ber (2 float64: bit errors between the Gray labels of the decisions and of Xd, bits compared)."""
         torch, p = self.torch, self.prob
         B = int(res.theta.shape[0])
         if res.nmse is None:
             raise ValueError("accumulate() needs Result.nmse: run(..., h_true=...) computes it")
         # joint decisions exist in the exhaustive and detector modes only (PM modes report kstar = -1)
-        ser_ok = (acc_ser is not None and res.kstar is not None and p.mode in ("soft", "hard", "zf", "mmse")
-                  and p.n_tx * int(math.log2(p.M)) <= 30)
+        decides = (res.kstar is not None and p.mode in ("soft", "hard", "zf", "mmse")
+                   and p.n_tx * int(math.log2(p.M)) <= 30)
+        ser_ok = acc_ser is not None and decides
         with self._on_device():
             stream = torch.cuda.current_stream(self.device).cuda_stream
             _lib.check(self.lib.sbce_accumulate_nmse(res.nmse.data_ptr(),
@@ -402,6 +430,9 @@ class DeviceSession:
                 cfg = p.cfg(B)
                 _lib.check(self.lib.sbce_accumulate_ser(C.byref(cfg), res.kstar.data_ptr(), Xd.data_ptr(), B,
                                                         acc_ser.data_ptr(), stream))
+            if acc_ber is not None and decides:
+                _lib.check(self.lib.sbce_accumulate_ber(C.byref(p.cfg(B)), res.kstar.data_ptr(), Xd.data_ptr(), B,
+                                                        acc_ber.data_ptr(), stream))
 
 
 def fp64_peak_tflops():

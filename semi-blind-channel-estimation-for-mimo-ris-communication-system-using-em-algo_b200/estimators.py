@@ -225,6 +225,40 @@ def em_mmse(Y_d, Y_p, T_d, T_p, Z_p, PsiTilde_td, all_possibleSymbols, M, varn, 
     return res.theta.reshape(-1, 1)
 
 
+def bit_llr(Y_d, PsiTilde_td, theta, M, varn, n_tx, *, X_p=None, device=0):
+    """Exact Gray-labelled bit LLRs of the data symbols at the estimate `theta` (the (D,1) vector em() returns),
+    in the reference's data conventions: Y_d the list of (n_rx,1) observations, PsiTilde_td the (N+1, T_d) phases
+    with the direct-link ones row.  X_p (list of (n_tx,1) pilot symbols): the parallel protocol's superimposed
+    pilots, added to the data of the first len(X_p) symbols (em_parallel).  Returns (T_d, n_tx * log2 M)
+    float64: ln P(bit = 0) - ln P(bit = 1) under the E-step's posterior (exponent d2/varn^2, uniform prior),
+    clamped to [-32, 32], bits in the order of qam.bit_labels per stream, stream 0 first."""
+    import torch
+
+    if M not in SUPPORTED_M:
+        raise ValueError("M must be one of %s" % (SUPPORTED_M,))
+    Yd = _stack_cols(Y_d)
+    T_d, n_rx = Yd.shape
+    PsiD = np.asarray(PsiTilde_td, dtype=np.complex128).T.copy()
+    if PsiD.shape[0] != T_d:
+        raise ValueError("PsiTilde_td has %d columns, Y_d %d symbols" % (PsiD.shape[0], T_d))
+    N1 = PsiD.shape[1]
+    L = N1 * n_tx
+    th = np.asarray(theta, dtype=np.complex128).reshape(1, L, n_rx)
+    Xoff = None
+    if X_p is not None:
+        Xoff = np.zeros((1, T_d, n_tx), dtype=np.complex128)
+        if len(X_p):
+            Xoff[0, :len(X_p)] = _stack_cols(X_p)
+    prob = engine.Problem(N=N1 - 1, n_tx=n_tx, n_rx=n_rx, M=M, T_p=0, T_d=T_d, itera=1,
+                          superimposed=Xoff is not None)
+    dev = torch.device("cuda", device)
+    ses = engine.DeviceSession(prob, 1, device=dev)
+    t = lambda a: None if a is None else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+    out = ses.bit_llr(t(Yd[None]), t(PsiD[None]), t(th), torch.full((1,), float(varn), dtype=torch.float64, device=dev),
+                      Xp=t(Xoff))
+    return out.cpu().numpy().reshape(T_d, -1)
+
+
 def nmse(theta_hat, h):
     """Proposed_method_NMSEvsTp.py:138."""
     a = np.asarray(theta_hat).reshape(-1)

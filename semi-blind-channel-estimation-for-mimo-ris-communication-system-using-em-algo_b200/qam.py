@@ -34,6 +34,26 @@ def symbols_of(k, M: int, n_tx: int) -> np.ndarray:
     return constellation(M)[digits_of(k, M, n_tx)]
 
 
+def bit_labels(M: int) -> np.ndarray:
+    """(M, log2 M) uint8 Gray labels of the constellation indices (include/sbce.h, sbce_bit_llr): with
+    m = iQ*sqrt(M) + iI and gray(a) = a ^ (a >> 1), the bits of m are gray(iI) MSB first, then gray(iQ) MSB
+    first -- [iI, iQ] for QPSK, one bit between adjacent PAM levels on each axis.  The reference's vendored
+    QAM.py carries a labelling of its own that no script uses, so no reference output pins this convention."""
+    constellation(M)   # validates M
+    q = int(round(np.log2(M))) // 2
+    sq = 1 << q
+    m = np.arange(M)
+    gi, gq = (m % sq) ^ ((m % sq) >> 1), (m // sq) ^ ((m // sq) >> 1)
+    shifts = np.arange(q - 1, -1, -1)
+    bits = np.concatenate([(gi[:, None] >> shifts) & 1, (gq[:, None] >> shifts) & 1], axis=1)
+    return np.ascontiguousarray(bits, dtype=np.uint8)
+
+
+def bits_of(k, M: int, n_tx: int) -> np.ndarray:
+    """(..., n_tx, log2 M) uint8 labels of joint hypothesis indices k (the layout of the bit LLRs)."""
+    return bit_labels(M)[digits_of(k, M, n_tx)]
+
+
 def constellation_from_table(all_possibleSymbols, M: int) -> np.ndarray:
     """Recover the per-stream constellation from the reference's (K, n_tx) table."""
     tab = np.asarray(all_possibleSymbols)
