@@ -254,6 +254,43 @@ int sbce_accumulate_ser(const sbce_cfg* cfg, const int32_t* kstar, const double*
 int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* llr, void* workspace,
                  size_t workspace_bytes, void* stream);
 
+/* ---- bit LLRs with a-priori input: extrinsic LLRs for iterative detection and decoding -----------------
+ * A-priori LLRs.  La[b][t][j][i] = ln P(bit = 0) - ln P(bit = 1) from a channel decoder, in the layout and
+ * labelling of llr; on read each is clamped to +-SBCE_LLR_CLAMP (an infinite prior counts as +-32).
+ *
+ * Metric.  A bit taking value v costs pen(v) = max(0, (2v - 1) La): nothing when it agrees with the prior's
+ * hard decision, |La| when it does not.  Stream j's symbol m costs P_j(m) = sum_i pen(bit_i(m)) >= 0, and
+ * min_m P_j(m) = 0 since the labelling is a bijection onto all bit patterns.  Hypothesis k has the metric
+ *     mu_k = d2_k + varn^2 sum_j P_j(x_j),
+ * and exp(-mu_k/varn^2) is its posterior under the prior up to a constant.  The penalties are non-negative and
+ * belong to single tree levels, so partial metrics stay lower bounds along the tree; and since the Gray label
+ * puts the in-phase bits on iI and the quadrature bits on iQ, P_0(m) = P_0I(iI) + P_0Q(iQ) and stream 0 keeps
+ * its closed form as separable in-phase / quadrature PAM weights.
+ *
+ * Extrinsic LLR.  llr_ext = ln S0 - ln S1 - La (La clamped), clamped to [-SBCE_LLR_CLAMP, SBCE_LLR_CLAMP], where
+ * S0, S1 are both sides of the bit under mu, each accumulated explicitly.  An empty side gives +-inf before the
+ * clamp, so exactly +-32.  With La = 0 this is sbce_bit_llr bit for bit: extrinsic and a-posteriori LLRs
+ * coincide without a prior.
+ *
+ * Window.  The walk skips subtrees whose partial metric exceeds min_k mu_k + (96 + A) varn^2, A the largest
+ * clamped |La| of the symbol (A = 0: sbce_bit_llr's window).  Whenever the true |llr_ext| < 32, the posterior
+ * LLR is below 32 + A in magnitude, so the smaller side holds at least e^-(32+A) / 2 of the best hypothesis's
+ * weight while the skipped part is at most K e^-(96+A), K <= 2^24: the relative error of either sum, hence the
+ * absolute error of llr_ext, is again below 2 * 2^24 * e^-64 < 1e-20.  A side the window leaves empty holds
+ * at most K e^-(96+A) against at least 1 on the other, so the posterior LLR exceeds 96 + A - ln 2^24 in
+ * magnitude, |llr_ext| > 78, and the clamp makes the result exactly +-32.
+ * SBCE_FLAG_FULL_SCAN disables the window.
+ *
+ * Non-finite input.  A NaN anywhere in a symbol's La, like a non-finite QR record, makes all of that symbol's
+ * outputs NaN; no other symbol changes. */
+
+/* sbce_bit_llr with a-priori LLRs llr_a (required) -> extrinsic LLRs llr_ext, both [B][T_d][n_tx][log2 M]
+ * float64 on the device.  Checks, shapes, modes, flags (SBCE_FLAG_PSI_SHARED, SBCE_FLAG_FULL_SCAN,
+ * SBCE_FLAG_SUPERIMPOSED), chunking and workspace are those of sbce_bit_llr.  llr_ext may be llr_a: each
+ * symbol's priors are read before its outputs are written, so a turbo loop can update its LLRs in place. */
+int sbce_bit_llr_apriori(const sbce_cfg* cfg, const sbce_io* io, const double* theta, const double* llr_a,
+                         double* llr_ext, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Bit-error accumulation for the BER curves: acc[0] += bit errors between the labels of the kstar digits
  * and of Xd_true, acc[1] += bits compared.  Same arguments and limits as sbce_accumulate_ser; acc is 2
  * float64 on the device. */

@@ -50,7 +50,8 @@ PHASES_KIND = {"random": 0, "dft": 1}
 EXPORTS = ["sbce_version", "sbce_error_string", "sbce_device_count", "sbce_workspace_bytes", "sbce_em_batch",
            "sbce_em_batch_host", "sbce_estep", "sbce_mstep", "sbce_accumulate_nmse", "sbce_measure_fp64_peak",
            "sbce_launch_count", "sbce_profile_begin", "sbce_profile_end", "sbce_generate_batch", "sbce_ls_start",
-           "sbce_accumulate_ser", "sbce_host_split_threshold", "sbce_bit_llr", "sbce_accumulate_ber"]
+           "sbce_accumulate_ser", "sbce_host_split_threshold", "sbce_bit_llr", "sbce_accumulate_ber",
+           "sbce_bit_llr_apriori"]
 
 LLR_CLAMP = 32.0   # SBCE_LLR_CLAMP: bit LLRs are clamped to [-32, 32]
 
@@ -86,6 +87,8 @@ def load():
     lib.sbce_accumulate_ser.argtypes = [C.POINTER(Cfg), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
     lib.sbce_bit_llr.argtypes = [C.POINTER(Cfg), C.POINTER(Io), C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                  C.c_void_p]
+    lib.sbce_bit_llr_apriori.argtypes = [C.POINTER(Cfg), C.POINTER(Io), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_size_t, C.c_void_p]
     lib.sbce_accumulate_ber.argtypes = [C.POINTER(Cfg), C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
     lib.sbce_measure_fp64_peak.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_double)]
     lib.sbce_profile_end.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int32]

@@ -421,8 +421,9 @@ int sbce_accumulate_ser(const sbce_cfg* cfg, const int32_t* kstar, const double*
     return 0;
 }
 
-int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* llr, void* workspace,
-                 size_t workspace_bytes, void* stream) {
+// sbce_bit_llr (prior = false, llr_a unused) and sbce_bit_llr_apriori
+static int run_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, bool prior, const double* llr_a,
+                       double* llr, void* workspace, size_t workspace_bytes, void* stream) {
     if (!cfg) return SBCE_E_NULL;
     // the LLRs are sums over the exhaustive tree: the partitioned and detector modes have none
     if (cfg->mode != SBCE_MODE_SOFT && cfg->mode != SBCE_MODE_HARD) return SBCE_E_UNSUPPORTED;
@@ -430,6 +431,7 @@ int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, do
     int rc = make_dims(cfg, &d);
     if (rc) return rc;
     if (!io || !io->Yd || !io->PsiD || !io->varn || !theta || !llr || !workspace) return SBCE_E_NULL;
+    if (prior && !llr_a) return SBCE_E_NULL;
     const bool sup = (d.flags & SBCE_FLAG_SUPERIMPOSED) != 0;
     if (sup && !io->Xp) return SBCE_E_NULL;
     if (cfg->batch == 0) return 0;
@@ -444,9 +446,23 @@ int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, do
         // the record holds y - Heff o_t with superimposed pilots: the LLRs are those of the data bits
         CK(launch_heff_qr(d, nb, o.Yd, o.PsiD, theta + (size_t)b0 * d.L * d.n_rx * 2, nullptr, sup ? o.Xp : nullptr,
                           ws.qr, s));
-        CK(launch_bit_llr(d, nb, ws.qr, o.varn, llr + (size_t)b0 * d.T_d * d.n_tx * d.bitsM, s));
+        const size_t off = (size_t)b0 * d.T_d * d.n_tx * d.bitsM;
+        if (prior)
+            CK(launch_bit_llr_apriori(d, nb, ws.qr, o.varn, llr_a + off, llr + off, s));
+        else
+            CK(launch_bit_llr(d, nb, ws.qr, o.varn, llr + off, s));
     }
     return 0;
+}
+
+int sbce_bit_llr(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* llr, void* workspace,
+                 size_t workspace_bytes, void* stream) {
+    return run_bit_llr(cfg, io, theta, false, nullptr, llr, workspace, workspace_bytes, stream);
+}
+
+int sbce_bit_llr_apriori(const sbce_cfg* cfg, const sbce_io* io, const double* theta, const double* llr_a,
+                         double* llr_ext, void* workspace, size_t workspace_bytes, void* stream) {
+    return run_bit_llr(cfg, io, theta, true, llr_a, llr_ext, workspace, workspace_bytes, stream);
 }
 
 int sbce_accumulate_ber(const sbce_cfg* cfg, const int32_t* kstar, const double* Xd_true, int32_t batch, double* acc,

@@ -151,6 +151,9 @@ cudaError_t launch_accumulate_ber(const Dims& d, int nb, const int32_t* kstar, c
                                   cudaStream_t s);
 // bit LLRs (llr.cu): qr as written by launch_heff_qr, llr [nb][T_d][n_tx][log2 M]
 cudaError_t launch_bit_llr(const Dims& d, int nb, const double* qr, const double* varn, double* llr, cudaStream_t s);
+// ... with a-priori LLRs la (same layout; llr may be la), writing the extrinsic LLRs
+cudaError_t launch_bit_llr_apriori(const Dims& d, int nb, const double* qr, const double* varn, const double* la,
+                                   double* llr, cudaStream_t s);
 
 void count_launch(int n = 1);
 

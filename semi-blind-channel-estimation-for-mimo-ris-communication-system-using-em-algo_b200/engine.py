@@ -316,12 +316,17 @@ class DeviceSession:
                                            ks.data_ptr(), ls.data_ptr(), self.ws.data_ptr(), self.ws_bytes, stream))
         return m, R, ks, ls
 
-    def bit_llr(self, Yd, PsiD, theta, varn, Xp=None, out=None):
+    def bit_llr(self, Yd, PsiD, theta, varn, Xp=None, out=None, llr_a=None):
         """Exact Gray-labelled bit LLRs of every data symbol at `theta` -> (B, T_d, n_tx, log2 M) float64 device
         tensor (written into `out` when given): ln P(bit = 0) - ln P(bit = 1) under the E-step's posterior
         (exponent d2/varn^2, uniform prior), clamped to [-32, 32]; NaN for a symbol whose inputs are not finite.
         Conventions: include/sbce.h (sbce_bit_llr), labels: qam.bit_labels.  Soft and hard modes only (both
-        give the same LLRs).  With Problem.superimposed the offsets Xp [B][T_d][n_tx] are required."""
+        give the same LLRs).  With Problem.superimposed the offsets Xp [B][T_d][n_tx] are required.
+
+        llr_a: a-priori LLRs from a channel decoder, a float64 device tensor of the same shape (clamped to +-32 on
+        read; a NaN makes its symbol NaN).  Then the result is the extrinsic LLR, the posterior under that prior
+        minus llr_a (sbce_bit_llr_apriori), for iterative detection and decoding; `out` may be llr_a itself.  With
+        no prior the extrinsic and a-posteriori LLRs coincide: llr_a = 0 gives the same bits as llr_a=None."""
         torch, p = self.torch, self.prob
         if p.mode not in ("soft", "hard"):
             raise ValueError("bit LLRs are defined for the soft and hard modes, not %r" % (p.mode,))
@@ -335,11 +340,17 @@ class DeviceSession:
             out = torch.empty(shape, dtype=torch.float64, device=dev)
         self._check(out, shape, "out", torch.float64)
         self._check(theta, (B, p.L, p.n_rx), "theta", torch.complex128)
+        if llr_a is not None:
+            self._check(llr_a, shape, "llr_a", torch.float64)
         cfg = p.cfg(B)
         with self._on_device():
             stream = torch.cuda.current_stream(dev).cuda_stream
-            _lib.check(self.lib.sbce_bit_llr(C.byref(cfg), C.byref(io), theta.data_ptr(), out.data_ptr(),
-                                             self.ws.data_ptr(), self.ws_bytes, stream))
+            if llr_a is None:
+                _lib.check(self.lib.sbce_bit_llr(C.byref(cfg), C.byref(io), theta.data_ptr(), out.data_ptr(),
+                                                 self.ws.data_ptr(), self.ws_bytes, stream))
+            else:
+                _lib.check(self.lib.sbce_bit_llr_apriori(C.byref(cfg), C.byref(io), theta.data_ptr(), llr_a.data_ptr(),
+                                                         out.data_ptr(), self.ws.data_ptr(), self.ws_bytes, stream))
         return out
 
     def mstep(self, Yd, Yp, PsiD, PsiP, Xp, stat_m, stat_R):

@@ -225,13 +225,16 @@ def em_mmse(Y_d, Y_p, T_d, T_p, Z_p, PsiTilde_td, all_possibleSymbols, M, varn, 
     return res.theta.reshape(-1, 1)
 
 
-def bit_llr(Y_d, PsiTilde_td, theta, M, varn, n_tx, *, X_p=None, device=0):
+def bit_llr(Y_d, PsiTilde_td, theta, M, varn, n_tx, *, X_p=None, llr_a=None, device=0):
     """Exact Gray-labelled bit LLRs of the data symbols at the estimate `theta` (the (D,1) vector em() returns),
     in the reference's data conventions: Y_d the list of (n_rx,1) observations, PsiTilde_td the (N+1, T_d) phases
     with the direct-link ones row.  X_p (list of (n_tx,1) pilot symbols): the parallel protocol's superimposed
     pilots, added to the data of the first len(X_p) symbols (em_parallel).  Returns (T_d, n_tx * log2 M)
     float64: ln P(bit = 0) - ln P(bit = 1) under the E-step's posterior (exponent d2/varn^2, uniform prior),
-    clamped to [-32, 32], bits in the order of qam.bit_labels per stream, stream 0 first."""
+    clamped to [-32, 32], bits in the order of qam.bit_labels per stream, stream 0 first.  llr_a: a-priori LLRs
+    from a channel decoder in the same (T_d, n_tx * log2 M) layout; then the result is the extrinsic LLR (the
+    posterior under that prior minus llr_a, include/sbce.h: sbce_bit_llr_apriori), which equals the a-posteriori
+    LLR when there is no prior (llr_a = 0)."""
     import torch
 
     if M not in SUPPORTED_M:
@@ -254,8 +257,15 @@ def bit_llr(Y_d, PsiTilde_td, theta, M, varn, n_tx, *, X_p=None, device=0):
     dev = torch.device("cuda", device)
     ses = engine.DeviceSession(prob, 1, device=dev)
     t = lambda a: None if a is None else torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+    La = None
+    if llr_a is not None:
+        La = np.asarray(llr_a, dtype=np.float64)
+        nb = n_tx * int(np.log2(M))
+        if La.shape != (T_d, nb):
+            raise ValueError("llr_a has shape %s, expected (%d, %d)" % (La.shape, T_d, nb))
+        La = La.reshape(1, T_d, n_tx, -1)
     out = ses.bit_llr(t(Yd[None]), t(PsiD[None]), t(th), torch.full((1,), float(varn), dtype=torch.float64, device=dev),
-                      Xp=t(Xoff))
+                      Xp=t(Xoff), llr_a=t(La))
     return out.cpu().numpy().reshape(T_d, -1)
 
 
