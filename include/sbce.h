@@ -85,7 +85,9 @@ extern "C" {
                                    "Proposed method/all_detectorsvsTd.py":127 has it (PMvsMLvsZFvsMMSE.py:128 does not) */
 
 /* per-trial status bits */
-#define SBCE_ST_NOT_PD 1    /* non-positive pivot in the Cholesky of the normal matrix (singular M-step) */
+/* SBCE_ST_NOT_PD: the Cholesky of the normal matrix met a pivot that is not above 1e-13 times the largest pivot
+ * so far in the trial (a NaN pivot included; the identity padding rows are exempt): numerically singular M-step */
+#define SBCE_ST_NOT_PD 1
 #define SBCE_ST_NONFINITE 2 /* a non-finite value appeared in theta                                      */
 
 /* argument errors */
@@ -212,7 +214,8 @@ int sbce_generate_batch(const sbce_cfg* cfg, const sbce_gen* gen, const sbce_io*
 /* LS start h_initial = pinv(Z_p) y_p (PM.py:147) for every trial: min-norm solution through the
  * T_p x T_p Gram (Psi Psi^H) o (X X^H) when T_p < L, pilot normal equations when T_p >= L.
  * Reads io->Yp, PsiP, Xp; writes theta0 [B][L][n_rx]; status (nullable) gets SBCE_ST_NOT_PD for
- * rank-deficient pilot blocks (where pinv would invert rounding noise).  Workspace as sbce_em_batch. */
+ * rank-deficient pilot blocks (where pinv would invert rounding noise): a Cholesky pivot not above 1e-13 times the
+ * largest pivot so far, NaN included.  Workspace as sbce_em_batch. */
 int sbce_ls_start(const sbce_cfg* cfg, const sbce_io* io, double* theta0, int32_t* status, void* workspace,
                   size_t workspace_bytes, void* stream);
 

@@ -98,7 +98,8 @@ __device__ __forceinline__ void chol_diag_factor_reg(const Dims& d, cplx* A, int
         double piv = __shfl_sync(full, s.x, c, 16);
         const bool live = c < nb;
         if (live) {
-            // numerically singular: non-positive, or below 1e-13 of the largest pivot so far; identity padding exempt
+            // numerically singular: not above 1e-13 times the largest pivot so far in the trial (NaN included, and
+            // non-positive pivots whatever the maximum); the identity padding (k0 + c >= L) is exempt
             if (!(piv > ((k0 + c < d.L) ? 1e-13 * maxpiv : 0.0))) {
                 if (lane == 0) *s_bad = 1;
                 piv = 1.0;

@@ -19,8 +19,9 @@
 //    rows below the matrix, and the padding.
 //  * k_chol: one CTA per trial, LEFT-looking blocked complex Cholesky (panel width 16) on the augmented
 //    lower trapezoid [G ; B^H], panel updates and the triangular solve as DMMA products; the B^H rows
-//    come out as (C^-1 B)^H for free, so only the back substitution C^H theta = z remains.  A
-//    non-positive pivot flags the trial (status bit) instead of poisoning the batch.
+//    come out as (C^-1 B)^H for free, so only the back substitution C^H theta = z remains.  A pivot
+//    that is not above 1e-13 times the largest pivot so far in the trial (NaN included; the identity padding is
+//    exempt) flags the trial (SBCE_ST_NOT_PD) instead of poisoning the batch.
 #include <math.h>
 
 #include "common.cuh"

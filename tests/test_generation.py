@@ -5,8 +5,14 @@ known-answer vectors of Philox4x32-10 and against the signal model's moments.
 GPU part: the CUDA generator element by element against that restatement (symbol indices
 bit-exact), sharding invariance, the LS start against numpy's pinv, and the fully on-device
 sweep driver against the oracle fed with the very same (copied-back) trials."""
+import os
+import sys
+
 import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import mstep_reference as mr  # noqa: E402
 
 
 def relerr(a, b):
@@ -146,6 +152,38 @@ def test_ls_start_matches_pinv(S, case):
         ref = np.linalg.pinv(Wp) @ Yp
         cond = np.linalg.cond(Wp)
         assert relerr(th0[b], ref) < max(1e-9, 1e-14 * cond * cond), (relerr(th0[b], ref), cond)
+
+
+@gpu
+@pytest.mark.parametrize("case", [(8, 2, 2, 40, None), (16, 4, 4, 90, None), (64, 4, 4, 320, None),
+                                  (6, 8, 8, 70, None), (16, 4, 4, 90, 1e-6), (6, 8, 8, 70, 1e-6)])
+def test_ls_start_primal_route_backward_error(S, case):
+    """T_p >= L with distinct, non-zero phase columns: the LS start solves the pilot normal equations
+    (W^H W) theta = W^H y_p with k_chol_solve, unscaled.  Backward error against the exact system within
+    tau(L) = 8 L u, also with column 2 a near-duplicate of column 1 (relative offset eps: cond ~ 1 / eps^2)."""
+    import torch
+
+    N, n_tx, n_rx, T_p, eps = case
+    B = 2
+    prob = S.Problem(N=N, n_tx=n_tx, n_rx=n_rx, M=4, T_p=T_p, T_d=8, itera=1)
+    ses = S.DeviceSession(prob, B)
+    rng = np.random.default_rng(N + T_p)
+    PsiP = np.exp(2j * np.pi * rng.random((B, T_p, N + 1)))
+    if eps is not None:
+        PsiP[:, :, 2] = PsiP[:, :, 1] * np.exp(1j * eps * rng.standard_normal((B, T_p)))
+    Xp = S.qam.constellation(16)[rng.integers(0, 16, (B, T_p, n_tx))]
+    Yp = rng.standard_normal((B, T_p, n_rx)) + 1j * rng.standard_normal((B, T_p, n_rx))
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(ses.device)
+    th0, st = ses.ls_start(t(Yp), t(PsiP), t(Xp))
+    th0, st = th0.cpu().numpy(), st.cpu().numpy()
+    assert st.tolist() == [0] * B
+    L = prob.L
+    for b in range(B):
+        G, Bm = mr.design_system(PsiP[b], Xp[b], Yp[b])
+        if eps is not None:
+            assert np.linalg.cond(G.astype(np.complex128)) > 1e8
+        eta = mr.backward_error(G, Bm, th0[b])
+        assert eta <= mr.tau(L), (eta, mr.tau(L))
 
 
 @gpu

@@ -2,10 +2,17 @@
 identical seeded inputs, and against the golden vectors minted from the literal
 reference.  Bars (BASELINE.json north_star): theta within 1e-9 relative Frobenius at
 equal iteration count, hard-decision indices bit-exact, NMSE to 4 significant figures."""
+import os
+import sys
+from types import SimpleNamespace
+
 import numpy as np
 import pytest
 
 from conftest import golden_names, load_golden
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import mstep_reference as mr  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -143,8 +150,10 @@ MSTEP_CASES = [(8, 2, 2, 4, 12, 30), (32, 2, 2, 4, 40, 50), (6, 1, 4, 16, 8, 20)
                (6, 5, 5, 4, 20, 40), (7, 6, 8, 4, 24, 50), (5, 7, 7, 4, 30, 41), (9, 8, 8, 4, 50, 77),
                (12, 8, 8, 16, 60, 120),
                # long channels: n_tx = 4 beyond the fixed-chunk Gram kernel (N = 256), and a solution vector
-               # that no longer fits in shared memory (L = 1288, n_rx = 8 -> global scratch)
-               (256, 4, 2, 4, 600, 800), (256, 2, 2, 4, 300, 400), (160, 8, 8, 4, 800, 900),
+               # that no longer fits in shared memory (L = 1288, n_rx = 8 -> global scratch); Gaussian-integer inputs
+               # ("int"), whose FP64 Gram is exact, so that the exact system stays cheap at L > 300
+               (256, 4, 2, 4, 600, 800, "int", None), (256, 2, 2, 4, 300, 400, "int", None),
+               (160, 8, 8, 4, 800, 900, "int", None),
                # random Hermitian PD statistics ("pd": no enumeration).  n_tx = 1, L = N + 1 = 2..17: every
                # residue of L mod 16 of the blocked Cholesky, incl. n_rx = 1 (three zero rows under the matrix)
                *[(N, 1, (1, 2, 3, 4, 6, 8)[N % 6], 4, 3, 2 * N + 4, "pd") for N in range(1, 17)],
@@ -153,9 +162,18 @@ MSTEP_CASES = [(8, 2, 2, 4, 12, 30), (32, 2, 2, 4, 40, 50), (6, 1, 4, 16, 8, 20)
                *[(N, n_tx, 3, 4, T_p, T_d, "pd") for N, n_tx in ((20, 2), (10, 4), (6, 6))
                  for T_p, T_d in ((1, 65), (65, 1), (15, 64), (64, 15), (16, 17), (17, 16))],
                # n_tx = 4 on both sides of the TMA / generic Gram switch
-               (143, 4, 2, 4, 64, 300, "pd"), (144, 4, 2, 4, 64, 300, "pd"),
+               (143, 4, 2, 4, 64, 300, "int", None), (144, 4, 2, 4, 64, 300, "int", None),
                # n_rx = 8, Lp = 48 / 56: the solution vector on both sides of the shared / global scratch switch
-               (5, 8, 8, 4, 16, 20, "pd"), (6, 8, 8, 4, 16, 20, "pd")]
+               (5, 8, 8, 4, 16, 20, "pd"), (6, 8, 8, 4, 16, 20, "pd"),
+               # ill-conditioned systems, cond(G) ~ 1e4 / 1e8 / 1e12 from nearly collinear RIS columns (integer
+               # inputs with weighted rows, mstep_reference.integer_inputs) on every Gram kernel: scalar n_tx = 1..3,
+               # TMA and generic n_tx = 4 at N = 143 / 144, wide n_tx = 5..8; L mod 16 = 0, 1, 15 and the solution
+               # vector in shared memory and in global scratch
+               *[(N, n_tx, n_rx, 4, T_p, T_d, "int", cond)
+                 for N, n_tx, n_rx, T_p, T_d in ((16, 1, 1, 4, 30), (23, 2, 2, 8, 40), (4, 3, 3, 2, 12),
+                                                  (143, 4, 2, 16, 170), (144, 4, 2, 16, 170), (6, 5, 5, 4, 12),
+                                                  (7, 6, 3, 4, 14), (6, 7, 7, 4, 12), (6, 8, 8, 4, 12))
+                 for cond in (1e4, 1e8, 1e12)]]
 
 
 def random_pd_stats(rng, B, T, n_tx):
@@ -169,43 +187,56 @@ def random_pd_stats(rng, B, T, n_tx):
 
 @pytest.mark.parametrize("case", MSTEP_CASES)
 def test_mstep_matches_oracle(S, orc, case):
+    """Backward error eta of theta against the exact normal equations (clongdouble, or FP64 from integer inputs)
+    within tau(L) = 8 L u at any conditioning, and the forward error against the refined reference solution within
+    8 L u cond(G)."""
     import torch
 
     N, n_tx, n_rx, M, T_p, T_d, *kind = case
     B = 2
-    tb = S.signal_model.generate_batch(N, n_tx, n_rx, M, T_p, T_d, 0.1, B, seed=5, legacy=False)
+    if kind[:1] == ["int"]:
+        inp = mr.integer_inputs(np.random.default_rng(N * 10 + n_tx), B, N + 1, n_tx, n_rx, T_p, T_d, cond=kind[1])
+        tb = SimpleNamespace(**inp)
+        sm, sR = inp["m"], inp["R"]
+    else:
+        tb = S.signal_model.generate_batch(N, n_tx, n_rx, M, T_p, T_d, 0.1, B, seed=5, legacy=False)
     if kind == ["pd"]:   # random pilot phases: the pilot block observes every RIS element, even when T_d = 1
         tb.PsiP[:] = np.exp(2j * np.pi * np.random.default_rng(N + T_p).random(tb.PsiP.shape))
     cons = orc.qam_constellation(M)
     # (the M-step does not depend on the mode; 8 streams of 16-QAM only exist in the partitioned modes)
     prob = S.Problem(N=N, n_tx=n_tx, n_rx=n_rx, M=M, T_p=T_p, T_d=T_d, itera=1,
                      mode="soft" if n_tx * np.log2(M) <= 24 else "pm_beta")
-    # soft statistics from a perturbed theta so R_t is full-rank-ish; computed by the oracle
-    # (for the 64x4x4 case use rank-one statistics of the true symbols to keep the CPU side fast)
-    sm = np.empty((B, T_d, n_tx), np.complex128)
-    sR = np.empty((B, T_d, n_tx, n_tx), np.complex128)
-    for b in range(B):
-        if kind == ["pd"]:
-            m_, R_ = random_pd_stats(np.random.default_rng(N * 100 + T_d + b), 1, T_d, n_tx)
-            sm[b], sR[b] = m_[0], R_[0]
-        elif M ** n_tx <= 4096 or (n_tx > 4 and N < 10 and M == 4):
-            sm[b], sR[b], _, _ = orc.posterior_stats(tb.Yd[b], tb.PsiD[b], 0.7 * tb.h[b], cons, n_tx, 2.0)
-        else:
-            sm[b], sR[b] = orc.pilot_stats(tb.Xd[b])
+    if kind[:1] != ["int"]:
+        # soft statistics from a perturbed theta so R_t is full-rank-ish; computed by the oracle
+        # (for the 64x4x4 case use rank-one statistics of the true symbols to keep the CPU side fast)
+        sm = np.empty((B, T_d, n_tx), np.complex128)
+        sR = np.empty((B, T_d, n_tx, n_tx), np.complex128)
+        for b in range(B):
+            if kind == ["pd"]:
+                m_, R_ = random_pd_stats(np.random.default_rng(N * 100 + T_d + b), 1, T_d, n_tx)
+                sm[b], sR[b] = m_[0], R_[0]
+            elif M ** n_tx <= 4096 or (n_tx > 4 and N < 10 and M == 4):
+                sm[b], sR[b], _, _ = orc.posterior_stats(tb.Yd[b], tb.PsiD[b], 0.7 * tb.h[b], cons, n_tx, 2.0)
+            else:
+                sm[b], sR[b] = orc.pilot_stats(tb.Xd[b])
     ses = S.DeviceSession(prob, B)
     dev = ses.device
     t = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)
     theta, status = ses.mstep(t(tb.Yd), t(tb.Yp), t(tb.PsiD), t(tb.PsiP), t(tb.Xp), t(sm), t(sR))
     torch.cuda.synchronize()
     theta = theta.cpu().numpy()
-    assert int(status.abs().max()) == 0
+    assert status.cpu().numpy().tolist() == [0] * B
+    L = prob.L
     for b in range(B):
-        mp_, Rp_ = orc.pilot_stats(tb.Xp[b])
-        Gp, Bp = orc.gram_and_rhs(tb.PsiP[b], tb.Yp[b], mp_, Rp_)
-        Gd, Bd = orc.gram_and_rhs(tb.PsiD[b], tb.Yd[b], sm[b], sR[b])
-        ref = np.linalg.solve(Gp + Gd, Bp + Bd)
-        cond = np.linalg.cond(Gp + Gd)
-        assert relerr(theta[b], ref) < max(RTOL, 1e-14 * cond), (relerr(theta[b], ref), cond)
+        if kind[:1] == ["int"]:
+            G, Bm, cond = inp["G"][b], inp["B"][b], inp["cond"][b]
+        else:
+            G, Bm = mr.system(tb.PsiP[b], tb.Yp[b], tb.Xp[b], tb.PsiD[b], tb.Yd[b], sm[b], sR[b])
+            cond = np.linalg.cond(G.astype(np.complex128))
+        eta = mr.backward_error(G, Bm, theta[b])
+        assert eta <= mr.tau(L), (eta, mr.tau(L))
+        err = mr.relerr(theta[b], mr.refined_solve(G, Bm))
+        assert err <= 8 * L * mr.U * cond, (err, cond)
 
 
 def test_mstep_flags_singular_system(S):
