@@ -84,6 +84,27 @@ extern "C" {
 #define SBCE_FLAG_ZF_STOP_GUARD 128u /* ZF mode: the genie stop also requires l != 0, as em_zf of
                                    "Proposed method/all_detectorsvsTd.py":127 has it (PMvsMLvsZFvsMMSE.py:128 does not) */
 
+/* Pilot normal equations.  For T_p > 0 every call first checks on the device, in one pass over the T_p (N+1)(N+2)/2
+ * phase products of the pilot design (once when shared, per trial otherwise, so that both layouts of one design
+ * give the same bits), whether the design is a DFT design up to the error of its phases: for every t and n >= n',
+ *     | conj(psi[t,n]) psi[t,n'] - conj(psi[t,lag]) | <= SBCE_PILOT_LAG_TOL_ULPS * (N+1) * 2^-53 * |psi[t,lag]|,
+ *     lag = n - n' + s for n' >= 1,  lag = n for n' = 0,
+ * for the shift s = 0 (psi[t,n] = w_t^n) or s = 1 (a ones column in front of w_t^0 .. w_t^(N-1), the design of
+ * SBCE_PILOTS_TOP).  A NaN or Inf fails, and so does a design whose entries are not of unit (or zero) modulus, since
+ * the bound is relative.  Then block (n, n') of the pilot Gram is F(lag) = sum_t conj(psi[t,lag]) R_t, N+1 distinct
+ * n_tx x n_tx blocks built by one GEMM instead of a sum per pair (mstep.cu, k_pilot_lag_gram).  A design that
+ * fails keeps the pair form; the choice is made on the device and is invisible to the caller.
+ * The bound: a DFT phase w_t^n = exp(-2j pi t n / T_p) has an argument below 2 pi N.  Computed from that argument
+ * as it stands (numpy's exp(-2j pi t n / T_p), the reference's own construction), a few roundings of it move the
+ * phase by O(N) units of 2^-53: measured, the left side reaches 833 * 2^-53 at T_p = 320, N = 64 and 3329 * 2^-53
+ * at T_p = 320, N = 256, i.e. 13 (N+1) units.  With the argument reduced exactly first (sbce_generate_batch:
+ * sincospi(-2q/T_p), q = t n mod T_p) it stays under 21 units at any N.  The bound, 32 (N+1) units, admits both
+ * constructions and no design that is further from a DFT design than its own phases' rounding makes it.  A term
+ * conj(psi[t,n]) psi[t,n'] R_t of the pilot Gram then moves by at most 32 (N+1) 2^-53 |R_t| (4.6e-13 relative at
+ * N = 64): the lag form gives the pilot Gram of the DFT design the input stands for, as accurately as the input
+ * phases themselves determine it. */
+#define SBCE_PILOT_LAG_TOL_ULPS 32
+
 /* per-trial status bits */
 /* SBCE_ST_NOT_PD: the Cholesky of the normal matrix met a pivot that is not above 1e-13 times the largest pivot
  * so far in the trial (a NaN pivot included; the identity padding rows are exempt): numerically singular M-step */

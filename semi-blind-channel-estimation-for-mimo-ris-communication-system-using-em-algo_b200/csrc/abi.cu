@@ -115,6 +115,8 @@ size_t carve_workspace(const Dims& d, int nb, void* base, Workspace* ws) {
     ws->psiw = (double*)take(B * d.T_p * d.N1 * 16 + 16);
     ws->ls_scale = (double*)take(B * d.N1 * 8);
     ws->ls_rep = (int32_t*)take(B * d.N1 * 4);
+    ws->pil_pair = (int32_t*)take(B * 4);
+    ws->lag_bad = (int32_t*)take(B * 4);
     ws->bytes = off;
     return off;
 }
@@ -166,7 +168,7 @@ static int em_chunk(const Dims& d, int nb, const sbce_io& io, Workspace& ws, cud
         // pilot part of the normal equations, once (the reference recomputes it every iteration:
         // Proposed_method_NMSEvsTp.py:63-65)
         CK(launch_pilot_stats(d, nb, io.Xp, ws.pil_m, ws.pil_R, s));
-        CK(launch_normal_equations(pilot_dims(d), nb, io.PsiP, d.T_p, io.Yp, ws.pil_m, ws.pil_R, nullptr, ws.Gp, nullptr, s));
+        CK(launch_pilot_normal_equations(pilot_dims(d), nb, io.PsiP, io.Yp, ws.pil_m, ws.pil_R, ws, s));
     }
     for (int l = 0; l < d.itera; ++l) {
         int rc = estep_dispatch(d, nb, io.Yd, io.PsiD, io.theta, io.varn, ws.active, ws, ws.stat_m, ws.stat_R,
@@ -352,7 +354,7 @@ int sbce_mstep(const sbce_cfg* cfg, const sbce_io* io, const double* stat_m, con
         const size_t sb = (size_t)b0 * d.T_d;
         CK(cudaMemsetAsync(ws.stat, 0, (size_t)nb * 4, s));
         CK(launch_pilot_stats(d, nb, o.Xp, ws.pil_m, ws.pil_R, s));
-        CK(launch_normal_equations(pilot_dims(d), nb, o.PsiP, d.T_p, o.Yp, ws.pil_m, ws.pil_R, nullptr, ws.Gp, nullptr, s));
+        CK(launch_pilot_normal_equations(pilot_dims(d), nb, o.PsiP, o.Yp, ws.pil_m, ws.pil_R, ws, s));
         CK(launch_normal_equations(d, nb, o.PsiD, d.T_d, o.Yd, stat_m + sb * d.n_tx * 2,
                                    stat_R + sb * d.n_tx * d.n_tx * 2, ws.Gp, ws.G, nullptr, s));
         CK(launch_chol_solve(d, nb, ws.G, theta_out + (size_t)b0 * d.L * d.n_rx * 2, nullptr, ws.stat, ws.thbuf, s));

@@ -107,6 +107,8 @@ struct Workspace {
     double* ls_scale; // [nb][N+1]  sqrt(multiplicity) of a kept column, 0 for a removed one
     int32_t* ls_rep;  // [nb][N+1]  representative column (-1: zero column)
     double* thbuf;    // [nb][Lp][n_rx] cplx  back-substitution vector when it does not fit in shared memory
+    int32_t* pil_pair;// [nb]  the pair-form pilot Gram runs for this trial (written by the lag-form kernel)
+    int32_t* lag_bad; // [nb]  pilot design check (one entry when shared): bit s set when shift s fails (mstep.cu)
     size_t bytes;
 };
 
@@ -125,6 +127,9 @@ cudaError_t launch_enum(const Dims& d, int nb, const double* qr, const double* v
 cudaError_t launch_normal_equations(const Dims& d, int nb, const double* Psi, int T, const double* Y,
                                     const double* sm, const double* sR, const double* Ginit, double* Gout,
                                     const int32_t* active, cudaStream_t s);
+// pilot part G_p, B^H rows and padding into ws.Gp; lag form when the shared pilot design qualifies (d: pilot dims)
+cudaError_t launch_pilot_normal_equations(const Dims& d, int nb, const double* Psi, const double* Y, const double* sm,
+                                          const double* sR, Workspace& ws, cudaStream_t s);
 bool gram_supports(int N1, int n_tx, int n_rx);   // the Gram launch of this shape fits in shared memory (mstep.cu)
 cudaError_t launch_chol_solve(const Dims& d, int nb, double* G, double* theta, const int32_t* active, int32_t* stat,
                               double* th_scratch, cudaStream_t s);

@@ -36,30 +36,19 @@ constexpr int GR_THREADS = 256;
 constexpr int GR_TC = 16;  // symbols per shared-memory chunk (default; shrunk at launch for very long psi rows)
 
 
-// The last CTA of every trial: right-hand side rows B^H stored under the matrix,
-//   row Lp + r, column l = n*n_tx + i :  conj(B[l][r]) = sum_t psi[t,n] conj(m_t[i] y_t[r]),
-// plus the identity padding of the trapezoid.  With Zc[t][i n_rx + r] = conj(m_t[i] y_t[r]) this is the complex
-// GEMM  Out (N+1 x n_tx n_rx) = Psi^T (N+1 x T) . Zc (T x n_tx n_rx)  and runs on the FP64 tensor path: a warp owns
-// one 16-row tile of RIS indices and two 8-column tiles; psi and Zc chunks are staged in shared memory (Zc rows
-// padded by two elements: conflict-free B fragments).  Its scalar predecessor -- one thread per column l, n_rx
-// complex accumulators, 5 shared loads per 4 complex FMAs -- executed 23 % of the Gram kernel's instructions
-// and held 21 % of its resident warp time (profiles/r02d) for 5 % of its arithmetic.
-template <int NTX>
-__device__ __forceinline__ void gram_rhs_cta(const Dims& d, int T, int b, cplx* sPsi, cplx* /*unused*/, const cplx* psi_b,
-                                             const cplx* __restrict__ Y, const cplx* __restrict__ sm, const cplx* Gi,
-                                             cplx* Gb) {
-    const int N1 = d.N1, n_rx = d.n_rx;
-    const int NC = NTX * n_rx;              // complex columns (i, r) -> i * n_rx + r
-    const int ZS = NC + 2;                  // padded row stride of the staged Zc
+// Out (N1 x NC) = Psi^T (N1 x T) . Z (T x NC), complex, on the FP64 tensor path: a warp owns one 16-row tile of
+// RIS indices and two 8-column tiles; psi and Z chunks are staged in shared memory (Z rows padded by two elements:
+// conflict-free B fragments).  zval(t, c) gives Z[t][c] (c < NC), put(n, c, v) takes Out[n][c].  The chunk length
+// is as many symbols as the CTA's dynamic shared memory holds (the pair CTAs of a Gram launch size it for their
+// operand ring), a multiple of 8 (one MMA k-step), at most 128.
+template <typename ZVal, typename Put>
+__device__ __forceinline__ void psi_t_gemm(int N1, int NC, int T, cplx* sPsi, const cplx* psi_b, ZVal zval, Put put) {
+    const int ZS = NC + 2;                  // padded row stride of the staged Z
     unsigned dyn_bytes;
     asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_bytes));
-    // chunk length: as many symbols as the CTA's dynamic shared memory holds (the pair CTAs of the same launch
-    // size it for their operand ring), a multiple of 8 (one MMA k-step), at most 128
     int TCR = (int)(dyn_bytes / (sizeof(cplx) * (N1 + ZS)));
     TCR = max(8, min(TCR & ~7, 128));
     cplx* sZ = sPsi + (size_t)TCR * N1;
-    const cplx* m_b = sm + (size_t)b * T * NTX;
-    const cplx* y_b = Y + (size_t)b * T * n_rx;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, tig = lane & 3;
     const int MT = (N1 + 15) >> 4, NTP = (NC + 15) >> 4;       // 16-row tiles, pairs of 8-column tiles
     const int units = MT * NTP;
@@ -83,12 +72,7 @@ __device__ __forceinline__ void gram_rhs_cta(const Dims& d, int T, int b, cplx* 
                 sPsi[e] = (e < tc * N1) ? psi_b[(size_t)t0 * N1 + e] : mk(0.0, 0.0);
             for (int e = threadIdx.x; e < tc8 * ZS; e += GR_THREADS) {
                 const int tt = e / ZS, c = e % ZS;
-                cplx v = mk(0.0, 0.0);
-                if (tt < tc && c < NC) {
-                    const int ii = c / n_rx, r = c % n_rx;
-                    v = cconj(cmul(m_b[(size_t)(t0 + tt) * NTX + ii], y_b[(size_t)(t0 + tt) * n_rx + r]));
-                }
-                sZ[e] = v;
+                sZ[e] = (tt < tc && c < NC) ? zval(t0 + tt, c) : mk(0.0, 0.0);
             }
             __syncthreads();
             if (live) {
@@ -113,7 +97,7 @@ __device__ __forceinline__ void gram_rhs_cta(const Dims& d, int T, int b, cplx* 
             }
         }
         if (live) {
-            // accumulator (row g + 8h, columns 8 j + 2 tig, + 1) -> G[(Lp + r) * Lp + n * NTX + i]
+            // accumulator (row g + 8h, columns 8 j + 2 tig, + 1)
 #pragma unroll
             for (int j = 0; j < 2; ++j)
 #pragma unroll
@@ -121,16 +105,36 @@ __device__ __forceinline__ void gram_rhs_cta(const Dims& d, int T, int b, cplx* 
 #pragma unroll
                     for (int e = 0; e < 2; ++e) {
                         const int n = n0 + g + 8 * h, c = c0 + 8 * j + 2 * tig + e;
-                        if (n < N1 && c < NC) {
-                            const int ii = c / n_rx, r = c % n_rx;
-                            const size_t o = (size_t)(d.Lp + r) * d.Lp + (n * NTX + ii);
-                            cplx v = mk(cr[j][2 * h + e], ci[j][2 * h + e]);
-                            if (Gi) v = cadd(v, Gi[o]);
-                            Gb[o] = v;
-                        }
+                        if (n < N1 && c < NC) put(n, c, mk(cr[j][2 * h + e], ci[j][2 * h + e]));
                     }
         }
     }
+}
+
+// The last CTA of every trial: right-hand side rows B^H stored under the matrix,
+//   row Lp + r, column l = n*n_tx + i :  conj(B[l][r]) = sum_t psi[t,n] conj(m_t[i] y_t[r]),
+// plus the identity padding of the trapezoid.  With Zc[t][i n_rx + r] = conj(m_t[i] y_t[r]) this is the complex
+// GEMM  Out (N+1 x n_tx n_rx) = Psi^T (N+1 x T) . Zc (T x n_tx n_rx)  (psi_t_gemm).  Its scalar predecessor -- one
+// thread per column l, n_rx complex accumulators, 5 shared loads per 4 complex FMAs -- executed 23 % of the Gram
+// kernel's instructions and held 21 % of its resident warp time (profiles/r02d) for 5 % of its arithmetic.
+template <int NTX>
+__device__ __forceinline__ void gram_rhs_cta(const Dims& d, int T, int b, cplx* sPsi, cplx* /*unused*/, const cplx* psi_b,
+                                             const cplx* __restrict__ Y, const cplx* __restrict__ sm, const cplx* Gi,
+                                             cplx* Gb) {
+    const int n_rx = d.n_rx;
+    const cplx* m_b = sm + (size_t)b * T * NTX;
+    const cplx* y_b = Y + (size_t)b * T * n_rx;
+    psi_t_gemm(d.N1, NTX * n_rx, T, sPsi, psi_b,
+               [&](int t, int c) {
+                   const int ii = c / n_rx, r = c % n_rx;
+                   return cconj(cmul(m_b[(size_t)t * NTX + ii], y_b[(size_t)t * n_rx + r]));
+               },
+               [&](int n, int c, cplx v) {   // -> G[(Lp + r) * Lp + n * NTX + i]
+                   const int ii = c / n_rx, r = c % n_rx;
+                   const size_t o = (size_t)(d.Lp + r) * d.Lp + (n * NTX + ii);
+                   if (Gi) v = cadd(v, Gi[o]);
+                   Gb[o] = v;
+               });
     // padding: identity on the padded diagonal rows L..Lp-1, zero padded columns / rows of B^H
     const int padrows = (d.Lp - d.L) + d.RP;
     for (int e = threadIdx.x; e < padrows * d.Lp; e += GR_THREADS) {
@@ -719,6 +723,144 @@ cudaError_t launch_normal_equations(const Dims& d, int nb, const double* Psi, in
         case 8: return run_gram_wide<8>(d, nb, Psi, T, sR, Y, sm, Ginit, Gout, active, s);
         default: return cudaErrorInvalidValue;
     }
+}
+
+// ---------------------------------------------------------------------------
+// Pilot normal equations in lag form (include/sbce.h, "Pilot normal equations").  When every phase product of the
+// pilot design is, to SBCE_PILOT_LAG_TOL_ULPS (N+1) 2^-53 relative, another column of the design,
+//   conj(psi[t,n]) psi[t,n'] = conj(psi[t,lag(n,n')]),  lag = n - n' + s  (n' >= 1),  lag = n  (n' = 0),
+// with the shift s = 0 (psi[t,n] = w_t^n) or s = 1 (the top-level scripts' design: a ones column in front of
+// w_t^0..w_t^(N-1)), the block (n, n') of G_p is F(lag) = sum_t conj(psi[t,lag]) R_t: N+1 distinct blocks
+// instead of (N+1)(N+2)/2 pair sums, one complex GEMM  Psi^T . conj(R)  of the shape of the right-hand side.
+// ---------------------------------------------------------------------------
+// the shift that qualified (1 preferred), -1: neither did -- the pair-form Gram builds G_p
+__device__ __forceinline__ int pilot_lag_shift(int bad) { return !(bad & 2) ? 1 : (!(bad & 1) ? 0 : -1); }
+
+// One CTA per pilot symbol t (x) and design (y: one when shared, else per trial), all (n >= n') pairs: bit s of
+// bad[y] is set when shift s fails the rule anywhere (a NaN or Inf fails).  bad is cleared before.  The comparison
+// is relative to |psi[t,lag]| (hypot: no underflow at any scale), so a design of any other magnitude fails.
+__global__ void __launch_bounds__(GR_THREADS) k_pilot_lag_check(int N1, int T, const cplx* __restrict__ Psi,
+                                                                int32_t* __restrict__ bad) {
+    const cplx* row = Psi + ((size_t)blockIdx.y * T + blockIdx.x) * N1;
+    const double tol = SBCE_PILOT_LAG_TOL_ULPS * (double)N1 * 0x1p-53;
+    int bits = 0;
+    for (int e = threadIdx.x; e < N1 * N1 && bits != 3; e += GR_THREADS) {
+        const int n = e / N1, np = e % N1;
+        if (np > n) continue;
+        const cplx p = cmulc(row[np], row[n]);   // conj(psi[t,n]) psi[t,n'], as the pair kernels form it
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+            const cplx q = row[(s && np == 0) ? n : n - np + s];
+            const double dx = p.x - q.x, dy = p.y + q.y;     // p - conj(q)
+            if (!(isfinite(dx) && isfinite(dy) && hypot(dx, dy) <= tol * hypot(q.x, q.y))) bits |= 1 << s;
+        }
+    }
+    const int f0 = __syncthreads_or(bits & 1), f1 = __syncthreads_or(bits & 2);
+    if (threadIdx.x == 0 && (f0 | f1)) atomicOr(bad + blockIdx.y, (f0 ? 1 : 0) | (f1 ? 2 : 0));
+}
+
+// Grid (2, nb).  x = 0: the lag table F[b][lag][i][j] into Ftab (the trial's slot of the working matrix, free
+// until the first data Gram), from  Out = Psi^T . Z  with Z[t][i NTX + j] = conj(R_t[i][j]) and F = conj(Out)
+// (R_t is Hermitian); it also tells the pair-form Gram of the same call whether to run (pair_on[b]).
+// x = 1: the right-hand-side rows B^H and the padding of G_p, exactly as the pair-form Gram writes them.
+template <int NTX>
+__global__ void __launch_bounds__(GR_THREADS) k_pilot_lag_gram(Dims d, int T, const cplx* __restrict__ Psi,
+                                                               const cplx* __restrict__ sR, const cplx* __restrict__ Y,
+                                                               const cplx* __restrict__ sm, const int32_t* __restrict__ bad,
+                                                               cplx* __restrict__ Ftab, cplx* __restrict__ Gout,
+                                                               int32_t* __restrict__ pair_on) {
+    extern __shared__ double2 gsm[];
+    const int b = blockIdx.y;
+    const bool lag = pilot_lag_shift(bad[d.psi_shared ? 0 : b]) >= 0;
+    if (blockIdx.x == 0 && threadIdx.x == 0) pair_on[b] = lag ? 0 : 1;
+    if (!lag) return;
+    const size_t gstride = (size_t)d.Ltot * d.Lp;
+    const cplx* psi_b = Psi + (size_t)(d.psi_shared ? 0 : b) * T * d.N1;
+    if (blockIdx.x == 1) {
+        gram_rhs_cta<NTX>(d, T, b, gsm, nullptr, psi_b, Y, sm, nullptr, Gout + (size_t)b * gstride);
+        return;
+    }
+    constexpr int NC = NTX * NTX;
+    const cplx* R_b = sR + (size_t)b * T * NC;
+    cplx* F = Ftab + (size_t)b * gstride;
+    psi_t_gemm(d.N1, NC, T, gsm, psi_b,
+               [&](int t, int c) { return cconj(R_b[(size_t)t * NC + c]); },
+               [&](int n, int c, cplx v) { F[(size_t)n * NC + c] = cconj(v); });
+}
+
+// Writes the lower block triangle of G_p, block (n, n') = F(lag(n, n')): a warp per matrix row, LAG_ROWS rows per
+// CTA (few CTAs to retire when the design does not qualify).
+constexpr int LAG_ROWS = 4 * (GR_THREADS / 32);
+__global__ void __launch_bounds__(GR_THREADS) k_pilot_lag_expand(Dims d, const int32_t* __restrict__ bad,
+                                                                 const cplx* __restrict__ Ftab, cplx* __restrict__ Gout) {
+    const int b = blockIdx.y;
+    const int s = pilot_lag_shift(bad[d.psi_shared ? 0 : b]);
+    if (s < 0) return;
+    const int ntx = d.n_tx, nc = ntx * ntx, lane = threadIdx.x & 31;
+    const size_t gstride = (size_t)d.Ltot * d.Lp;
+    for (int r = blockIdx.x * LAG_ROWS + (threadIdx.x >> 5); r < min(d.L, (blockIdx.x + 1) * LAG_ROWS);
+         r += GR_THREADS / 32) {
+        const int n = r / ntx, i = r - n * ntx;
+        const cplx* F = Ftab + (size_t)b * gstride + i * ntx;
+        cplx* row = Gout + (size_t)b * gstride + (size_t)r * d.Lp;
+        for (int c = lane; c < (n + 1) * ntx; c += 32) {
+            const int np = c / ntx, j = c - np * ntx;
+            const int lag = (s && np == 0) ? n : n - np + s;
+            row[c] = F[(size_t)lag * nc + j];
+        }
+    }
+}
+
+template <int NTX>
+static cudaError_t run_pilot_lag_gram(const Dims& d, int nb, const double* Psi, int T, const double* Y,
+                                      const double* sm, const double* sR, Workspace& ws, cudaStream_t s) {
+    static SmemOptIn optin;
+    // the two GEMM CTAs stage chunks of up to 32 symbols, at least one 8-symbol MMA step (gram_supports())
+    const int zs = (NTX * NTX > NTX * d.n_rx ? NTX * NTX : NTX * d.n_rx) + 2;
+    int tc = 32;
+    while (tc > 8 && sizeof(cplx) * (size_t)(tc * (d.N1 + zs)) > 100 * 1024) tc >>= 1;
+    const size_t smem = sizeof(cplx) * (size_t)(tc * (d.N1 + zs));
+    cudaError_t e = opt_in_smem(optin, (const void*)k_pilot_lag_gram<NTX>, smem);
+    if (e != cudaSuccess) return e;
+    k_pilot_lag_gram<NTX><<<dim3(2, nb), GR_THREADS, smem, s>>>(d, T, (const cplx*)Psi, (const cplx*)sR, (const cplx*)Y,
+                                                               (const cplx*)sm, ws.lag_bad, (cplx*)ws.G, (cplx*)ws.Gp,
+                                                               ws.pil_pair);
+    count_launch();
+    return cudaGetLastError();
+}
+
+// Pilot part of the normal equations into ws.Gp (lower triangle, B^H rows, padding).  The pilot design (once when
+// shared, else per trial, so that both layouts of one design give the same bits) is checked on the device; the lag form runs when it qualifies, the pair-form Gram otherwise.  Both are launched and
+// the one not chosen exits at once, so the schedule does not depend on the data (no host synchronisation, and the
+// same CUDA graph serves either design).
+cudaError_t launch_pilot_normal_equations(const Dims& d, int nb, const double* Psi, const double* Y, const double* sm,
+                                          const double* sR, Workspace& ws, cudaStream_t s) {
+    const int T = d.T_p;
+    if (T == 0) return launch_normal_equations(d, nb, Psi, T, Y, sm, sR, nullptr, ws.Gp, nullptr, s);
+    if (d.n_rx > RH_MAXR) return cudaErrorInvalidValue;
+    const int npsi = d.psi_shared ? 1 : nb;
+    cudaError_t e = cudaMemsetAsync(ws.lag_bad, 0, sizeof(int32_t) * npsi, s);
+    if (e != cudaSuccess) return e;
+    k_pilot_lag_check<<<dim3(T, npsi), GR_THREADS, 0, s>>>(d.N1, T, (const cplx*)Psi, ws.lag_bad);
+    count_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    switch (d.n_tx) {
+        case 1: e = run_pilot_lag_gram<1>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 2: e = run_pilot_lag_gram<2>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 3: e = run_pilot_lag_gram<3>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 4: e = run_pilot_lag_gram<4>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 5: e = run_pilot_lag_gram<5>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 6: e = run_pilot_lag_gram<6>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 7: e = run_pilot_lag_gram<7>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        case 8: e = run_pilot_lag_gram<8>(d, nb, Psi, T, Y, sm, sR, ws, s); break;
+        default: return cudaErrorInvalidValue;
+    }
+    if (e != cudaSuccess) return e;
+    k_pilot_lag_expand<<<dim3((d.L + LAG_ROWS - 1) / LAG_ROWS, nb), GR_THREADS, 0, s>>>(
+        d, ws.lag_bad, (const cplx*)ws.G, (cplx*)ws.Gp);
+    count_launch();
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    return launch_normal_equations(d, nb, Psi, T, Y, sm, sR, nullptr, ws.Gp, ws.pil_pair, s);
 }
 
 }  // namespace sbce
