@@ -186,7 +186,11 @@ int sbce_host_split_threshold(void);
  * pointers.  stat_m [B][T_d][n_tx], stat_R [B][T_d][n_tx][n_tx] complex128,
  * kstar [B][T_d] int32 (nullable), lse_sym [B][T_d] float64 (nullable).
  * Uses cfg->mode exactly as the EM loop does; as there, kstar is -1 in the PM / PM_BETA
- * modes and lse_sym is NaN in the PM, PM_BETA, ZF and MMSE modes. */
+ * modes and lse_sym is NaN in the PM, PM_BETA, ZF and MMSE modes.
+ * Scale: the soft and hard statistics, kstar and lse_sym depend on (Yd, theta, varn) only through d2/varn^2, and
+ * scaling all three by 2^k leaves every output bit unchanged as long as every d2, varn^2 and 1/varn^2 stays a
+ * normal FP64 number below 1e300 (the E-step's initial reference distance and slicer sentinels).  The bit LLRs
+ * (sbce_bit_llr, sbce_bit_llr_apriori with La unscaled) share that property. */
 int sbce_estep(const sbce_cfg* cfg, const sbce_io* io, const double* theta, double* stat_m,
                double* stat_R, int32_t* kstar, double* lse_sym, void* workspace,
                size_t workspace_bytes, void* stream);

@@ -427,7 +427,9 @@ __device__ __noinline__ void enum_flush(double* ws, double warp_best, int count)
     const double inv_s2 = ws[E::O_S2];
     double aref = ws[E::O_AREF];
     if (warp_best < aref) {
-        const double f = exp((warp_best - aref) * inv_s2);  // aref = +inf initially -> f = 0
+        // aref starts at the finite sentinel 1e300, above every admitted d2 (include/sbce.h): the argument is then
+        // hugely negative (or -inf), f = 0, and the still-zero accumulators stay zero
+        const double f = exp((warp_best - aref) * inv_s2);
         for (int i = lane; i < E::NACC; i += E::G) ws[E::O_ACC + i] *= f;
         aref = warp_best;
     }

@@ -12,6 +12,7 @@ import pytest
 from conftest import golden_names, load_golden
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+import estep_reference as er  # noqa: E402
 import mstep_reference as mr  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -59,9 +60,15 @@ ESTEP_CASES = [
 ]
 
 
+_ESTEP_REFS = {}
+
+
 @pytest.mark.parametrize("case", ESTEP_CASES)
 @pytest.mark.parametrize("hard", [False, True])
 def test_estep_matches_oracle(S, orc, case, hard):
+    """m, R and lse within the derived bound tau of the exact (clongdouble) statistics, kstar by the gap rule
+    (tests/estep_reference.py): the oracle's FP64 distances are formed directly, the device's through a QR, so
+    neither is bit-exact against the other; the extended-precision reference decides."""
     import torch
 
     N, n_tx, n_rx, M, T_d, varn = case
@@ -79,14 +86,14 @@ def test_estep_matches_oracle(S, orc, case, hard):
     torch.cuda.synchronize()
     m, R, ks, ls = m.cpu().numpy(), R.cpu().numpy(), ks.cpu().numpy(), ls.cpu().numpy()
     cons = orc.qam_constellation(M)
-    stats = orc.posterior_stats if M ** n_tx <= 1 << 18 else orc.posterior_stats_split
+    if case not in _ESTEP_REFS:    # soft and hard share the reference
+        _ESTEP_REFS[case] = [er.reference(tb.Yd[b], tb.PsiD[b], theta[b], cons, n_tx, varn) for b in range(B)]
     for b in range(B):
-        mo, Ro, ko, lo = stats(tb.Yd[b], tb.PsiD[b], theta[b], cons, n_tx, varn, hard=hard)
-        assert np.array_equal(ks[b], ko), "hard-decision indices must be bit-exact"
-        assert np.abs(m[b] - mo).max() < 1e-10 * max(1.0, np.abs(mo).max())
-        assert np.abs(R[b] - Ro).max() < 1e-10 * max(1.0, np.abs(Ro).max())
-        if not hard:
-            np.testing.assert_allclose(ls[b], lo, rtol=1e-10, atol=1e-8)
+        ref = _ESTEP_REFS[case][b]
+        assert not er.kstar_bad(ref, ks[b]), er.kstar_bad(ref, ks[b])[:4]
+        r, adm = er.ratios(ref, m[b], R[b], ls[b], hard, ks[b])
+        assert r <= 1.0, (b, r)
+        assert adm == T_d or hard
 
 
 @pytest.mark.parametrize("case", [(8, 2, 2, 16, 40, 0.1), (6, 3, 3, 16, 24, 0.4), (8, 4, 4, 16, 24, 0.1),
